@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the B200 BLS12-381 pairing path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): a batch of 2^16 independent full pairings (Miller loop + final
 exponentiation) per GPU per step, on synthetic subgroup points generated on the device by the
@@ -36,6 +36,7 @@ MAC32_PER_MM_PAIR = 4684 * 300           # multi-Miller per pair incl. on-the-fl
 MAC32_PER_G2_WNAF_PREP = 7992 * 300      # G2 wNAF w=4 + normalisation + G2Prepared::from_affine
 HBM_BYTES_PER_PAIRING = 104 + 200 + 576  # G1Affine + G2Affine in, Fq12 out
 SEED = 0x5DBE62598D313D76
+DUMP_ROWS = 1 << 15                      # 2^15 GT elements x 144 words x 8 B = 37.7 MB per dump
 
 
 def parse():
@@ -53,7 +54,12 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-mgpu", action="store_true")
     ap.add_argument("--no-wnaf-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the pairings the last step computed (rank 0) to DIR/*.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; the reference arm times a host-sized sample")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -252,6 +258,18 @@ def make_inputs(eng, n, seed, torch, np):
     return pa, qa, p, scalars(seed ^ 0x3333)
 
 
+def dump_outputs(dirname, out, np):
+    """Write the (n, 72) GT elements of one step as DIR/pairing.npy: the rows of a fixed, seeded sample of at most
+    DUMP_ROWS pairings (every row of a smaller batch), each as its 144 32-bit words (12 Fq coefficients x 12 Montgomery
+    limbs, least significant first), in float64, which holds every word exactly.  DIR/pairing_rows.npy: the row indices."""
+    n = out.shape[0]
+    rows = np.sort(np.random.default_rng(SEED).choice(n, min(n, DUMP_ROWS), replace=False))
+    words = out.cpu().numpy()[rows].view(np.uint32)
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "pairing.npy"), words.astype(np.float64))
+    np.save(os.path.join(dirname, "pairing_rows.npy"), rows.astype(np.float64))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -320,6 +338,8 @@ def run_ours(args):
     kernel_ms = sum(a.elapsed_time(b) for a, b in kev) / args.steps     # the pairing kernel alone, this rank
     clocks = sampler.stop() if rank == 0 else None
     value = world * n * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, np)               # `out` holds the last timed step's result
 
     # ---- e2e: host buffers through the C-ABI call a user makes (copies inside the timed region)
     ph = torch.empty(pa.shape, dtype=torch.int64).pin_memory(); ph.copy_(pa.cpu())
