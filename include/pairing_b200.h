@@ -149,6 +149,14 @@ int bls_g2_into_affine_batch(bls_ctx*, const bls_g2* in, bls_g2_affine* out, siz
 enum { BLS_PT_DOUBLE = 0, BLS_PT_ADD = 1, BLS_PT_ADD_MIXED = 2, BLS_PT_NEGATE = 3, BLS_PT_SUB = 6 };
 int bls_g1_op_batch(bls_ctx*, int op, const bls_g1* a, const void* b, bls_g1* out, size_t n);
 int bls_g2_op_batch(bls_ctx*, int op, const bls_g2* a, const void* b, bls_g2* out, size_t n);
+/* Multi-scalar multiplication: out1 = sum_i k_i * bases_i (the shape downstream provers and batch verifiers build from
+ * CurveAffine::add_assign_mixed, ec.rs:446-526), by the bucket (Pippenger) method.  k_i is the full 256-bit integer of the
+ * FrRepr, NOT reduced mod r, so the sum is exact for bases outside the r-order subgroup as well.  Infinity bases and zero
+ * scalars contribute nothing.  out1 is the NORMALISED representative -- (x, y, one) as into_projective(into_affine(S)) gives
+ * it, or G::zero() = (0, one, 0) -- unique, hence bit-exact whatever the summation order.  n = 0 gives G::zero().
+ * n is at most 2^26 (BLS_ERR_INVALID_ARGUMENT above). */
+int bls_g1_msm(bls_ctx*, const bls_g1_affine* bases, const bls_fr_repr* k, size_t n, bls_g1* out1);
+int bls_g2_msm(bls_ctx*, const bls_g2_affine* bases, const bls_fr_repr* k, size_t n, bls_g2* out1);
 
 /* ------------------------------------------------------------------ point encodings (host buffers)
  * EncodedPoint::into_affine (checked != 0: on-curve and r-order-subgroup checks) / into_affine_unchecked and
@@ -236,6 +244,13 @@ int bls_g2_wnaf_fixed_base_dev(bls_ctx*, const bls_g2* table, int window, const 
 size_t bls_batch_normalization_scratch_bytes(const bls_ctx*, int degree, size_t n);
 int bls_g1_batch_normalization_dev(bls_ctx*, bls_g1* inout, size_t n, void* scratch, void* stream);
 int bls_g2_batch_normalization_dev(bls_ctx*, bls_g2* inout, size_t n, void* scratch, void* stream);
+/* bls_g*_msm on device pointers; out1 is one device point.  window = bucket width c in bits, 2..20, or 0 = the library's
+ * choice for n.  n <= 2^26 and ceil(257 / c) * n < 2^31, else BLS_ERR_INVALID_ARGUMENT.  scratch: bls_msm_scratch_bytes(ctx,
+ * degree, n, window) bytes (degree 1 = G1, 2 = G2; 0 for invalid arguments); it holds everything, including the radix sort's
+ * temporary storage: the call allocates nothing. */
+size_t bls_msm_scratch_bytes(const bls_ctx*, int degree, size_t n, int window);
+int bls_g1_msm_dev(bls_ctx*, const bls_g1_affine* bases, const bls_fr_repr* k, size_t n, int window, bls_g1* out1, void* scratch, void* stream);
+int bls_g2_msm_dev(bls_ctx*, const bls_g2_affine* bases, const bls_fr_repr* k, size_t n, int window, bls_g2* out1, void* scratch, void* stream);
 
 /* ------------------------------------------------------------------ several GPUs behind ONE call
  * Engine::miller_loop takes ALL pairs of a product in one call (mod.rs:40-102), and a Rust / C caller is one process.

@@ -336,6 +336,14 @@ template <class Proj, class Aff, bool IS_G2> struct Curve {
     else g.check(bls_g1_wnaf_mul_batch(g.ctx(), bases.data(), k.data(), out.data(), bases.size()));
     return out;
   }
+  // sum_i k_i * bases_i (bucket method): the normalised representative, (x, y, one) or zero() = (0, one, 0)
+  static Proj multiexp(Gpu& g, const std::vector<Aff>& bases, const std::vector<FrRepr>& k) {
+    require_same_length(bases.size(), k.size(), "multiexp");
+    Proj out;
+    if constexpr (IS_G2) g.check(bls_g2_msm(g.ctx(), bases.data(), k.data(), bases.size(), &out));
+    else g.check(bls_g1_msm(g.ctx(), bases.data(), k.data(), bases.size(), &out));
+    return out;
+  }
   // From<affine> for projective (ec.rs:570-582)
   static std::vector<Proj> into_projective(const std::vector<Aff>& a) {
     std::vector<Proj> out(a.size());

@@ -49,6 +49,7 @@ SYMBOLS = [
     "bls_mgpu_create", "bls_mgpu_destroy", "bls_mgpu_device_count", "bls_mgpu_ctx", "bls_mgpu_multi_miller_loop",
     "bls_mgpu_pairing_product", "bls_mgpu_pairing_batch", "bls_mgpu_g1_wnaf_mul_batch", "bls_mgpu_g2_wnaf_mul_batch",
     "bls_mgpu_last_phase_ms",
+    "bls_g1_msm", "bls_g2_msm", "bls_msm_scratch_bytes", "bls_g1_msm_dev", "bls_g2_msm_dev",
 ]
 
 
@@ -88,6 +89,8 @@ def load():
         getattr(lib, name).argtypes = [vp, sz]
     lib.bls_batch_normalization_scratch_bytes.restype = sz
     lib.bls_batch_normalization_scratch_bytes.argtypes = [vp, ci, sz]
+    lib.bls_msm_scratch_bytes.restype = sz
+    lib.bls_msm_scratch_bytes.argtypes = [vp, ci, sz, ci]
     sig = {
         "bls_g2_prepare_batch": [vp, vp, vp, sz],
         "bls_miller_loop_batch": [vp, vp, vp, vp, sz],
@@ -159,6 +162,10 @@ def load():
         "bls_mgpu_g1_wnaf_mul_batch": [vp, vp, vp, vp, sz],
         "bls_mgpu_g2_wnaf_mul_batch": [vp, vp, vp, vp, sz],
         "bls_mgpu_last_phase_ms": [vp, ctypes.POINTER(ctypes.c_double)],
+        "bls_g1_msm": [vp, vp, vp, sz, vp],
+        "bls_g2_msm": [vp, vp, vp, sz, vp],
+        "bls_g1_msm_dev": [vp, vp, vp, sz, ci, vp, vp, vp],
+        "bls_g2_msm_dev": [vp, vp, vp, sz, ci, vp, vp, vp],
     }
     lib.bls_mgpu_create.restype = vp
     lib.bls_mgpu_create.argtypes = [ctypes.POINTER(ci), ci, ctypes.POINTER(ci)]
@@ -440,6 +447,23 @@ class Context:
     def g1_op(self, op, a, b=None): return self._pt_op(False, op, a, b)
     def g2_op(self, op, a, b=None): return self._pt_op(True, op, a, b)
 
+    def _msm(self, g2, bases, k):
+        bases, k = _arr(bases, W_G2A if g2 else W_G1A, "bases"), _arr(k, W_FR, "k")
+        if bases.shape[0] != k.shape[0]:
+            raise ValueError("bases and k must have the same length")
+        out = np.zeros((1, W_G2 if g2 else W_G1), dtype=np.uint64)
+        fn = self._lib.bls_g2_msm if g2 else self._lib.bls_g1_msm
+        self._check(fn(self._ctx, _p(bases), _p(k), bases.shape[0], _p(out)))
+        return out
+
+    def g1_msm(self, bases, k):
+        """sum_i k_i * bases_i over (n, 13) affine bases and (n, 4) FrRepr scalars -> one normalised Jacobian row (1, 18)."""
+        return self._msm(False, bases, k)
+
+    def g2_msm(self, bases, k):
+        """sum_i k_i * bases_i over (n, 25) affine bases and (n, 4) FrRepr scalars -> one normalised Jacobian row (1, 36)."""
+        return self._msm(True, bases, k)
+
     # ------------------------------------------------------------------ field tower, host arrays
     def field_op(self, degree, op, a, b=None):
         a = _arr(a, 6 * degree, "a")
@@ -514,6 +538,13 @@ class Context:
 
     def batch_normalization_scratch_bytes(self, degree, n):
         return int(self._lib.bls_batch_normalization_scratch_bytes(self._ctx, degree, n))
+
+    def msm_scratch_bytes(self, degree, n, window=0):
+        """device scratch of bls_g*_msm_dev (degree 1 = G1, 2 = G2); raises for arguments the call would reject"""
+        b = int(self._lib.bls_msm_scratch_bytes(self._ctx, degree, n, window))
+        if b == 0:
+            raise ValueError("no MSM of degree %r, n = %d, window = %d" % (degree, n, window))
+        return b
 
     def imad_peak(self, variant=0, iters=2000):
         macs, ms = ctypes.c_double(0), ctypes.c_double(0)

@@ -158,6 +158,22 @@ class DeviceEngine:
         self.ctx.call_dev("bls_g2_wnaf_mul_dev", bases.data_ptr(), k.data_ptr(), out.data_ptr(), bases.shape[0], window, self._stream())
         return out
 
+    def msm(self, bases, k, g2=False, window=0, out=None):
+        """sum_i k_i * bases_i over affine rows ((n, 13) G1 / (n, 25) G2) and (n, 4) FrRepr scalars -> one normalised
+        Jacobian row (1, 18) / (1, 36).  window: bucket width c in 2..20, 0 = the library's choice for n."""
+        _check(bases, nat.W_G2A if g2 else nat.W_G1A, "bases"); _check(k, nat.W_FR, "k")
+        n = bases.shape[0]
+        if k.shape[0] != n:
+            raise ValueError("bases and k must have the same length")
+        if out is None:
+            out = torch.empty((1, nat.W_G2 if g2 else nat.W_G1), dtype=torch.int64, device=self.device)
+        else:
+            _check(out, nat.W_G2 if g2 else nat.W_G1, "out")
+        scr = self._buf("msm", self.ctx.msm_scratch_bytes(2 if g2 else 1, n, window))
+        self.ctx.call_dev("bls_g2_msm_dev" if g2 else "bls_g1_msm_dev", bases.data_ptr(), k.data_ptr(), n, window, out.data_ptr(),
+                          scr.data_ptr(), self._stream())
+        return out
+
     def wnaf_table(self, base, window, g2=False):
         """Wnaf::base(g, n): the shared window table (2^(window-1), W) on the device."""
         w = nat.W_G2 if g2 else nat.W_G1

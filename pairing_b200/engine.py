@@ -98,6 +98,13 @@ class _Curve:
         c = _ctx(ctx)
         return (c.g2_batch_normalization if cls._g2 else c.g1_batch_normalization)(v)
 
+    # sum_i k_i * bases_i over affine bases (the sum provers and batch verifiers build from add_assign_mixed, ec.rs:446-526):
+    # one normalised Jacobian row, (x, y, one) or zero() = (0, one, 0).  Scalars are full 256-bit FrRepr integers.
+    @classmethod
+    def multiexp(cls, bases_affine, scalars, ctx=None):
+        c = _ctx(ctx)
+        return (c.g2_msm if cls._g2 else c.g1_msm)(bases_affine, scalars)
+
     # ec.rs:895-905 / 1586-1596
     @classmethod
     def recommended_wnaf_for_scalar(cls, scalars):

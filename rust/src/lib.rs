@@ -120,6 +120,18 @@ impl Gpu {
         Ok(out.iter().map(marshal::g1_back).collect())
     }
 
+    /// `sum_i k_i * bases_i` by the bucket method: the normalised sum (`into_projective(into_affine(S))`, or `G1::zero()`).
+    /// Scalars are full 256-bit `FrRepr` integers (not reduced mod r).
+    pub fn g1_multiexp(&self, bases: &[G1Affine], k: &[FrRepr]) -> Result<G1, GpuError> {
+        assert_eq!(bases.len(), k.len());
+        let bb: Vec<bls_g1_affine> = bases.iter().map(marshal::g1_affine).collect();
+        let kk: Vec<bls_fr_repr> = k.iter().map(|r| bls_fr_repr { l: r.0 }).collect();
+        let mut out = bls_g1 { x: marshal::FQ_ZERO, y: marshal::FQ_ZERO, z: marshal::FQ_ZERO };
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_g1_msm(*ctx, bb.as_ptr(), kk.as_ptr(), bb.len(), &mut out) }, *ctx)?;
+        Ok(marshal::g1_back(&out))
+    }
+
     /// `let q = Q.prepare(); ps.iter().map(|p| Bls12::pairing(p, Q))` with the one `G2Prepared` staged on the device.
     pub fn pairing_shared_q(&self, p: &[G1Affine], q: &G2Affine) -> Result<Vec<Fq12>, GpuError> {
         let pp: Vec<bls_g1_affine> = p.iter().map(marshal::g1_affine).collect();
@@ -143,7 +155,7 @@ impl Gpu {
         check(unsafe { bls_g1_decode_batch(*ctx, bytes.as_ptr(), 1, 1, out.as_mut_ptr(), status.as_mut_ptr(), n) }, *ctx)?;
         Ok(out.iter().zip(status).map(|(a, s)| if s == 0 { Ok(marshal::g1_affine_back(a)) } else { Err(s) }).collect())
     }
-    // g2_wnaf_mul_batch, g2_batch_normalization, g2_prepare_batch, miller_loop_batch, the other encodings: same pattern.
+    // g2_wnaf_mul_batch, g2_batch_normalization, g2_prepare_batch, miller_loop_batch, g2_multiexp, the other encodings: same pattern.
 }
 
 impl Drop for Gpu {
