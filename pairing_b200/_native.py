@@ -9,8 +9,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# PAIRING_B200_LIB lets tuning experiments point at an alternative build of the same library
-LIB_PATH = os.environ.get("PAIRING_B200_LIB") or os.path.join(_HERE, "lib", "libpairing_b200.so")
+LIB_PATH = os.path.join(_HERE, "lib", "libpairing_b200.so")
 
 # u64 words per ABI struct
 W_FQ, W_FQ2, W_FQ6, W_FQ12 = 6, 12, 36, 72

@@ -76,12 +76,8 @@ struct bls_ctx {
 };
 // Defaults of the two limits: below them one WARP per element (~2 ms for one pairing or for a thousand) beats the lane-pair
 // throughput kernels (8.8 ms of latency, 1.49 M pairings/s); bls_ctx_set_latency_path_limits overrides them per context.
-#ifndef BLS_WIDE_PAIRING_MAX
 #define BLS_WIDE_PAIRING_MAX 2560
-#endif
-#ifndef BLS_WIDE_FINAL_EXP_MAX
 #define BLS_WIDE_FINAL_EXP_MAX 2560
-#endif
 
 #define CK(call)                                                                      \
   do {                                                                                \

@@ -148,19 +148,8 @@ template <class F> __device__ __forceinline__ bool is_on_curve(const Aff<F>& p) 
 //   G1:  (beta x, y) = [-u^2] P      beta = the primitive cube root of unity acting as -u^2 on G1 (BLS_ENDO_BETA)
 //   G2:  psi(Q) = [u] Q              psi = twist o Frobenius o untwist: (conj(x) BLS_PSI_X, conj(y) BLS_FROB_FQ12_C1[3])
 // with u = -0xd201000000010000: one (G2) or two (G1) 64-bit multiplications by |u| -- 63 doublings and 5 additions each.
-// -DBLS_SUBGROUP_CHECK_BY_ORDER=1 keeps the reference's multiplication by r (A/B runs, tests/test_gpu_codec.py compares both
-// answers with the big-integer model on points inside and outside the subgroup).
-#ifndef BLS_SUBGROUP_CHECK_BY_ORDER
-#define BLS_SUBGROUP_CHECK_BY_ORDER 0
-#endif
-template <class F> __device__ __forceinline__ bool is_in_correct_subgroup_by_order(const Aff<F>& p) {
-  Jac<F> j;
-  if (p.inf) { pt_set_zero(j); } else { j.x = p.x; j.y = p.y; f_set_one(j.z); }
-  // r = 0x73eda753299d7d483339d80809a1d80553bda402fffe5bfeffffffff00000001 (fr.rs:6-12)
-  const Scalar r = {{0x00000001u, 0xffffffffu, 0xfffe5bfeu, 0x53bda402u, 0x09a1d805u, 0x3339d808u, 0x299d7d48u, 0x73eda753u}};
-  pt_mul(j, r);
-  return pt_is_zero(j);
-}
+// tests/test_gpu_codec.py compares the answers with the big-integer model on points inside and outside the subgroup.  The
+// reference's multiplication by r was removed from this file; it can be recovered from git history at commit 7b088bd.
 // [|u|] P for an affine P (mixed additions) and for a Jacobian P (general additions); |u| = 2^63 + 2^62 + 2^60 + 2^57 + 2^48 + 2^16
 template <class F> __device__ __noinline__ void pt_mul_u_abs(Jac<F>& out, const Aff<F>& p) {
   Jac<F> res;
@@ -187,23 +176,20 @@ template <class F> __device__ __forceinline__ bool jac_neg_equals_affine(const J
   const F zz = f_sqr(t.z);
   return f_eq(t.x, f_mul(x, zz)) && f_eq(f_neg(t.y), f_mul(y, f_mul(zz, t.z)));
 }
-__device__ __forceinline__ bool is_in_correct_subgroup_fast(const Aff<Fp>& p) {
+__device__ __forceinline__ bool is_in_correct_subgroup(const Aff<Fp>& p) {
   if (p.inf) return true;
   Jac<Fp> t, t2;
   pt_mul_u_abs(t, p);
   pt_mul_u_abs(t2, t);                                   // [u^2] P
   return jac_neg_equals_affine(t2, fp_mul(p.x, fp_from_const(BLS_ENDO_BETA)), p.y);
 }
-__device__ __forceinline__ bool is_in_correct_subgroup_fast(const Aff<Fp2>& p) {
+__device__ __forceinline__ bool is_in_correct_subgroup(const Aff<Fp2>& p) {
   if (p.inf) return true;
   Jac<Fp2> t;
   pt_mul_u_abs(t, p);                                    // [|u|] Q = -[u] Q
   const Fp2 px = fp2_mul(Fp2{p.x.c0, fp_neg(p.x.c1)}, fp2_from_const(BLS_PSI_X[0]));
   const Fp2 py = fp2_mul(Fp2{p.y.c0, fp_neg(p.y.c1)}, fp2_from_const(BLS_FROB_FQ12_C1[3]));
   return jac_neg_equals_affine(t, px, py);
-}
-template <class F> __device__ __forceinline__ bool is_in_correct_subgroup(const Aff<F>& p) {
-  return BLS_SUBGROUP_CHECK_BY_ORDER ? is_in_correct_subgroup_by_order(p) : is_in_correct_subgroup_fast(p);
 }
 
 // $affine::mul_bits with the cofactor (ec.rs:86-94, 871-875, 1564-1578): MSB-first over ALL bits of the limb array,

@@ -428,16 +428,9 @@ static __device__ __noinline__ Fp fp_mul2(Fp x, Fp bx, Fp y, Fp by) { return fp_
 #include "fp_sqr_gen.cuh"
 namespace bls {
 // fq.rs:963-1016 `square`: the dedicated 234-MAC32 routine of fp_sqr_gen.cuh (generated and emulated by
-// tools/gen_fp_sqr.py).  A translation unit may fall back to fp_mul(a, a) -- one copy of the product code, the same
-// canonical value -- with -DBLS_FP_SQR_DEDICATED=0 when the instruction-cache footprint matters more than the 66 MACs.
-#ifndef BLS_FP_SQR_DEDICATED
-#define BLS_FP_SQR_DEDICATED 1
-#endif
-#if BLS_FP_SQR_DEDICATED
+// tools/gen_fp_sqr.py).  The fallback to fp_mul(a, a) -- one copy of the product code, the same canonical value -- was
+// removed; it can be recovered from git history at commit 7b088bd.
 static __device__ __noinline__ Fp fp_sqr(Fp a) { return fp_sqr_inline(a); }
-#else
-__device__ __forceinline__ Fp fp_sqr(const Fp& a) { return fp_mul(a, a); }
-#endif
 
 // FrRepr (fr.rs:57-58): a canonical 256-bit integer as 8 x u32 -- scalars and GT exponents
 struct Scalar { uint32_t v[8]; };

@@ -169,9 +169,7 @@ __global__ void __launch_bounds__(128) k_fq12_product(const uint64_t* in, size_t
 // ------------------------------------------------------------------------------------------------
 // Curve kernels
 // ------------------------------------------------------------------------------------------------
-#ifndef BLS_WNAF_MINB
 #define BLS_WNAF_MINB 3
-#endif
 template <class F, int K, int MAXT> struct LocalTables {
   Jac<F> t[K][MAXT];
   __device__ __forceinline__ Jac<F> get(int j, int e) const { return t[j][e]; }
@@ -182,16 +180,10 @@ template <class F> struct SharedTable {
 };
 
 // K points per thread (pt_wnaf_run_lazy): thread t owns points t, t + T, ..., t + (K-1) T
-#ifndef BLS_WNAF_K
 #define BLS_WNAF_K 3      /* G1: 9.57 M muls/s at 2^22 against 9.33 M for K = 2 (lane efficiency 95 % vs 91 %) */
-#endif
-#ifndef BLS_WNAF_K_G2
 #define BLS_WNAF_K_G2 2
-#endif
 // blocks per SM: 3 for G2 (168 registers; 3.29 M muls/s at 2^20 against 3.19 M with 2 and 2.90 M with 4), BLS_WNAF_MINB_G1 for G1
-#ifndef BLS_WNAF_MINB_G1
 #define BLS_WNAF_MINB_G1 4   /* 128 registers.  With the dedicated squaring (r2, 2^22 points, one box): 398.8 ms with 4 blocks, 405.1 with 5 (96 registers), 415.2 with 3, 425.7 with 6; K = 2 at 4 blocks 404.4 */
-#endif
 // MAXT = table entries per point: 8 for the windows the per-scalar heuristics pick (2..4, ec.rs:895-905, 1586-1596),
 // 64 (K = 1) for the explicit windows 5..7 of wnaf_table / wnaf_exp
 template <class F, bool IS_G2, int K, int MAXT>
@@ -911,10 +903,7 @@ int run_pipelined(bls_ctx* ctx, size_t n, size_t chunk, const PipeIn* in, int n_
 // per SM, pair_io.cuh) -- 18 944 on a B200.  The chunk kernels alternate between two streams (run_pipelined), so a 2^16 batch still
 // runs as 3.46 back-to-back waves, but only the first chunk's H2D (5.8 MB) and the last chunk's D2H are exposed instead of the
 // whole 19.9 MB in and 37.7 MB out.
-#ifndef BLS_PIPE_TWO_STREAMS
-#define BLS_PIPE_TWO_STREAMS 1      /* 0: one kernel stream, one 2^16 launch per chunk (the first build of round 2; kept for A/B runs) */
-#endif
-static size_t pipe_chunk_pairings(const bls_ctx* ctx) { return BLS_PIPE_TWO_STREAMS ? (size_t)ctx->sm_count * 128 : (size_t)1 << 16; }
+static size_t pipe_chunk_pairings(const bls_ctx* ctx) { return (size_t)ctx->sm_count * 128; }
 const size_t PIPE_CHUNK_POINTS = (size_t)1 << 21;
 }  // namespace
 
@@ -940,7 +929,7 @@ static int miller_like(bls_ctx* ctx, const bls_g1_affine* p, const bls_g2_affine
   return run_pipelined(ctx, n, pipe_chunk_pairings(ctx), in, 2, out, sizeof(*out), [&](const void* const* d, void* o, size_t cn, cudaStream_t s) -> int {
     return final_exp ? bls_pairing_dev(ctx, (const bls_g1_affine*)d[0], (const bls_g2_affine*)d[1], (bls_fq12*)o, cn, s)
                      : bls_miller_loop_dev(ctx, (const bls_g1_affine*)d[0], (const bls_g2_affine*)d[1], (bls_fq12*)o, cn, s);
-  }, BLS_PIPE_TWO_STREAMS != 0);
+  }, true);
 }
 int bls_pairing_projective_batch(bls_ctx* ctx, const bls_g1* p, const bls_g2* q, bls_fq12* out, size_t n) {
   if (!ctx || (n && (!p || !q || !out))) return BLS_ERR_INVALID_ARGUMENT;
@@ -1070,7 +1059,7 @@ static int wnaf_host(bls_ctx* ctx, int degree, const void* bases, const bls_fr_r
     else k_pt_mul<Fp, false, BLS_WNAF_K><<<blocks_for((cn + BLS_WNAF_K - 1) / BLS_WNAF_K, TPB), TPB, 0, ks>>>((const uint64_t*)d[0], (const uint64_t*)d[1], (uint64_t*)o, cn);
     LAUNCH_CHECK();
     return BLS_OK;
-  }, BLS_PIPE_TWO_STREAMS != 0);
+  }, true);
 }
 int bls_g1_wnaf_mul_batch(bls_ctx* ctx, const bls_g1* b, const bls_fr_repr* k, bls_g1* out, size_t n) { return wnaf_host(ctx, 1, b, k, out, n, 0, 0); }
 int bls_g2_wnaf_mul_batch(bls_ctx* ctx, const bls_g2* b, const bls_fr_repr* k, bls_g2* out, size_t n) { return wnaf_host(ctx, 2, b, k, out, n, 0, 0); }

@@ -9,21 +9,14 @@
 // count is short (below BLS_MM_SINGLE_VIA_PAIR_BELOW): there the leftover is a seventh of the work and mul_by_014 -- code no other
 // step of the loop executes -- costs 45 % more per product than the pair path (instruction-cache misses); for long trip counts the
 // leftover is negligible and the cheaper 13-product path stays.
-#ifndef BLS_MM_SINGLE_VIA_PAIR_BELOW
 #define BLS_MM_SINGLE_VIA_PAIR_BELOW 32
-#endif
-#ifndef BLS_MM_MINB
 #define BLS_MM_MINB 2      /* blocks per SM of the multi-pairing kernels; 3 (168 registers) measured 3.22 vs 4.87 M pairs/s at 2^20 */
-#endif
 
-// BLS_MM_SMEM = 1: the accumulator f and the three Fq6 temporaries of the products that update it live in SHARED memory (181 words
-// per lane: an odd stride, conflict-free 32-bit accesses; 92.7 KB per block, two blocks per SM) instead of the per-thread stack.
+// The accumulator f and the three Fq6 temporaries of the products that update it live in SHARED memory (181 words per lane: an
+// odd stride, conflict-free 32-bit accesses; 92.7 KB per block, two blocks per SM) instead of the per-thread stack.
 // Why here and not in the fused pairing kernel (DESIGN.md 8.1): this kernel streams 302 MB of running points through L2 per loop
 // bit, next to 73 MB of stack that wants to stay there -- ncu showed 72 GB of the 113 GB of DRAM traffic per 2^20-pair launch to be
 // evicted and re-fetched stack lines.
-#ifndef BLS_MM_SMEM
-#define BLS_MM_SMEM 1
-#endif
 #define BLS_MM_SMEM_WORDS 181   /* P12 (72) + 3 x P6 (108) + 1 */
 struct MmTmp { P6 a, b, s; };
 // fq12.rs:34-48 x 2 (pair_tower.cuh: p12_mul_by_line_pair) with the temporaries supplied by the caller
@@ -77,17 +70,11 @@ __device__ __forceinline__ void mm_sqr(P12& f, MmTmp& t) {
   p6_mul_by_nonresidue(t.a, t.a);
   p6_sub(f.c0, t.s, t.a);
 }
-#if BLS_MM_SMEM
 extern __shared__ __align__(16) uint32_t mm_smem[];
 #define MM_STATE(f, t)                                                                  \
   P12& f = *reinterpret_cast<P12*>(mm_smem + BLS_MM_SMEM_WORDS * threadIdx.x);          \
   MmTmp& t = *reinterpret_cast<MmTmp*>(mm_smem + BLS_MM_SMEM_WORDS * threadIdx.x + 72)
-#else
-#define MM_STATE(f, t) \
-  P12 f;               \
-  MmTmp t
-#endif
-static size_t mm_smem_bytes() { return BLS_MM_SMEM ? (size_t)BLS_MM_SMEM_WORDS * 4 * BLS_PAIR_TPB : 0; }
+static size_t mm_smem_bytes() { return (size_t)BLS_MM_SMEM_WORDS * 4 * BLS_PAIR_TPB; }
 
 // One partial product per BLOCK: the 64 lane pairs of a block fold their accumulators by a shared-memory tree (6 levels of
 // Fq12 products) and lane pair 0 stores the result -- 296 partials per launch instead of 18 944, so that ONE small tail
@@ -96,15 +83,11 @@ static size_t mm_smem_bytes() { return BLS_MM_SMEM ? (size_t)BLS_MM_SMEM_WORDS *
 #define MM_LP (BLS_PAIR_TPB / 2)
 __device__ __forceinline__ void mm_block_reduce_store(const P12& fin, uint64_t* partial) {
   P12 f = fin;                                         // off the shared state area, which the tree is about to reuse
-#if BLS_MM_SMEM
   uint32_t* s_tree = mm_smem;                          // (MM_LP / 2) * 144 words = 18 KB of the 92.7 KB
   __syncthreads();
-#else
-  __shared__ uint32_t s_tree[(MM_LP / 2) * 144];       // at level s the lane pairs [s, 2s) publish, the lane pairs [0, s) multiply
-#endif
   const int lp = threadIdx.x >> 1;
 #pragma unroll 1
-  for (int s = MM_LP / 2; s >= 1; s >>= 1) {
+  for (int s = MM_LP / 2; s >= 1; s >>= 1) {         // at level s the lane pairs [s, 2s) publish, the lane pairs [0, s) multiply
     __syncthreads();
     if (lp >= s && lp < 2 * s) {
       uint32_t* dst = s_tree + (lp - s) * 144 + pair_c() * 72;
@@ -175,39 +158,17 @@ __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_MM_MINB) k_pair_multi_miller
 // touches one contiguous 4608-byte block.  (A word-major array over all n -- plane stride n words -- measured bimodal,
 // 222 or 252 ms per 2^20 pairs from one process to the next.)
 __host__ __device__ __forceinline__ size_t mm_rstate_words(size_t n) { return ((n + 15) / 16) * (36 * 32); }
-// BLS_MM_STREAM = 1 marks these accesses evict-first (ld.global.cs / st.global.cs): the 302 MB of running points of a 2^20
-// batch stream through L2 once per loop iteration and compete with the 62 MB of local memory the kernel keeps there.
-// Unmeasured (default off): an A/B candidate for the two timing modes described in DESIGN.md section 4.
-#ifndef BLS_MM_STREAM
-#define BLS_MM_STREAM 0
-#endif
-// BLS_MM_STREAM = 2: an explicit L2 evict-first policy on the running-point traffic (createpolicy + cache_hint), L1 left alone
-__device__ __forceinline__ uint64_t mm_evict_first_policy() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ uint32_t mm_ld_evict_first(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.global.L2::cache_hint.u32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(mm_evict_first_policy()));
-  return v;
-}
-__device__ __forceinline__ void mm_st_evict_first(uint32_t* p, uint32_t v) {
-  asm volatile("st.global.L2::cache_hint.u32 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(mm_evict_first_policy()) : "memory");
-}
 __device__ __forceinline__ void ld_pjac_blk(PJac& r, const uint32_t* s, size_t pair) {
   uint32_t* w = reinterpret_cast<uint32_t*>(&r);
   const uint32_t* b = s + (pair >> 4) * (36 * 32) + 2 * (pair & 15) + pair_c();
 #pragma unroll
-  for (int k = 0; k < 36; k++) w[k] = BLS_MM_STREAM == 2 ? mm_ld_evict_first(b + k * 32) : BLS_MM_STREAM ? __ldcs(b + k * 32) : b[k * 32];
+  for (int k = 0; k < 36; k++) w[k] = b[k * 32];
 }
 __device__ __forceinline__ void st_pjac_blk(uint32_t* s, size_t pair, const PJac& r) {
   const uint32_t* w = reinterpret_cast<const uint32_t*>(&r);
   uint32_t* b = s + (pair >> 4) * (36 * 32) + 2 * (pair & 15) + pair_c();
 #pragma unroll
-  for (int k = 0; k < 36; k++) {
-    if (BLS_MM_STREAM == 2) mm_st_evict_first(b + k * 32, w[k]); else if (BLS_MM_STREAM) __stcs(b + k * 32, w[k]); else b[k * 32] = w[k];
-  }
+  for (int k = 0; k < 36; k++) b[k * 32] = w[k];
 }
 // one step (phase 0: doubling, phase 1: addition) of pair i's running point, and its line value at P_i
 __device__ __forceinline__ PLine mm_step_line(const uint64_t* p, const uint64_t* q, size_t n, uint32_t* rstate, size_t i, int phase, int b) {
@@ -257,7 +218,7 @@ __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_MM_MINB) k_pair_multi_miller
 
 // more than 48 KB of dynamic shared memory per block needs an opt-in per function and per DEVICE: once per context
 static cudaError_t mm_smem_optin(bls_ctx* ctx) {
-  if (!BLS_MM_SMEM || ctx->mm_smem_ready) return cudaSuccess;
+  if (ctx->mm_smem_ready) return cudaSuccess;
   cudaError_t e = cudaFuncSetAttribute(k_pair_multi_miller, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mm_smem_bytes());
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_pair_multi_miller_prepared, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mm_smem_bytes());
   ctx->mm_smem_ready = e == cudaSuccess;

@@ -18,12 +18,8 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #define MSM_TPB 128
-#ifndef BLS_MSM_MINB_G1
 #define BLS_MSM_MINB_G1 4
-#endif
-#ifndef BLS_MSM_MINB_G2
 #define BLS_MSM_MINB_G2 3
-#endif
 #define MSM_NONE 0xffffffffu              /* key of an empty node */
 #define MSM_SIGN 0x80000000u              /* entry value: point index | sign of the digit */
 #define BLS_MSM_MAX_N ((size_t)1 << 26)   /* and ceil(257 / c) * n < 2^31 (entries are indexed by 32-bit integers) */

@@ -4,12 +4,6 @@
 
 #include "pair_io.cuh"
 
-// BLS_PAIR_SMEM = 1 keeps the Miller accumulator f and the running G2 point R of every lane in shared memory (an odd
-// number of words per lane: conflict-free 32-bit accesses) instead of the per-thread stack.
-#ifndef BLS_PAIR_SMEM
-#define BLS_PAIR_SMEM 0
-#endif
-#define BLS_PAIR_SMEM_WORDS 109   /* P12 (72) + PJac (36) + 1 */
 template <bool FINAL_EXP>
 __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_PAIR_MINB) k_pair_miller(const uint64_t* p, const uint64_t* q, uint64_t* out, size_t n) {
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -21,16 +15,8 @@ __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_PAIR_MINB) k_pair_miller(con
   const bool live = pi[12] == 0 && qi[24] == 0;
   Fp px = ld_fp(pi), py = ld_fp(pi + 6);
   P2 qx = ld_p2(qi), qy = ld_p2(qi + 12);
-#if BLS_PAIR_SMEM
-  extern __shared__ uint32_t pair_smem[];
-  uint32_t* slot = pair_smem + BLS_PAIR_SMEM_WORDS * threadIdx.x;
-  P12& f = *reinterpret_cast<P12*>(slot);
-  PJac& r = *reinterpret_cast<PJac*>(slot + 72);
-  p_miller_loop_single(f, r, px, py, qx, qy);
-#else
   P12 f;
   p_miller_loop_single(f, px, py, qx, qy);
-#endif
   if (!live) p12_one(f);                       // mod.rs:49-54: skipped pair, f stays one
   if (FINAL_EXP) {
     P12 g;
@@ -39,13 +25,6 @@ __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_PAIR_MINB) k_pair_miller(con
   } else {
     if (active) st_p12(out + FQ12_W * i, f);
   }
-}
-static size_t pair_miller_smem_bytes() { return BLS_PAIR_SMEM ? (size_t)BLS_PAIR_SMEM_WORDS * 4 * BLS_PAIR_TPB : 0; }
-template <bool FE> static cudaError_t pair_miller_smem_optin() {
-  static bool done = false;      // per process; the attribute is per function and idempotent
-  if (done || !BLS_PAIR_SMEM) return cudaSuccess;
-  done = true;
-  return cudaFuncSetAttribute(k_pair_miller<FE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pair_miller_smem_bytes());
 }
 
 __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_PAIR_MINB) k_pair_g2_prepare(const uint64_t* q, uint64_t* out, size_t n) {
@@ -326,8 +305,7 @@ int bls_miller_loop_dev(bls_ctx* ctx, const bls_g1_affine* p, const bls_g2_affin
   if (!n) return BLS_OK;
   USE_DEVICE(ctx);
   if (n <= ctx->wide_pairing_max) return bls_internal_wide_miller(ctx, p, q, out, n, pick(ctx, stream));
-  CK(pair_miller_smem_optin<false>());
-  k_pair_miller<false><<<blocks_for(2 * n, BLS_PAIR_TPB), BLS_PAIR_TPB, pair_miller_smem_bytes(), pick(ctx, stream)>>>((const uint64_t*)p, (const uint64_t*)q, (uint64_t*)out, n);
+  k_pair_miller<false><<<blocks_for(2 * n, BLS_PAIR_TPB), BLS_PAIR_TPB, 0, pick(ctx, stream)>>>((const uint64_t*)p, (const uint64_t*)q, (uint64_t*)out, n);
   LAUNCH_CHECK();
   return BLS_OK;
 }
@@ -353,8 +331,7 @@ int bls_pairing_dev(bls_ctx* ctx, const bls_g1_affine* p, const bls_g2_affine* q
   if (!n) return BLS_OK;
   USE_DEVICE(ctx);
   if (n <= ctx->wide_pairing_max) return bls_internal_wide_pairing(ctx, p, q, out, n, pick(ctx, stream));
-  CK(pair_miller_smem_optin<true>());
-  k_pair_miller<true><<<blocks_for(2 * n, BLS_PAIR_TPB), BLS_PAIR_TPB, pair_miller_smem_bytes(), pick(ctx, stream)>>>((const uint64_t*)p, (const uint64_t*)q, (uint64_t*)out, n);
+  k_pair_miller<true><<<blocks_for(2 * n, BLS_PAIR_TPB), BLS_PAIR_TPB, 0, pick(ctx, stream)>>>((const uint64_t*)p, (const uint64_t*)q, (uint64_t*)out, n);
   LAUNCH_CHECK();
   return BLS_OK;
 }

@@ -20,12 +20,8 @@ __device__ __forceinline__ void st_p12(uint64_t* p, const P12& a) {
 
 // launch shape of the lane-pair kernels: BLS_PAIR_TPB threads per block, BLS_PAIR_MINB blocks per SM
 // (registers per thread <= 65536 / (TPB * MINB)).  Small blocks keep the tail of a 2^16 batch short.
-#ifndef BLS_PAIR_TPB
 #define BLS_PAIR_TPB 128
-#endif
-#ifndef BLS_PAIR_MINB
 #define BLS_PAIR_MINB 2
-#endif
 
 // line coefficients of a pair that does not count (infinity member, past the end): the sparse element one
 __device__ __forceinline__ void pcoeffs_set_one_if(bool dead, PCoeffs& c) {

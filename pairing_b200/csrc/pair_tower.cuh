@@ -352,10 +352,11 @@ static __device__ __noinline__ void p12_mul_by_line_pair(P12& f, const PLine& l,
 // mod.rs:40-102 for one pair, G2 steps on the fly
 // (no early exit for pairs with an infinity member: every lane must reach every shuffle; the
 // caller overwrites f with one for those pairs)
-__device__ __forceinline__ void p_miller_loop_single(P12& f, PJac& r, const Fp& px, const Fp& py, const P2& qx, const P2& qy) {
+__device__ __forceinline__ void p_miller_loop_single(P12& f, const Fp& px, const Fp& py, const P2& qx, const P2& qy) {
   p12_one(f);
-  r.x = qx; r.y = qy; r.z = p2_one();
   PCoeffs c;
+  PJac r;
+  r.x = qx; r.y = qy; r.z = p2_one();
 #pragma unroll 1
   for (int b = BLS_LOOP_TOP; b >= 0; b--) {
     pg2_doubling_step(r, c);
@@ -369,10 +370,6 @@ __device__ __forceinline__ void p_miller_loop_single(P12& f, PJac& r, const Fp& 
   pg2_doubling_step(r, c);
   p_ell(f, c, px, py);
   p12_conjugate(f);
-}
-__device__ __forceinline__ void p_miller_loop_single(P12& f, const Fp& px, const Fp& py, const P2& qx, const P2& qy) {
-  PJac r;
-  p_miller_loop_single(f, r, px, py, qx, qy);
 }
 
 // exp_by_x (mod.rs:116-121): Field::pow(&[x]) (lib.rs:306-324) followed by a conjugation.  Two value-preserving
@@ -415,14 +412,12 @@ static __device__ __noinline__ void pk4_sqr(PK4& c) {
   P2 z5 = p2_add(t3, c.g5); z5 = p2_add(p2_dbl(z5), t3);
   c.g2 = z2; c.g3 = z3; c.g4 = z4; c.g5 = z5;
 }
-// BLS_EXP_NCOMP: how many of the set bits (from the low end) are reached by compressed squarings.  3 (default): the powers at
+// BLS_EXP_NCOMP: how many of the set bits (from the low end) are reached by compressed squarings.  3: the powers at
 // bits 16, 48, 57 are decompressed and the three close bits above (60, 62, 63) are reached from the decompressed a^(2^57) by six
 // uncompressed cyclotomic squarings -- 12 Fq2 products fewer per call than decompressing all six powers (BLS_EXP_NCOMP = 6) and
 // half the stored powers: 42.6 - 43.4 ms against 45.4 ms per 2^16 pairings for 6 in this code shape (4: 43.4 - 44.1 ms), same GPU call;
 // the earlier all-six build measured 43.1 - 44.6 ms over its boxes, this one 42.6 - 44.0 ms.
-#ifndef BLS_EXP_NCOMP
 #define BLS_EXP_NCOMP 3
-#endif
 static __device__ __noinline__ void p12_exp_by_x_compressed(P12& out, const P12& a, uint64_t x) {
   PK4 pts[BLS_EXP_NCOMP];
   P2 pre[BLS_EXP_NCOMP];
@@ -473,16 +468,6 @@ static __device__ __noinline__ void p12_exp_by_x_compressed(P12& out, const P12&
   }
   out = res;
 }
-#ifndef BLS_EXP_COMPRESSED
-#define BLS_EXP_COMPRESSED 1
-#endif
-__device__ __forceinline__ void p12_exp_by_x_hard(P12& out, const P12& a, uint64_t x) {
-#if BLS_EXP_COMPRESSED
-  p12_exp_by_x_compressed(out, a, x);
-#else
-  p12_exp_by_x(out, a, x);
-#endif
-}
 
 // both lanes learn whether the Fq12 value is zero
 __device__ __forceinline__ bool p12_is_zero(const P12& a) {
@@ -493,12 +478,10 @@ __device__ __forceinline__ bool p12_is_zero(const P12& a) {
 }
 
 // mod.rs:104-160
-// BLS_Y0_CYCLOTOMIC_SQR = 1 squares r with the 6-product cyclotomic routine instead of the generic 12-product one (the same
-// value).  Off: under bench.py's conditions (L2 flushed between launches) the fused kernel measured 45.3 - 45.5 ms with it and
-// 43.1 - 44.6 ms without, three boxes; back to back without the flush the two builds are equal (43.2 ms).
-#ifndef BLS_Y0_CYCLOTOMIC_SQR
-#define BLS_Y0_CYCLOTOMIC_SQR 0
-#endif
+// y0 = r^2 by the generic 12-product squaring.  The 6-product cyclotomic squaring gives the same value (r is in the cyclotomic
+// subgroup after the easy part) but lost: under bench.py's conditions (L2 flushed between launches) the fused kernel measured
+// 45.3 - 45.5 ms with it and 43.1 - 44.6 ms without, three boxes; back to back without the flush the two builds are equal
+// (43.2 ms).  That variant was removed; it can be recovered from git history at commit 7b088bd.
 __device__ __forceinline__ bool p_final_exponentiation(P12& out, const P12& in) {
   P12 f1 = in, f2, r;
   p12_conjugate(f1);
@@ -509,26 +492,22 @@ __device__ __forceinline__ bool p_final_exponentiation(P12& out, const P12& in) 
   p12_mul(r, r, f2);
   const uint64_t x = BLS_X_ABS;
   P12 y0, y1, y2, y3;
-#if BLS_Y0_CYCLOTOMIC_SQR
-  p12_cyclotomic_sqr(y0, r);          // r is in the cyclotomic subgroup after the easy part: the same value as `square`
-#else
   p12_sqr(y0, r);
-#endif
-  p12_exp_by_x_hard(y1, y0, x);
-  p12_exp_by_x_hard(y2, y1, x >> 1);
+  p12_exp_by_x_compressed(y1, y0, x);
+  p12_exp_by_x_compressed(y2, y1, x >> 1);
   y3 = r; p12_conjugate(y3);
   p12_mul(y1, y1, y3);
   p12_conjugate(y1);
   p12_mul(y1, y1, y2);
-  p12_exp_by_x_hard(y2, y1, x);
-  p12_exp_by_x_hard(y3, y2, x);
+  p12_exp_by_x_compressed(y2, y1, x);
+  p12_exp_by_x_compressed(y3, y2, x);
   p12_conjugate(y1);
   p12_mul(y3, y3, y1);
   p12_conjugate(y1);
   p12_frobenius(y1, y1, 3);
   p12_frobenius(y2, y2, 2);
   p12_mul(y1, y1, y2);
-  p12_exp_by_x_hard(y2, y3, x);
+  p12_exp_by_x_compressed(y2, y3, x);
   p12_mul(y2, y2, y0);
   p12_mul(y2, y2, r);
   p12_mul(y1, y1, y2);

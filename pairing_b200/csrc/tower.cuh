@@ -52,43 +52,13 @@ __device__ __forceinline__ Fp2 fp2_mul_fp(const Fp2& a, const Fp& s) { return Fp
 
 // Fq inversion (fq.rs:849-902).  The reference runs a binary extended Euclid; the inverse is unique and the result is
 // canonical, so the algorithm is free: Bernstein-Yang division steps on signed 30-bit limbs (fp_inv_gcd.cuh), about a
-// tenth of the multiplier work of the Fermat power a^(q-2) that round 1 used (kept under -DBLS_FP_INV_FERMAT=1 for A/B
-// measurements).  Returns false (and zero) for a == 0, the reference's `None`.
-#ifndef BLS_FP_INV_FERMAT
-#define BLS_FP_INV_FERMAT 0
-#endif
-#if !BLS_FP_INV_FERMAT
+// tenth of the multiplier work of the Fermat power a^(q-2) that round 1 used (removed; it can be recovered from git history
+// at commit 7b088bd).  Returns false (and zero) for a == 0, the reference's `None`.
 static __device__ __noinline__ bool fp_inv(Fp& out, const Fp& a) {
   const Fp c = fp_canon(a);
   gcd30::invert_words(out.v, c.v);
   return !fp_is_zero_raw(c);
 }
-#else
-// a^(q-2) by a fixed 4-bit window over the (compile-time) exponent
-static __device__ __noinline__ bool fp_inv(Fp& out, const Fp& a) {
-  if (fp_is_zero(a)) { out = fp_zero(); return false; }
-  Fp tbl[16];
-  tbl[0] = fp_one();
-  tbl[1] = a;
-#pragma unroll 1
-  for (int i = 2; i < 16; i++) tbl[i] = fp_mul(tbl[i - 1], a);
-  // q - 2, most significant nibble first (96 nibbles)
-  const uint32_t e[12] = {BLS_Q0 - 2u, BLS_Q1, BLS_Q2, BLS_Q3, BLS_Q4, BLS_Q5, BLS_Q6, BLS_Q7, BLS_Q8, BLS_Q9, BLS_Q10, BLS_Q11};
-  Fp r = fp_one();
-  bool started = false;
-#pragma unroll 1
-  for (int i = 95; i >= 0; i--) {
-    uint32_t nib = (e[i >> 3] >> ((i & 7) * 4)) & 0xf;
-    if (started) { r = fp_sqr(r); r = fp_sqr(r); r = fp_sqr(r); r = fp_sqr(r); }
-    if (nib) {
-      r = started ? fp_mul(r, tbl[nib]) : tbl[nib];
-      started = true;
-    }
-  }
-  out = r;
-  return true;
-}
-#endif
 
 // fq2.rs:138-155
 __device__ __forceinline__ bool fp2_inv(Fp2& out, const Fp2& a) {

@@ -9,12 +9,17 @@ fn main() {
     let root = PathBuf::from(env::var("CARGO_MANIFEST_DIR").unwrap()).join("..");
     let lib = out.join("libpairing_b200.a");
     let nvcc = env::var("NVCC").unwrap_or_else(|_| "/usr/local/cuda/bin/nvcc".into());
-    // four translation units: the lane-pair pairing engine and the warp-cooperative engine are compiled on their own
-    // (pairing_b200/csrc/abi_common.cuh); mgpu.cu is the host-side multi-device layer
+    // every .cu of the source directory is a translation unit of its own (pairing_b200/csrc/abi_common.cuh)
+    let csrc = root.join("pairing_b200/csrc");
+    let mut srcs: Vec<PathBuf> = std::fs::read_dir(&csrc)
+        .expect("pairing_b200/csrc")
+        .map(|e| e.expect("pairing_b200/csrc").path())
+        .filter(|p| p.extension().map_or(false, |x| x == "cu"))
+        .collect();
+    srcs.sort();
     let mut objs = Vec::new();
-    for unit in &["kernels", "kernels_pair", "kernels_mm", "kernels_wide", "mgpu"] {
-        let src = root.join(format!("pairing_b200/csrc/{}.cu", unit));
-        let obj = out.join(format!("{}.o", unit));
+    for src in &srcs {
+        let obj = out.join(src.file_stem().unwrap()).with_extension("o");
         let status = Command::new(&nvcc)
             .args(&["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
                     "-Xcompiler", "-fPIC", "-c", "-o"])
@@ -33,9 +38,6 @@ fn main() {
     println!("cargo:rustc-link-lib=dylib=cudart");
     println!("cargo:rustc-link-lib=dylib=stdc++");
     println!("cargo:rustc-link-lib=dylib=pthread");
-    for f in &["kernels.cu", "kernels_pair.cu", "kernels_mm.cu", "kernels_wide.cu", "mgpu.cu", "abi_common.cuh", "pair_io.cuh", "fr.cuh", "fp.cuh", "fp_inv_gcd.cuh", "fp_sqr_gen.cuh", "tower.cuh", "curve.cuh",
-               "pair_tower.cuh", "wide.cuh", "wide_prog_gen.cuh", "codec.cuh", "constants.cuh"] {
-        println!("cargo:rerun-if-changed={}", root.join("pairing_b200/csrc").join(f).display());
-    }
+    println!("cargo:rerun-if-changed={}", csrc.display());
     println!("cargo:rerun-if-changed={}", root.join("include/pairing_b200.h").display());
 }
