@@ -208,6 +208,18 @@ int bls_pair_field_op_dev(bls_ctx*, int degree, int op, const void* a, const voi
  * FROM_REPR (bls_fr_repr -> bls_fr; ok = 0 for values >= r) / INTO_REPR (bls_fr -> bls_fr_repr).  The step after the
  * path: callers combine scalars (c * d in the reference's bilinearity test, tests/engine.rs:117-119). */
 int bls_fr_op_batch(bls_ctx*, int op, const bls_fr* a, const bls_fr* b, bls_fr* out, uint8_t* ok, size_t n);
+/* Radix-2 FFT over Fr for m polynomials of n = 2^log_n coefficients each, back to back (m * n bls_fr, natural order in
+ * and out): bellman's EvaluationDomain with the crate's constants (fr.rs: S = 32, multiplicative_generator() g = 7,
+ * root_of_unity() = 7^t, r - 1 = t * 2^32), omega = root_of_unity() squared (32 - log_n) times.  For i < n:
+ *   BLS_FFT         out[i] = sum_j a_j omega^(ij)
+ *   BLS_IFFT        out[i] = n^-1 sum_j a_j omega^(-ij)
+ *   BLS_COSET_FFT   out[i] = sum_j a_j (g omega^i)^j              (distribute_powers(g), then fft)
+ *   BLS_ICOSET_FFT  out[i] = g^-i n^-1 sum_j a_j omega^(-ij)      (ifft, then distribute_powers(g^-1))
+ * Inputs must be canonical (< r); outputs are canonical.  in == out (in place) is allowed, otherwise the buffers must not
+ * overlap and `in` is left unchanged.  m = 0 does nothing.  log_n in 0..28 and m * 2^log_n <= 2^30, kind in 0..3, else
+ * BLS_ERR_INVALID_ARGUMENT. */
+enum { BLS_FFT = 0, BLS_IFFT = 1, BLS_COSET_FFT = 2, BLS_ICOSET_FFT = 3 };
+int bls_fr_fft_batch(bls_ctx*, int kind, const bls_fr* in, bls_fr* out, int log_n, size_t m);
 
 /* ------------------------------------------------------------------ device-pointer variants
  * Same semantics; every pointer is a device pointer on the context's device, the work is enqueued
@@ -251,6 +263,11 @@ int bls_g2_batch_normalization_dev(bls_ctx*, bls_g2* inout, size_t n, void* scra
 size_t bls_msm_scratch_bytes(const bls_ctx*, int degree, size_t n, int window);
 int bls_g1_msm_dev(bls_ctx*, const bls_g1_affine* bases, const bls_fr_repr* k, size_t n, int window, bls_g1* out1, void* scratch, void* stream);
 int bls_g2_msm_dev(bls_ctx*, const bls_g2_affine* bases, const bls_fr_repr* k, size_t n, int window, bls_g2* out1, void* scratch, void* stream);
+/* bls_fr_fft_batch on device pointers, same arguments and limits.  scratch: bls_fr_fft_scratch_bytes(ctx, log_n, m)
+ * bytes (0 for invalid arguments; the same for every kind); it holds the twiddle tables the call builds and, for
+ * log_n > 10, one buffer of m * 2^log_n elements between passes: the call allocates nothing. */
+size_t bls_fr_fft_scratch_bytes(const bls_ctx*, int log_n, size_t m);
+int bls_fr_fft_dev(bls_ctx*, int kind, const bls_fr* in, bls_fr* out, int log_n, size_t m, void* scratch, void* stream);
 
 /* ------------------------------------------------------------------ several GPUs behind ONE call
  * Engine::miller_loop takes ALL pairs of a product in one call (mod.rs:40-102), and a Rust / C caller is one process.

@@ -255,6 +255,17 @@ struct FrField {
   static std::vector<Elem> double_(Gpu& g, const std::vector<Elem>& a) { return op(g, BLS_OP_DBL, a, nullptr); }
   // Field::inverse: ok[i] == 0 is the reference's None (zero has no inverse)
   static std::vector<Elem> inverse(Gpu& g, const std::vector<Elem>& a, std::vector<uint8_t>* ok = nullptr) { return op(g, BLS_OP_INV, a, nullptr, ok); }
+  // bellman's EvaluationDomain over Fr: a.size() = m * 2^log_n coefficients of m polynomials back to back, natural order
+  static std::vector<Elem> transform(Gpu& g, int kind, const std::vector<Elem>& a, int log_n) {
+    if (log_n < 0 || log_n > 28 || a.size() % (size_t(1) << log_n)) throw std::invalid_argument("FrField: a.size() is not a multiple of 2^log_n");
+    std::vector<Elem> out(a.size());
+    g.check(bls_fr_fft_batch(g.ctx(), kind, a.data(), out.data(), log_n, a.size() >> log_n));
+    return out;
+  }
+  static std::vector<Elem> fft(Gpu& g, const std::vector<Elem>& a, int log_n) { return transform(g, BLS_FFT, a, log_n); }
+  static std::vector<Elem> ifft(Gpu& g, const std::vector<Elem>& a, int log_n) { return transform(g, BLS_IFFT, a, log_n); }
+  static std::vector<Elem> coset_fft(Gpu& g, const std::vector<Elem>& a, int log_n) { return transform(g, BLS_COSET_FFT, a, log_n); }
+  static std::vector<Elem> icoset_fft(Gpu& g, const std::vector<Elem>& a, int log_n) { return transform(g, BLS_ICOSET_FFT, a, log_n); }
 };
 
 // ------------------------------------------------------------------------------------------------ curves

@@ -19,6 +19,7 @@ OPS = dict(add=0, sub=1, mul=2, sqr=3, neg=4, dbl=5, inv=6, from_repr=7, into_re
            frob1=10, frob2=11, frob3=12, conj=13, mul_by_014=14, mul_by_01=15, mul_by_1=16, sqrt=17,
            mul_by_line_pair=18, cyclotomic_sqr=19)
 PT_OPS = dict(double=0, add=1, add_mixed=2, negate=3, sub=6)
+FFT_KINDS = dict(fft=0, ifft=1, coset_fft=2, icoset_fft=3)
 
 # every symbol include/pairing_b200.h declares (tests/test_abi.py checks the header against this list)
 SYMBOLS = [
@@ -49,6 +50,7 @@ SYMBOLS = [
     "bls_mgpu_pairing_product", "bls_mgpu_pairing_batch", "bls_mgpu_g1_wnaf_mul_batch", "bls_mgpu_g2_wnaf_mul_batch",
     "bls_mgpu_last_phase_ms",
     "bls_g1_msm", "bls_g2_msm", "bls_msm_scratch_bytes", "bls_g1_msm_dev", "bls_g2_msm_dev",
+    "bls_fr_fft_batch", "bls_fr_fft_scratch_bytes", "bls_fr_fft_dev",
 ]
 
 
@@ -90,6 +92,8 @@ def load():
     lib.bls_batch_normalization_scratch_bytes.argtypes = [vp, ci, sz]
     lib.bls_msm_scratch_bytes.restype = sz
     lib.bls_msm_scratch_bytes.argtypes = [vp, ci, sz, ci]
+    lib.bls_fr_fft_scratch_bytes.restype = sz
+    lib.bls_fr_fft_scratch_bytes.argtypes = [vp, ci, sz]
     sig = {
         "bls_g2_prepare_batch": [vp, vp, vp, sz],
         "bls_miller_loop_batch": [vp, vp, vp, vp, sz],
@@ -165,6 +169,8 @@ def load():
         "bls_g2_msm": [vp, vp, vp, sz, vp],
         "bls_g1_msm_dev": [vp, vp, vp, sz, ci, vp, vp, vp],
         "bls_g2_msm_dev": [vp, vp, vp, sz, ci, vp, vp, vp],
+        "bls_fr_fft_batch": [vp, ci, vp, vp, ci, sz],
+        "bls_fr_fft_dev": [vp, ci, vp, vp, ci, sz, vp, vp],
     }
     lib.bls_mgpu_create.restype = vp
     lib.bls_mgpu_create.argtypes = [ctypes.POINTER(ci), ci, ctypes.POINTER(ci)]
@@ -524,6 +530,29 @@ class Context:
         ok = np.zeros(a.shape[0], dtype=np.uint8)
         self._check(self._lib.bls_fr_op_batch(self._ctx, OPS[op], _p(a), _p(b) if b is not None else None, _p(out), _p(ok), a.shape[0]))
         return out, ok
+
+    def fr_fft(self, kind, a):
+        """bellman's EvaluationDomain transforms over Fr: kind "fft" | "ifft" | "coset_fft" | "icoset_fft" on one
+        polynomial (n, 4) or m polynomials (m, n, 4) of Montgomery-form values, n a power of two -> same shape."""
+        kind = FFT_KINDS[kind]
+        a = np.ascontiguousarray(a, dtype=np.uint64)
+        if a.ndim not in (2, 3) or a.shape[-1] != W_FR:
+            raise ValueError("a must have shape (n, 4) or (m, n, 4) uint64, got %r" % (a.shape,))
+        n = a.shape[-2]
+        log_n = n.bit_length() - 1
+        if n != 1 << log_n:
+            raise ValueError("the polynomial length must be a power of two, got %d" % n)
+        m = a.shape[0] if a.ndim == 3 else 1
+        out = np.zeros_like(a)
+        self._check(self._lib.bls_fr_fft_batch(self._ctx, kind, _p(a), _p(out), log_n, m))
+        return out
+
+    def fr_fft_scratch_bytes(self, log_n, m=1):
+        """device scratch of bls_fr_fft_dev for m polynomials of 2^log_n; raises for arguments the call would reject"""
+        b = int(self._lib.bls_fr_fft_scratch_bytes(self._ctx, log_n, m))
+        if b == 0:
+            raise ValueError("no FFT of log_n = %d, m = %d" % (log_n, m))
+        return b
 
     def call_dev(self, name, *args):
         """Raw access to a `*_dev` entry point: args are ints (device pointers / sizes / stream)."""

@@ -174,6 +174,25 @@ class DeviceEngine:
                           scr.data_ptr(), self._stream())
         return out
 
+    def fr_fft(self, a, kind="fft", out=None):
+        """bellman's EvaluationDomain transforms over Fr on the device: kind "fft" | "ifft" | "coset_fft" | "icoset_fft"
+        on one polynomial (n, 4) or m polynomials (m, n, 4) of Montgomery-form values, n a power of two.  out may be a
+        (contiguous, same-shape) tensor, `a` itself included (in place)."""
+        if not (a.is_cuda and a.dtype == torch.int64 and a.dim() in (2, 3) and a.shape[-1] == nat.W_FR and a.is_contiguous()):
+            raise ValueError("a must be a contiguous CUDA int64 tensor of shape (n, 4) or (m, n, 4)")
+        n = a.shape[-2]
+        log_n = n.bit_length() - 1
+        if n != 1 << log_n:
+            raise ValueError("the polynomial length must be a power of two, got %d" % n)
+        m = a.shape[0] if a.dim() == 3 else 1
+        if out is None:
+            out = torch.empty_like(a)
+        elif not (out.is_cuda and out.dtype == torch.int64 and out.shape == a.shape and out.is_contiguous()):
+            raise ValueError("out must be a contiguous CUDA int64 tensor of shape %r" % (tuple(a.shape),))
+        scr = self._buf("fft", self.ctx.fr_fft_scratch_bytes(log_n, m))
+        self.ctx.call_dev("bls_fr_fft_dev", nat.FFT_KINDS[kind], a.data_ptr(), out.data_ptr(), log_n, m, scr.data_ptr(), self._stream())
+        return out
+
     def wnaf_table(self, base, window, g2=False):
         """Wnaf::base(g, n): the shared window table (2^(window-1), W) on the device."""
         w = nat.W_G2 if g2 else nat.W_G1

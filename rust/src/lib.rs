@@ -15,7 +15,7 @@
 pub mod ffi;
 
 use self::ffi::*;
-use crate::bls12_381::{Fq12, FrRepr, G1Affine, G2Affine, G1, G2};
+use crate::bls12_381::{Fq12, Fr, FrRepr, G1Affine, G2Affine, G1, G2};
 use std::sync::Mutex;
 
 #[derive(Debug)]
@@ -132,6 +132,17 @@ impl Gpu {
         Ok(marshal::g1_back(&out))
     }
 
+    /// bellman's `EvaluationDomain` transforms over `Fr` for `a.len() / 2^log_n` polynomials back to back, natural order:
+    /// kind 0 `fft`, 1 `ifft`, 2 `coset_fft`, 3 `icoset_fft` (`BLS_FFT` ... in the C header).
+    pub fn fr_fft(&self, kind: i32, a: &[Fr], log_n: u32) -> Result<Vec<Fr>, GpuError> {
+        assert!(log_n <= 28 && a.len() % (1usize << log_n) == 0);
+        let aa: Vec<bls_fr_repr> = a.iter().map(marshal::fr).collect();
+        let mut out = vec![bls_fr_repr { l: [0; 4] }; a.len()];
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_fr_fft_batch(*ctx, kind, aa.as_ptr(), out.as_mut_ptr(), log_n as i32, a.len() >> log_n) }, *ctx)?;
+        Ok(out.iter().map(marshal::fr_back).collect())
+    }
+
     /// `let q = Q.prepare(); ps.iter().map(|p| Bls12::pairing(p, Q))` with the one `G2Prepared` staged on the device.
     pub fn pairing_shared_q(&self, p: &[G1Affine], q: &G2Affine) -> Result<Vec<Fq12>, GpuError> {
         let pp: Vec<bls_g1_affine> = p.iter().map(marshal::g1_affine).collect();
@@ -184,6 +195,9 @@ mod marshal {
     // (two one-line additions to fq.rs) so that no Montgomery conversion happens at the boundary.
     pub fn fq(x: &Fq) -> bls_fq { bls_fq { l: x.mont_limbs() } }
     pub fn fq_back(x: &bls_fq) -> Fq { Fq::from_mont_limbs(x.l) }
+    // `Fr(FrRepr)` in Montgomery form (fr.rs:54-58), through the same kind of accessors on fr.rs
+    pub fn fr(x: &Fr) -> bls_fr_repr { bls_fr_repr { l: x.mont_limbs() } }
+    pub fn fr_back(x: &bls_fr_repr) -> Fr { Fr::from_mont_limbs(x.l) }
     pub fn fq2(x: &Fq2) -> bls_fq2 { bls_fq2 { c0: fq(&x.c0), c1: fq(&x.c1) } }
     pub fn fq2_back(x: &bls_fq2) -> Fq2 { Fq2 { c0: fq_back(&x.c0), c1: fq_back(&x.c1) } }
     pub fn fq6(x: &Fq6) -> bls_fq6 { bls_fq6 { c0: fq2(&x.c0), c1: fq2(&x.c1), c2: fq2(&x.c2) } }
