@@ -157,6 +157,15 @@ int bls_g2_op_batch(bls_ctx*, int op, const bls_g2* a, const void* b, bls_g2* ou
  * n is at most 2^26 (BLS_ERR_INVALID_ARGUMENT above). */
 int bls_g1_msm(bls_ctx*, const bls_g1_affine* bases, const bls_fr_repr* k, size_t n, bls_g1* out1);
 int bls_g2_msm(bls_ctx*, const bls_g2_affine* bases, const bls_fr_repr* k, size_t n, bls_g2* out1);
+/* m independent sums in one call: out[j] = sum_{i<n} k[j*n + i] * bases[b(j, i)] for j < m, where b(j, i) = i if
+ * shared_bases != 0 (one set of n bases for every sum: one SRS or proving key) and j*n + i otherwise (m sets of n bases back
+ * to back: the different base sets of one proof).  Each out[j] is exactly what bls_g*_msm returns for its n bases and
+ * scalars: full 256-bit FrRepr scalars, infinity bases and zero scalars contribute nothing, the normalised representative is
+ * stored.  n = 0 stores m zeros; m = 0 does nothing.  Sums of different lengths are padded with zero scalars: a zero digit
+ * costs sort work but no addition.  m <= 2^16 and m * n <= 2^26, else BLS_ERR_INVALID_ARGUMENT.  A loop of m bls_g*_msm
+ * calls pays the latency of the reduction m times; one batch pays it once. */
+int bls_g1_msm_batch(bls_ctx*, const bls_g1_affine* bases, int shared_bases, const bls_fr_repr* k, size_t n, size_t m, bls_g1* out);
+int bls_g2_msm_batch(bls_ctx*, const bls_g2_affine* bases, int shared_bases, const bls_fr_repr* k, size_t n, size_t m, bls_g2* out);
 
 /* ------------------------------------------------------------------ point encodings (host buffers)
  * EncodedPoint::into_affine (checked != 0: on-curve and r-order-subgroup checks) / into_affine_unchecked and
@@ -263,6 +272,13 @@ int bls_g2_batch_normalization_dev(bls_ctx*, bls_g2* inout, size_t n, void* scra
 size_t bls_msm_scratch_bytes(const bls_ctx*, int degree, size_t n, int window);
 int bls_g1_msm_dev(bls_ctx*, const bls_g1_affine* bases, const bls_fr_repr* k, size_t n, int window, bls_g1* out1, void* scratch, void* stream);
 int bls_g2_msm_dev(bls_ctx*, const bls_g2_affine* bases, const bls_fr_repr* k, size_t n, int window, bls_g2* out1, void* scratch, void* stream);
+/* bls_g*_msm_batch on device pointers; out holds m device points.  window as for bls_g*_msm_dev, with W = ceil(257 / c):
+ * m <= 2^16, m * n <= 2^26, W * m * n < 2^31 and m * W * 2^(c-1) < 2^31, else BLS_ERR_INVALID_ARGUMENT; window = 0 is
+ * valid for every such m and n.  scratch: bls_msm_batch_scratch_bytes(ctx, degree, n, m, window) bytes (0 for invalid
+ * arguments); bls_msm_scratch_bytes(ctx, degree, n, window) equals it for m = 1, and bls_g*_msm_dev is the m = 1 call. */
+size_t bls_msm_batch_scratch_bytes(const bls_ctx*, int degree, size_t n, size_t m, int window);
+int bls_g1_msm_batch_dev(bls_ctx*, const bls_g1_affine* bases, int shared_bases, const bls_fr_repr* k, size_t n, size_t m, int window, bls_g1* out, void* scratch, void* stream);
+int bls_g2_msm_batch_dev(bls_ctx*, const bls_g2_affine* bases, int shared_bases, const bls_fr_repr* k, size_t n, size_t m, int window, bls_g2* out, void* scratch, void* stream);
 /* bls_fr_fft_batch on device pointers, same arguments and limits.  scratch: bls_fr_fft_scratch_bytes(ctx, log_n, m)
  * bytes (0 for invalid arguments; the same for every kind); it holds the twiddle tables the call builds and, for
  * log_n > 10, one buffer of m * 2^log_n elements between passes: the call allocates nothing. */

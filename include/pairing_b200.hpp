@@ -355,6 +355,18 @@ template <class Proj, class Aff, bool IS_G2> struct Curve {
     else g.check(bls_g1_msm(g.ctx(), bases.data(), k.data(), bases.size(), &out));
     return out;
   }
+  // m independent multiexp sums in one call: sum j = sum_i k[j*n + i] * bases[b(j, i)], n = k.size() / m, with
+  // b(j, i) = i when bases.size() == n (one set for every sum) and j*n + i when bases.size() == k.size()
+  static std::vector<Proj> multiexp_batch(Gpu& g, const std::vector<Aff>& bases, const std::vector<FrRepr>& k, size_t m) {
+    if (m == 0 ? !k.empty() : k.size() % m != 0) throw Error(BLS_ERR_INVALID_ARGUMENT, "multiexp_batch: k.size() is not a multiple of m");
+    const size_t n = m ? k.size() / m : 0;
+    if (bases.size() != n && bases.size() != k.size()) throw Error(BLS_ERR_INVALID_ARGUMENT, "multiexp_batch: bases.size() is neither k.size() / m nor k.size()");
+    const int shared = bases.size() == n;
+    std::vector<Proj> out(m);
+    if constexpr (IS_G2) g.check(bls_g2_msm_batch(g.ctx(), bases.data(), shared, k.data(), n, m, out.data()));
+    else g.check(bls_g1_msm_batch(g.ctx(), bases.data(), shared, k.data(), n, m, out.data()));
+    return out;
+  }
   // From<affine> for projective (ec.rs:570-582)
   static std::vector<Proj> into_projective(const std::vector<Aff>& a) {
     std::vector<Proj> out(a.size());

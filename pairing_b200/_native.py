@@ -50,6 +50,7 @@ SYMBOLS = [
     "bls_mgpu_pairing_product", "bls_mgpu_pairing_batch", "bls_mgpu_g1_wnaf_mul_batch", "bls_mgpu_g2_wnaf_mul_batch",
     "bls_mgpu_last_phase_ms",
     "bls_g1_msm", "bls_g2_msm", "bls_msm_scratch_bytes", "bls_g1_msm_dev", "bls_g2_msm_dev",
+    "bls_g1_msm_batch", "bls_g2_msm_batch", "bls_msm_batch_scratch_bytes", "bls_g1_msm_batch_dev", "bls_g2_msm_batch_dev",
     "bls_fr_fft_batch", "bls_fr_fft_scratch_bytes", "bls_fr_fft_dev",
 ]
 
@@ -92,6 +93,8 @@ def load():
     lib.bls_batch_normalization_scratch_bytes.argtypes = [vp, ci, sz]
     lib.bls_msm_scratch_bytes.restype = sz
     lib.bls_msm_scratch_bytes.argtypes = [vp, ci, sz, ci]
+    lib.bls_msm_batch_scratch_bytes.restype = sz
+    lib.bls_msm_batch_scratch_bytes.argtypes = [vp, ci, sz, sz, ci]
     lib.bls_fr_fft_scratch_bytes.restype = sz
     lib.bls_fr_fft_scratch_bytes.argtypes = [vp, ci, sz]
     sig = {
@@ -169,6 +172,10 @@ def load():
         "bls_g2_msm": [vp, vp, vp, sz, vp],
         "bls_g1_msm_dev": [vp, vp, vp, sz, ci, vp, vp, vp],
         "bls_g2_msm_dev": [vp, vp, vp, sz, ci, vp, vp, vp],
+        "bls_g1_msm_batch": [vp, vp, ci, vp, sz, sz, vp],
+        "bls_g2_msm_batch": [vp, vp, ci, vp, sz, sz, vp],
+        "bls_g1_msm_batch_dev": [vp, vp, ci, vp, sz, sz, ci, vp, vp, vp],
+        "bls_g2_msm_batch_dev": [vp, vp, ci, vp, sz, sz, ci, vp, vp, vp],
         "bls_fr_fft_batch": [vp, ci, vp, vp, ci, sz],
         "bls_fr_fft_dev": [vp, ci, vp, vp, ci, sz, vp, vp],
     }
@@ -469,6 +476,29 @@ class Context:
         """sum_i k_i * bases_i over (n, 25) affine bases and (n, 4) FrRepr scalars -> one normalised Jacobian row (1, 36)."""
         return self._msm(True, bases, k)
 
+    def _msm_batch(self, g2, bases, k):
+        wa = W_G2A if g2 else W_G1A
+        k = np.ascontiguousarray(k, dtype=np.uint64)
+        bases = np.ascontiguousarray(bases, dtype=np.uint64)
+        if k.ndim != 3 or k.shape[2] != W_FR:
+            raise ValueError("k must have shape (m, n, %d) uint64, got %r" % (W_FR, k.shape))
+        m, n = k.shape[:2]
+        if bases.shape not in ((n, wa), (m, n, wa)):
+            raise ValueError("bases must have shape (n, %d) (shared) or (m, n, %d), got %r for k of %r" % (wa, wa, bases.shape, k.shape))
+        out = np.zeros((m, W_G2 if g2 else W_G1), dtype=np.uint64)
+        fn = self._lib.bls_g2_msm_batch if g2 else self._lib.bls_g1_msm_batch
+        self._check(fn(self._ctx, _p(bases), 1 if bases.ndim == 2 else 0, _p(k), n, m, _p(out)))
+        return out
+
+    def g1_msm_batch(self, bases, k):
+        """m independent sums: k (m, n, 4) FrRepr scalars against (n, 13) affine bases shared by every sum or (m, n, 13),
+        one set per sum -> (m, 18) normalised Jacobian rows, row j = g1_msm(bases (of sum j), k[j])."""
+        return self._msm_batch(False, bases, k)
+
+    def g2_msm_batch(self, bases, k):
+        """g1_msm_batch in G2: bases (n, 25) or (m, n, 25) -> (m, 36)."""
+        return self._msm_batch(True, bases, k)
+
     # ------------------------------------------------------------------ field tower, host arrays
     def field_op(self, degree, op, a, b=None):
         a = _arr(a, 6 * degree, "a")
@@ -572,6 +602,13 @@ class Context:
         b = int(self._lib.bls_msm_scratch_bytes(self._ctx, degree, n, window))
         if b == 0:
             raise ValueError("no MSM of degree %r, n = %d, window = %d" % (degree, n, window))
+        return b
+
+    def msm_batch_scratch_bytes(self, degree, n, m, window=0):
+        """device scratch of bls_g*_msm_batch_dev for m sums of n points; raises for arguments the call would reject"""
+        b = int(self._lib.bls_msm_batch_scratch_bytes(self._ctx, degree, n, m, window))
+        if b == 0:
+            raise ValueError("no MSM batch of degree %r, n = %d, m = %d, window = %d" % (degree, n, m, window))
         return b
 
     def imad_peak(self, variant=0, iters=2000):

@@ -174,6 +174,24 @@ class DeviceEngine:
                           scr.data_ptr(), self._stream())
         return out
 
+    def msm_batch(self, bases, k, g2=False, window=0, out=None):
+        """m independent sums: k (m, n, 4) FrRepr scalars against affine bases shared by every sum ((n, 13) G1 / (n, 25) G2)
+        or one set per sum ((m, n, 13) / (m, n, 25)) -> (m, 18) / (m, 36) normalised Jacobian rows.  window as for msm."""
+        wa, w = (nat.W_G2A, nat.W_G2) if g2 else (nat.W_G1A, nat.W_G1)
+        if not (k.is_cuda and k.dtype == torch.int64 and k.dim() == 3 and k.shape[2] == nat.W_FR and k.is_contiguous()):
+            raise ValueError("k must be a contiguous CUDA int64 tensor of shape (m, n, 4)")
+        m, n = k.shape[:2]
+        if not (bases.is_cuda and bases.dtype == torch.int64 and tuple(bases.shape) in ((n, wa), (m, n, wa)) and bases.is_contiguous()):
+            raise ValueError("bases must be a contiguous CUDA int64 tensor of shape (%d, %d) or (%d, %d, %d)" % (n, wa, m, n, wa))
+        if out is None:
+            out = torch.empty((m, w), dtype=torch.int64, device=self.device)
+        elif not (out.is_cuda and out.dtype == torch.int64 and tuple(out.shape) == (m, w) and out.is_contiguous()):
+            raise ValueError("out must be a contiguous CUDA int64 tensor of shape (%d, %d)" % (m, w))
+        scr = self._buf("msm", self.ctx.msm_batch_scratch_bytes(2 if g2 else 1, n, m, window))
+        self.ctx.call_dev("bls_g2_msm_batch_dev" if g2 else "bls_g1_msm_batch_dev", bases.data_ptr(), 1 if bases.dim() == 2 else 0,
+                          k.data_ptr(), n, m, window, out.data_ptr(), scr.data_ptr(), self._stream())
+        return out
+
     def fr_fft(self, a, kind="fft", out=None):
         """bellman's EvaluationDomain transforms over Fr on the device: kind "fft" | "ifft" | "coset_fft" | "icoset_fft"
         on one polynomial (n, 4) or m polynomials (m, n, 4) of Montgomery-form values, n a power of two.  out may be a

@@ -105,6 +105,13 @@ class _Curve:
         c = _ctx(ctx)
         return (c.g2_msm if cls._g2 else c.g1_msm)(bases_affine, scalars)
 
+    # m independent multiexp sums in one call: scalars (m, n, 4); bases_affine (n, W) shared by every sum or (m, n, W), one
+    # set per sum -> (m, 18|36), row j = multiexp(bases of sum j, scalars[j])
+    @classmethod
+    def multiexp_batch(cls, bases_affine, scalars, ctx=None):
+        c = _ctx(ctx)
+        return (c.g2_msm_batch if cls._g2 else c.g1_msm_batch)(bases_affine, scalars)
+
     # ec.rs:895-905 / 1586-1596
     @classmethod
     def recommended_wnaf_for_scalar(cls, scalars):

@@ -77,4 +77,6 @@ extern "C" {
     pub fn bls_g2_op_batch(ctx: *mut bls_ctx, op: c_int, a: *const bls_g2, b: *const c_void, out: *mut bls_g2, n: usize) -> c_int;
     pub fn bls_g1_msm(ctx: *mut bls_ctx, bases: *const bls_g1_affine, k: *const bls_fr_repr, n: usize, out1: *mut bls_g1) -> c_int;
     pub fn bls_g2_msm(ctx: *mut bls_ctx, bases: *const bls_g2_affine, k: *const bls_fr_repr, n: usize, out1: *mut bls_g2) -> c_int;
+    pub fn bls_g1_msm_batch(ctx: *mut bls_ctx, bases: *const bls_g1_affine, shared_bases: c_int, k: *const bls_fr_repr, n: usize, m: usize, out: *mut bls_g1) -> c_int;
+    pub fn bls_g2_msm_batch(ctx: *mut bls_ctx, bases: *const bls_g2_affine, shared_bases: c_int, k: *const bls_fr_repr, n: usize, m: usize, out: *mut bls_g2) -> c_int;
 }

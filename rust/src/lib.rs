@@ -132,6 +132,21 @@ impl Gpu {
         Ok(marshal::g1_back(&out))
     }
 
+    /// `m` independent multiexp sums in one call, `m = k.len() / n`: sum `j` is `sum_i k[j*n + i] * bases[b(j, i)]` with
+    /// `b(j, i) = i` when `bases.len() == n` (one set of bases for every sum) and `j*n + i` when `bases.len() == k.len()`.
+    /// Each result equals `g1_multiexp` of its sum; a loop of `g1_multiexp` calls becomes one call.
+    pub fn g1_multiexp_batch(&self, bases: &[G1Affine], k: &[FrRepr], n: usize) -> Result<Vec<G1>, GpuError> {
+        assert!(n > 0 && k.len() % n == 0 && (bases.len() == n || bases.len() == k.len()));
+        let m = k.len() / n;
+        let bb: Vec<bls_g1_affine> = bases.iter().map(marshal::g1_affine).collect();
+        let kk: Vec<bls_fr_repr> = k.iter().map(|r| bls_fr_repr { l: r.0 }).collect();
+        let mut out = vec![bls_g1 { x: marshal::FQ_ZERO, y: marshal::FQ_ZERO, z: marshal::FQ_ZERO }; m];
+        let shared = (bases.len() == n) as i32;
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_g1_msm_batch(*ctx, bb.as_ptr(), shared, kk.as_ptr(), n, m, out.as_mut_ptr()) }, *ctx)?;
+        Ok(out.iter().map(marshal::g1_back).collect())
+    }
+
     /// bellman's `EvaluationDomain` transforms over `Fr` for `a.len() / 2^log_n` polynomials back to back, natural order:
     /// kind 0 `fft`, 1 `ifft`, 2 `coset_fft`, 3 `icoset_fft` (`BLS_FFT` ... in the C header).
     pub fn fr_fft(&self, kind: i32, a: &[Fr], log_n: u32) -> Result<Vec<Fr>, GpuError> {
