@@ -229,6 +229,17 @@ int bls_fr_op_batch(bls_ctx*, int op, const bls_fr* a, const bls_fr* b, bls_fr* 
  * BLS_ERR_INVALID_ARGUMENT. */
 enum { BLS_FFT = 0, BLS_IFFT = 1, BLS_COSET_FFT = 2, BLS_ICOSET_FFT = 3 };
 int bls_fr_fft_batch(bls_ctx*, int kind, const bls_fr* in, bls_fr* out, int log_n, size_t m);
+/* Groth16's quotient polynomial H for m proofs: the `h` block of bellman's groth16::create_proof.  Proof j has len
+ * evaluations in each of a, b, c (the ProvingAssignment vectors, Montgomery bls_fr, canonical) at a[j*len + i], and so on.
+ * With n = 2^log_n the smallest power of two >= len (n = 1 for len <= 1), each proof computes
+ *   A, B, C = coset_fft(ifft(x zero-padded to n))                  (EvaluationDomain::from_coeffs, ifft, coset_fft)
+ *   H = icoset_fft((A B - C) z(g)^-1), z(g) = g^n - 1, g = 7        (mul_assign, sub_assign, divide_by_z_on_coset)
+ * and stores coefficients 0 .. n - 2 of H as canonical bls_fr_repr (coefficient n - 1 is dropped, every one goes through
+ * into_repr()) at h[j*(n-1) + i]: the scalars of bls_g1_msm_batch(h_bases, shared_bases = 1, h, n - 1, m, ...).  Outputs are
+ * canonical, so bit-exact with any correct evaluation order.  The inputs are left unchanged; h must not overlap them.
+ * m = 0 does nothing; len <= 1 stores nothing (n - 1 = 0).  log_n <= 28 and m * n <= 2^28, else BLS_ERR_INVALID_ARGUMENT,
+ * as for a NULL pointer when there is something to store. */
+int bls_fr_groth16_h_batch(bls_ctx*, const bls_fr* a, const bls_fr* b, const bls_fr* c, size_t len, size_t m, bls_fr_repr* h);
 
 /* ------------------------------------------------------------------ device-pointer variants
  * Same semantics; every pointer is a device pointer on the context's device, the work is enqueued
@@ -284,6 +295,14 @@ int bls_g2_msm_batch_dev(bls_ctx*, const bls_g2_affine* bases, int shared_bases,
  * log_n > 10, one buffer of m * 2^log_n elements between passes: the call allocates nothing. */
 size_t bls_fr_fft_scratch_bytes(const bls_ctx*, int log_n, size_t m);
 int bls_fr_fft_dev(bls_ctx*, int kind, const bls_fr* in, bls_fr* out, int log_n, size_t m, void* scratch, void* stream);
+/* bls_fr_groth16_h_batch on device pointers, same arguments and limits.  scratch: bls_fr_groth16_h_scratch_bytes(ctx, len,
+ * m) bytes (0 for invalid arguments): 3m * n elements for A, B and C of every proof, then bls_fr_fft_scratch_bytes(ctx,
+ * log_n, 3m) for the transforms; it must not overlap the other buffers.  The call allocates nothing. */
+size_t bls_fr_groth16_h_scratch_bytes(const bls_ctx*, size_t len, size_t m);
+int bls_fr_groth16_h_dev(bls_ctx*, const bls_fr* a, const bls_fr* b, const bls_fr* c, size_t len, size_t m, bls_fr_repr* h, void* scratch, void* stream);
+/* bls_fr_op_batch on device pointers: the same ops, NULL rules for b and ok, and results.  out may equal a or b.  The way
+ * between Montgomery bls_fr and bls_fr_repr (FROM_REPR / INTO_REPR) for data that stays on the device. */
+int bls_fr_op_dev(bls_ctx*, int op, const bls_fr* a, const bls_fr* b, bls_fr* out, uint8_t* ok, size_t n, void* stream);
 
 /* ------------------------------------------------------------------ several GPUs behind ONE call
  * Engine::miller_loop takes ALL pairs of a product in one call (mod.rs:40-102), and a Rust / C caller is one process.

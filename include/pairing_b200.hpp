@@ -266,6 +266,19 @@ struct FrField {
   static std::vector<Elem> ifft(Gpu& g, const std::vector<Elem>& a, int log_n) { return transform(g, BLS_IFFT, a, log_n); }
   static std::vector<Elem> coset_fft(Gpu& g, const std::vector<Elem>& a, int log_n) { return transform(g, BLS_COSET_FFT, a, log_n); }
   static std::vector<Elem> icoset_fft(Gpu& g, const std::vector<Elem>& a, int log_n) { return transform(g, BLS_ICOSET_FFT, a, log_n); }
+  // Groth16's quotient polynomial for m proofs (the `h` block of bellman's create_proof): a, b, c hold m * len evaluations,
+  // proof after proof; the result holds m * (n - 1) canonical FrRepr, n the smallest power of two >= len (1 for len <= 1)
+  static std::vector<FrRepr> groth16_h(Gpu& g, const std::vector<Elem>& a, const std::vector<Elem>& b, const std::vector<Elem>& c, size_t m) {
+    require_same_length(a.size(), b.size(), "FrField::groth16_h");
+    require_same_length(a.size(), c.size(), "FrField::groth16_h");
+    if (m == 0 ? !a.empty() : a.size() % m) throw std::invalid_argument("FrField::groth16_h: a.size() is not a multiple of m");
+    const size_t len = m ? a.size() / m : 0;
+    size_t n = 1;
+    while (n < len) n <<= 1;
+    std::vector<FrRepr> h(m * (n - 1));
+    g.check(bls_fr_groth16_h_batch(g.ctx(), a.data(), b.data(), c.data(), len, m, h.data()));
+    return h;
+  }
 };
 
 // ------------------------------------------------------------------------------------------------ curves

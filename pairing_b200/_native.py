@@ -52,6 +52,7 @@ SYMBOLS = [
     "bls_g1_msm", "bls_g2_msm", "bls_msm_scratch_bytes", "bls_g1_msm_dev", "bls_g2_msm_dev",
     "bls_g1_msm_batch", "bls_g2_msm_batch", "bls_msm_batch_scratch_bytes", "bls_g1_msm_batch_dev", "bls_g2_msm_batch_dev",
     "bls_fr_fft_batch", "bls_fr_fft_scratch_bytes", "bls_fr_fft_dev",
+    "bls_fr_groth16_h_batch", "bls_fr_groth16_h_scratch_bytes", "bls_fr_groth16_h_dev", "bls_fr_op_dev",
 ]
 
 
@@ -97,6 +98,8 @@ def load():
     lib.bls_msm_batch_scratch_bytes.argtypes = [vp, ci, sz, sz, ci]
     lib.bls_fr_fft_scratch_bytes.restype = sz
     lib.bls_fr_fft_scratch_bytes.argtypes = [vp, ci, sz]
+    lib.bls_fr_groth16_h_scratch_bytes.restype = sz
+    lib.bls_fr_groth16_h_scratch_bytes.argtypes = [vp, sz, sz]
     sig = {
         "bls_g2_prepare_batch": [vp, vp, vp, sz],
         "bls_miller_loop_batch": [vp, vp, vp, vp, sz],
@@ -178,6 +181,9 @@ def load():
         "bls_g2_msm_batch_dev": [vp, vp, ci, vp, sz, sz, ci, vp, vp, vp],
         "bls_fr_fft_batch": [vp, ci, vp, vp, ci, sz],
         "bls_fr_fft_dev": [vp, ci, vp, vp, ci, sz, vp, vp],
+        "bls_fr_groth16_h_batch": [vp, vp, vp, vp, sz, sz, vp],
+        "bls_fr_groth16_h_dev": [vp, vp, vp, vp, sz, sz, vp, vp, vp],
+        "bls_fr_op_dev": [vp, ci, vp, vp, vp, vp, sz, vp],
     }
     lib.bls_mgpu_create.restype = vp
     lib.bls_mgpu_create.argtypes = [ctypes.POINTER(ci), ci, ctypes.POINTER(ci)]
@@ -582,6 +588,27 @@ class Context:
         b = int(self._lib.bls_fr_fft_scratch_bytes(self._ctx, log_n, m))
         if b == 0:
             raise ValueError("no FFT of log_n = %d, m = %d" % (log_n, m))
+        return b
+
+    def fr_groth16_h(self, a, b, c):
+        """Groth16's quotient polynomial (the `h` block of bellman's create_proof): a, b, c are the evaluations of one
+        proof (len, 4) or of m proofs (m, len, 4), Montgomery-form values -> H's coefficients 0 .. n - 2 as canonical
+        FrRepr, (n - 1, 4) or (m, n - 1, 4), n the smallest power of two >= len (1 for len <= 1)."""
+        a, b, c = (np.ascontiguousarray(x, dtype=np.uint64) for x in (a, b, c))
+        if a.ndim not in (2, 3) or a.shape[-1] != W_FR or b.shape != a.shape or c.shape != a.shape:
+            raise ValueError("a, b and c must have one shape (len, 4) or (m, len, 4) uint64, got %r, %r, %r" % (a.shape, b.shape, c.shape))
+        length = a.shape[-2]
+        m = a.shape[0] if a.ndim == 3 else 1
+        n = 1 << max(length - 1, 0).bit_length()
+        out = np.zeros(a.shape[:-2] + (n - 1, W_FR), dtype=np.uint64)
+        self._check(self._lib.bls_fr_groth16_h_batch(self._ctx, _p(a), _p(b), _p(c), length, m, _p(out)))
+        return out
+
+    def fr_groth16_h_scratch_bytes(self, length, m=1):
+        """device scratch of bls_fr_groth16_h_dev for m proofs of `length` evaluations; raises for arguments the call would reject"""
+        b = int(self._lib.bls_fr_groth16_h_scratch_bytes(self._ctx, length, m))
+        if b == 0:
+            raise ValueError("no Groth16 H of len = %d, m = %d" % (length, m))
         return b
 
     def call_dev(self, name, *args):

@@ -1323,19 +1323,33 @@ int bls_pair_field_op_batch(bls_ctx* ctx, int degree, int op, const void* a, con
   return BLS_OK;
 }
 
-int bls_fr_op_batch(bls_ctx* ctx, int op, const bls_fr* a, const bls_fr* b, bls_fr* out, uint8_t* ok, size_t n) {
-  if (!ctx || (n && (!a || !out))) return BLS_ERR_INVALID_ARGUMENT;
-  const bool binary = op == BLS_OP_ADD || op == BLS_OP_SUB || op == BLS_OP_MUL;
+// bls_fr_op_batch / _dev argument rules; *binary: the op reads b
+static bool fr_op_args_ok(bls_ctx* ctx, int op, const void* a, const void* b, const void* out, size_t n, bool* binary) {
+  *binary = op == BLS_OP_ADD || op == BLS_OP_SUB || op == BLS_OP_MUL;
   const bool unary = op == BLS_OP_SQR || op == BLS_OP_NEG || op == BLS_OP_DBL || op == BLS_OP_INV || op == BLS_OP_FROM_REPR || op == BLS_OP_INTO_REPR;
-  if ((!binary && !unary) || (binary && n && !b)) return BLS_ERR_INVALID_ARGUMENT;
+  return ctx && !(n && (!a || !out)) && (*binary || unary) && !(*binary && n && !b);
+}
+
+int bls_fr_op_dev(bls_ctx* ctx, int op, const bls_fr* a, const bls_fr* b, bls_fr* out, uint8_t* ok, size_t n, void* stream) {
+  bool binary;
+  if (!fr_op_args_ok(ctx, op, a, b, out, n, &binary)) return BLS_ERR_INVALID_ARGUMENT;
+  if (!n) return BLS_OK;
+  USE_DEVICE(ctx);
+  k_fr_op<<<blocks_for(n, TPB), TPB, 0, pick(ctx, stream)>>>(op, (const uint64_t*)a, binary ? (const uint64_t*)b : nullptr, (uint64_t*)out, ok, n);
+  LAUNCH_CHECK();
+  return BLS_OK;
+}
+
+int bls_fr_op_batch(bls_ctx* ctx, int op, const bls_fr* a, const bls_fr* b, bls_fr* out, uint8_t* ok, size_t n) {
+  bool binary;
+  if (!fr_op_args_ok(ctx, op, a, b, out, n, &binary)) return BLS_ERR_INVALID_ARGUMENT;
   if (!n) return BLS_OK;
   USE_DEVICE(ctx);
   H2D(da, a, n * sizeof(*a));
   H2D(db, binary ? b : nullptr, binary ? n * sizeof(*b) : 1);
   DALLOC(dout, n * sizeof(*out));
   DALLOC(dok, n);
-  k_fr_op<<<blocks_for(n, TPB), TPB, 0, ctx->stream>>>(op, (const uint64_t*)da.p, binary ? (const uint64_t*)db.p : nullptr, (uint64_t*)dout.p, (uint8_t*)dok.p, n);
-  LAUNCH_CHECK();
+  TRY(bls_fr_op_dev(ctx, op, (const bls_fr*)da.p, binary ? (const bls_fr*)db.p : nullptr, (bls_fr*)dout.p, (uint8_t*)dok.p, n, ctx->stream));
   D2H(out, dout, n * sizeof(*out));
   if (ok) D2H(ok, dok, n);
   SYNC();

@@ -15,6 +15,10 @@
 // Twiddles are built on the device by k_fft_tables into the caller's scratch, every entry a product of the powers
 // x^(2^b) of fr_fft_consts.cuh: w^e = T_hi[e >> s] * T_lo[e & (2^s - 1)] (s = ceil(L / 2)), the same two-level scheme
 // for g^(+-j), and the stage table S[bit + di] = omega_(2 bit)^di that the butterflies read.
+//
+// Groth16's quotient polynomial (bls_fr_groth16_h_*) runs on the same transforms: gather and pad, ifft and coset_fft of
+// all 3m polynomials in two calls, the element-wise (A B - C) z(g)^-1, icoset_fft of the m results, conversion to
+// FrRepr without the last coefficient.  The element-wise steps are kernels of their own, not fused into k_fr_fft_pass.
 #include "abi_common.cuh"
 #include "fr_fft_consts.cuh"
 
@@ -164,6 +168,38 @@ __global__ void __launch_bounds__(FFT_TPB, FFT_MINB) k_fr_fft_pass(const FftPass
   }
 }
 
+// ---- Groth16's quotient polynomial H (bellman's groth16::create_proof, the `h` block) ---------------------------------
+// m proofs of len evaluations in each of a, b, c; the work buffer holds 3m polynomials of n = 2^L: A_0 .. A_(m-1),
+// B_0 .. B_(m-1), C_0 .. C_(m-1), so that one transform call covers all 3m and the A regions are the first m.
+
+// one thread per element of the work buffer: EvaluationDomain::from_coeffs (copy, zero-pad to n)
+__global__ void __launch_bounds__(128) k_fr_h_gather(const Fr* a, const Fr* b, const Fr* c, size_t len, size_t m, int L, Fr* w) {
+  const size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= 3 * (m << L)) return;
+  const size_t poly = id >> L, i = id & (((size_t)1 << L) - 1), which = poly / m, j = poly - which * m;
+  const Fr* src = which == 0 ? a : which == 1 ? b : c;
+  st_fr(w + id, i < len ? ld_fr(src + j * len + i) : fr_zero());
+}
+
+// one thread per element of the A regions: a.mul_assign(&b), a.sub_assign(&c), divide_by_z_on_coset -- (A B - C) z(g)^-1
+__global__ void __launch_bounds__(128) k_fr_h_combine(Fr* w, size_t mn, int L) {
+  const size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= mn) return;
+  const Fr x = fr_mul(ld_fr(w + id), ld_fr(w + mn + id));
+  st_fr(w + id, fr_mul(fr_sub(x, ld_fr(w + 2 * mn + id)), FR_Z_INV[L]));
+}
+
+// one thread per element of the A regions: coefficient i < n - 1 of proof j to h[j (n - 1) + i] as into_repr() (x * 1 R^-1)
+__global__ void __launch_bounds__(128) k_fr_into_repr_truncate(const Fr* w, size_t mn, int L, Fr* h) {
+  const size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= mn) return;
+  const size_t j = id >> L, i = id & (((size_t)1 << L) - 1);
+  if (i == ((size_t)1 << L) - 1) return;                   // the dropped coefficient n - 1
+  Fr one = fr_zero();
+  one.v[0] = 1;
+  st_fr(h + id - j, fr_mul(ld_fr(w + id), one));
+}
+
 // ---- host side ----------------------------------------------------------------------------------------------------------
 
 static bool fft_args_ok(int log_n, size_t m) { return log_n >= 0 && log_n <= FFT_MAX_LOG_N && m <= (FFT_MAX_ELEMS >> log_n); }
@@ -256,6 +292,63 @@ static int fft_host(bls_ctx* ctx, int kind, const bls_fr* in, bls_fr* out, int l
   return BLS_OK;
 }
 
+#define GH_MAX_ELEMS ((size_t)1 << 28)     /* m * n, so that the 3m polynomials stay within FFT_MAX_ELEMS */
+
+// n = 2^L, the smallest power of two >= len (1 for len <= 1); false for L > 28 or m * n > 2^28
+static bool gh_args_ok(size_t len, size_t m, int& L) {
+  if (len > ((size_t)1 << FFT_MAX_LOG_N)) return false;
+  for (L = 0; ((size_t)1 << L) < len; L++) {}
+  return m <= (GH_MAX_ELEMS >> L);
+}
+
+// scratch: the work buffer of 3m * n elements, then the scratch of the 3m-polynomial transforms
+static size_t gh_scratch_bytes(int L, size_t m) {
+  FftPlan p;
+  fft_plan(L, 3 * m, p);
+  return fft_align(3 * (m << L) * sizeof(bls_fr)) + p.total;
+}
+
+static int groth16_h_dev_impl(bls_ctx* ctx, const bls_fr* a, const bls_fr* b, const bls_fr* c, size_t len, size_t m, bls_fr_repr* h,
+                              void* scratch, void* stream) {
+  int L;
+  if (!ctx || !gh_args_ok(len, m, L)) return BLS_ERR_INVALID_ARGUMENT;
+  if (m == 0 || len <= 1) return BLS_OK;                   // nothing to store: n - 1 = 0 coefficients per proof
+  if (!a || !b || !c || !h || !scratch) return BLS_ERR_INVALID_ARGUMENT;
+  USE_DEVICE(ctx);
+  cudaStream_t st = pick(ctx, stream);
+  const size_t mn = m << L, work = fft_align(3 * mn * sizeof(bls_fr));
+  Fr* w = (Fr*)scratch;
+  void* fscr = (char*)scratch + work;
+  k_fr_h_gather<<<blocks_for(3 * mn, 128), 128, 0, st>>>((const Fr*)a, (const Fr*)b, (const Fr*)c, len, m, L, w);
+  LAUNCH_CHECK();
+  TRY(fft_dev_impl(ctx, BLS_IFFT, (bls_fr*)w, (bls_fr*)w, L, 3 * m, fscr, st));
+  TRY(fft_dev_impl(ctx, BLS_COSET_FFT, (bls_fr*)w, (bls_fr*)w, L, 3 * m, fscr, st));
+  k_fr_h_combine<<<blocks_for(mn, 128), 128, 0, st>>>(w, mn, L);
+  LAUNCH_CHECK();
+  TRY(fft_dev_impl(ctx, BLS_ICOSET_FFT, (bls_fr*)w, (bls_fr*)w, L, m, fscr, st));   // the m-polynomial plan fits in the 3m one
+  k_fr_into_repr_truncate<<<blocks_for(mn, 128), 128, 0, st>>>(w, mn, L, (Fr*)h);
+  LAUNCH_CHECK();
+  return BLS_OK;
+}
+
+static int groth16_h_host(bls_ctx* ctx, const bls_fr* a, const bls_fr* b, const bls_fr* c, size_t len, size_t m, bls_fr_repr* h) {
+  int L;
+  if (!ctx || !gh_args_ok(len, m, L)) return BLS_ERR_INVALID_ARGUMENT;
+  if (m == 0 || len <= 1) return BLS_OK;
+  if (!a || !b || !c || !h) return BLS_ERR_INVALID_ARGUMENT;
+  USE_DEVICE(ctx);
+  const size_t in_bytes = m * len * sizeof(bls_fr), out_bytes = m * (((size_t)1 << L) - 1) * sizeof(bls_fr_repr);
+  H2D(da, a, in_bytes);
+  H2D(db, b, in_bytes);
+  H2D(dc, c, in_bytes);
+  DALLOC(dh, out_bytes);
+  DALLOC(dscr, gh_scratch_bytes(L, m));
+  TRY(groth16_h_dev_impl(ctx, (const bls_fr*)da.p, (const bls_fr*)db.p, (const bls_fr*)dc.p, len, m, (bls_fr_repr*)dh.p, dscr.p, ctx->stream));
+  D2H(h, dh, out_bytes);
+  SYNC();
+  return BLS_OK;
+}
+
 extern "C" {
 
 size_t bls_fr_fft_scratch_bytes(const bls_ctx* ctx, int log_n, size_t m) {
@@ -268,5 +361,18 @@ int bls_fr_fft_dev(bls_ctx* ctx, int kind, const bls_fr* in, bls_fr* out, int lo
   return fft_dev_impl(ctx, kind, in, out, log_n, m, scratch, stream);
 }
 int bls_fr_fft_batch(bls_ctx* ctx, int kind, const bls_fr* in, bls_fr* out, int log_n, size_t m) { return fft_host(ctx, kind, in, out, log_n, m); }
+
+size_t bls_fr_groth16_h_scratch_bytes(const bls_ctx* ctx, size_t len, size_t m) {
+  int L;
+  if (!ctx || !gh_args_ok(len, m, L)) return 0;
+  return gh_scratch_bytes(L, m);
+}
+int bls_fr_groth16_h_dev(bls_ctx* ctx, const bls_fr* a, const bls_fr* b, const bls_fr* c, size_t len, size_t m, bls_fr_repr* h,
+                         void* scratch, void* stream) {
+  return groth16_h_dev_impl(ctx, a, b, c, len, m, h, scratch, stream);
+}
+int bls_fr_groth16_h_batch(bls_ctx* ctx, const bls_fr* a, const bls_fr* b, const bls_fr* c, size_t len, size_t m, bls_fr_repr* h) {
+  return groth16_h_host(ctx, a, b, c, len, m, h);
+}
 
 }  // extern "C"

@@ -211,6 +211,45 @@ class DeviceEngine:
         self.ctx.call_dev("bls_fr_fft_dev", nat.FFT_KINDS[kind], a.data_ptr(), out.data_ptr(), log_n, m, scr.data_ptr(), self._stream())
         return out
 
+    def groth16_h(self, a, b, c, out=None):
+        """Groth16's quotient polynomial on the device (the `h` block of bellman's create_proof): a, b, c are the
+        evaluations of one proof (len, 4) or of m proofs (m, len, 4), Montgomery-form values -> H's coefficients 0 .. n - 2
+        as canonical FrRepr, (n - 1, 4) or (m, n - 1, 4), n the smallest power of two >= len.  The (m, n - 1, 4) result is
+        the k of msm_batch against n - 1 shared bases."""
+        if not (a.is_cuda and a.dtype == torch.int64 and a.dim() in (2, 3) and a.shape[-1] == nat.W_FR and a.is_contiguous()):
+            raise ValueError("a must be a contiguous CUDA int64 tensor of shape (len, 4) or (m, len, 4)")
+        for t, name in ((b, "b"), (c, "c")):
+            if not (t.is_cuda and t.dtype == torch.int64 and t.shape == a.shape and t.is_contiguous()):
+                raise ValueError("%s must be a contiguous CUDA int64 tensor of shape %r" % (name, tuple(a.shape)))
+        length = a.shape[-2]
+        m = a.shape[0] if a.dim() == 3 else 1
+        shape = tuple(a.shape[:-2]) + ((1 << max(length - 1, 0).bit_length()) - 1, nat.W_FR)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.int64, device=self.device)
+        elif not (out.is_cuda and out.dtype == torch.int64 and tuple(out.shape) == shape and out.is_contiguous()):
+            raise ValueError("out must be a contiguous CUDA int64 tensor of shape %r" % (shape,))
+        scr = self._buf("groth16_h", self.ctx.fr_groth16_h_scratch_bytes(length, m))
+        self.ctx.call_dev("bls_fr_groth16_h_dev", a.data_ptr(), b.data_ptr(), c.data_ptr(), length, m, out.data_ptr(), scr.data_ptr(),
+                          self._stream())
+        return out
+
+    def fr_op(self, op, a, b=None, out=None):
+        """Fr element-wise operation on (n, 4) tensors (bls_fr_op_batch's ops: "add", "mul", ..., "from_repr", "into_repr")
+        -> (out, ok), ok an (n,) uint8 tensor, 0 for the inverse of zero or from_repr of a value >= r.  out may be a or b."""
+        _check(a, nat.W_FR, "a")
+        if b is not None:
+            _check(b, nat.W_FR, "b")
+            if b.shape != a.shape:
+                raise ValueError("a and b must have the same length")
+        if out is None:
+            out = torch.empty_like(a)
+        elif not (out.is_cuda and out.dtype == torch.int64 and out.shape == a.shape and out.is_contiguous()):
+            raise ValueError("out must be a contiguous CUDA int64 tensor of shape %r" % (tuple(a.shape),))
+        ok = torch.empty(a.shape[0], dtype=torch.uint8, device=self.device)
+        self.ctx.call_dev("bls_fr_op_dev", nat.OPS[op], a.data_ptr(), b.data_ptr() if b is not None else None, out.data_ptr(),
+                          ok.data_ptr(), a.shape[0], self._stream())
+        return out, ok
+
     def wnaf_table(self, base, window, g2=False):
         """Wnaf::base(g, n): the shared window table (2^(window-1), W) on the device."""
         w = nat.W_G2 if g2 else nat.W_G1

@@ -56,6 +56,7 @@ extern "C" {
     pub fn bls_g2_scale_by_cofactor_batch(ctx: *mut bls_ctx, input: *const bls_g2_affine, out: *mut bls_g2, n: usize) -> c_int;
     pub fn bls_fr_op_batch(ctx: *mut bls_ctx, op: c_int, a: *const bls_fr_repr, b: *const bls_fr_repr, out: *mut bls_fr_repr, ok: *mut u8, n: usize) -> c_int;
     pub fn bls_fr_fft_batch(ctx: *mut bls_ctx, kind: c_int, input: *const bls_fr_repr, out: *mut bls_fr_repr, log_n: c_int, m: usize) -> c_int;
+    pub fn bls_fr_groth16_h_batch(ctx: *mut bls_ctx, a: *const bls_fr_repr, b: *const bls_fr_repr, c: *const bls_fr_repr, len: usize, m: usize, h: *mut bls_fr_repr) -> c_int;
     pub fn bls_fq12_pow_batch(ctx: *mut bls_ctx, a: *const bls_fq12, k: *const bls_fr_repr, out: *mut bls_fq12, n: usize) -> c_int;
     pub fn bls_fq12_product(ctx: *mut bls_ctx, input: *const bls_fq12, n: usize, out1: *mut bls_fq12) -> c_int;
 

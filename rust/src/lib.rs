@@ -158,6 +158,22 @@ impl Gpu {
         Ok(out.iter().map(marshal::fr_back).collect())
     }
 
+    /// Groth16's quotient polynomial for `m` proofs, the `h` block of bellman's `create_proof`: `a`, `b`, `c` are the
+    /// `ProvingAssignment` evaluations of the proofs back to back (`len = a.len() / m` each).  Returns `m * (n - 1)`
+    /// canonical `FrRepr` coefficients, `n` the smallest power of two `>= len`: the scalars of `g1_multiexp_batch` against
+    /// the `n - 1` bases of the proving key's `h` query.
+    pub fn groth16_h(&self, a: &[Fr], b: &[Fr], c: &[Fr], m: usize) -> Result<Vec<FrRepr>, GpuError> {
+        assert!(m > 0 && a.len() % m == 0 && b.len() == a.len() && c.len() == a.len());
+        let len = a.len() / m;
+        let n = len.max(1).next_power_of_two();
+        let (aa, bb, cc): (Vec<bls_fr_repr>, Vec<bls_fr_repr>, Vec<bls_fr_repr>) =
+            (a.iter().map(marshal::fr).collect(), b.iter().map(marshal::fr).collect(), c.iter().map(marshal::fr).collect());
+        let mut h = vec![bls_fr_repr { l: [0; 4] }; m * (n - 1)];
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_fr_groth16_h_batch(*ctx, aa.as_ptr(), bb.as_ptr(), cc.as_ptr(), len, m, h.as_mut_ptr()) }, *ctx)?;
+        Ok(h.iter().map(|r| FrRepr(r.l)).collect())
+    }
+
     /// `let q = Q.prepare(); ps.iter().map(|p| Bls12::pairing(p, Q))` with the one `G2Prepared` staged on the device.
     pub fn pairing_shared_q(&self, p: &[G1Affine], q: &G2Affine) -> Result<Vec<Fq12>, GpuError> {
         let pp: Vec<bls_g1_affine> = p.iter().map(marshal::g1_affine).collect();

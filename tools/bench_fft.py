@@ -7,6 +7,11 @@ the inter-pass twiddles, the coset and n^-1 scalings and the table set-up are no
 the time, divided by the IMAD.WIDE rate measured in the same run (bls_imad_peak variant 0).  HBM share = one read and one
 write of m * n * 32 bytes per pass over the time, divided by 7.7 TB/s.
     python tools/bench_fft.py --out fft.json
+--groth16-h times Groth16's quotient polynomial instead (bls_fr_groth16_h_dev through DeviceEngine.groth16_h) for m proofs
+of len = n evaluations, m = 1 at n = 2^16, 2^20, 2^22, 2^24, m = 64 at 2^12 and m = 8 at 2^20, under the same conditions.
+Each shape also times, in the same process, the fr_fft calls the one call contains: ifft and coset_fft of 3m polynomials
+and icoset_fft of m, in place.
+    python tools/bench_fft.py --groth16-h --out groth16_h.json
 """
 import argparse
 import json
@@ -27,11 +32,38 @@ def passes(log_n):
     return 1 if log_n <= 10 else (log_n + 9) // 10
 
 
+def bench_groth16_h(eng, timed, gen):
+    import torch
+    rows = []
+    for lg, m in ((16, 1), (20, 1), (22, 1), (24, 1), (12, 64), (20, 8)):
+        n = 1 << lg
+        abc = torch.randint(-(1 << 63), (1 << 63) - 1, (3 * m, n, 4), dtype=torch.int64, device=eng.device, generator=gen)
+        abc[..., 3] &= (1 << 60) - 1
+        a, b, c = (abc[i * m:(i + 1) * m].clone() for i in range(3))
+        out = torch.empty((m, n - 1, 4), dtype=torch.int64, device=eng.device)
+
+        def transforms():
+            eng.fr_fft(abc, "ifft", out=abc)
+            eng.fr_fft(abc, "coset_fft", out=abc)
+            eng.fr_fft(abc[:m], "icoset_fft", out=abc[:m])
+
+        ms_call = timed(lambda: eng.groth16_h(a, b, c, out=out))
+        ms_fft = timed(transforms)
+        rows.append({"log_n": lg, "m": m, "passes": passes(lg), "ms_groth16_h": ms_call, "ms_fft_calls": ms_fft,
+                     "ratio": ms_call / ms_fft, "ms_per_proof": ms_call / m})
+        print(json.dumps(rows[-1]), flush=True)
+        del abc, a, b, c, out
+        eng._scratch.clear()
+        torch.cuda.empty_cache()
+    return rows
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True)
     ap.add_argument("--reps", type=int, default=7)
     ap.add_argument("--sizes", default="10,12,16,20,24,26")
+    ap.add_argument("--groth16-h", action="store_true", help="time Groth16's quotient polynomial H instead of the transforms")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -64,6 +96,13 @@ def main():
             ts.append(a.elapsed_time(b))
         return median(ts)
 
+    if args.groth16_h:
+        res = {"gpu": gpu, "reps": args.reps, "flush_bytes": 256 << 20,
+               "inputs": "torch.randint limbs, top limb masked to 60 bits (canonical), len = n evaluations per proof",
+               "rows": bench_groth16_h(eng, timed, gen)}
+        with open(args.out, "w") as f:
+            json.dump(res, f, indent=1)
+        return
     shapes = [(kind, lg, 1) for lg in (int(x) for x in args.sizes.split(",")) for kind in KINDS]
     shapes += [(kind, 20, 3) for kind in KINDS] + [(kind, 10, 256) for kind in KINDS]
     rows = []
