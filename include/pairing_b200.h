@@ -240,6 +240,39 @@ int bls_fr_fft_batch(bls_ctx*, int kind, const bls_fr* in, bls_fr* out, int log_
  * m = 0 does nothing; len <= 1 stores nothing (n - 1 = 0).  log_n <= 28 and m * n <= 2^28, else BLS_ERR_INVALID_ARGUMENT,
  * as for a NULL pointer when there is something to store. */
 int bls_fr_groth16_h_batch(bls_ctx*, const bls_fr* a, const bls_fr* b, const bls_fr* c, size_t len, size_t m, bls_fr_repr* h);
+/* Groth16 proofs: bellman's groth16::create_proof for m proofs of one circuit, from the assignments to the proofs.
+ * Proof j: a, b, c as for bls_fr_groth16_h_batch (len each, the input constraints create_proof appends included); its
+ * input_assignment at input[j*num_inputs + i] (input[0] = one by bellman's convention, not enforced) and aux_assignment at
+ * aux[j*num_aux + i]; the blinding values r[j], s[j].  All Montgomery bls_fr.  Density bitmaps (DensityTracker, shared by the
+ * m proofs): 32-bit words, bit i at word i / 32, bit i % 32 (bit-vec's BitVec<u32> storage); bits past the end are ignored.
+ * With rank_D(i) the number of set bits of D below i and every scalar through into_repr():
+ *   h_ans  = sum_{i < n-1} H_i h[i]                                  (H: bls_fr_groth16_h_batch, n the smallest power of two >= len)
+ *   l_ans  = sum_{i < num_aux} aux_i l[i]
+ *   a_ans  = sum_{i < num_inputs} input_i a[i] + sum_{a_aux_density[i]} aux_i a[num_inputs + rank_a_aux(i)]
+ *   b1_ans = sum_{b_input_density[i]} input_i b_g1[rank_b_in(i)] + sum_{b_aux_density[i]} aux_i b_g1[popcount(b_in) + rank_b_aux(i)]
+ *   b2_ans = the same over b_g2
+ *   A = r delta_g1 + alpha_g1 + a_ans,  B = s delta_g2 + beta_g2 + b2_ans,
+ *   C = (r s) delta_g1 + s alpha_g1 + r beta_g1 + s a_ans + r b1_ans + h_ans + l_ans   (bellman's g_c; C = s A + r B_g1 - rs delta_g1)
+ * out[j] = (A, B, C) in affine form (into_affine(); the identity is (0, one, infinity = 1)).  Outputs are canonical, so
+ * bit-exact with any correct summation order.  Entries of a query past the used prefix are ignored.
+ * Differences from bellman: a query base at infinity is summed as zero (bellman stops with UnexpectedIdentity; a key from
+ * its generator has none), and one density set serves every proof (the m proofs come from one circuit).
+ * BLS_ERR_INVALID_ARGUMENT, before any work: delta_g1 or delta_g2 at infinity (bellman's UnexpectedIdentity); a query
+ * shorter than the formula indexes (h_len < n - 1, l_len < num_aux, a_len < num_inputs + popcount(a_aux), b_len <
+ * popcount(b_in) + popcount(b_aux)); m > 2^16 or m times one multiexp's length (n - 1, num_aux, a's or b's) > 2^26; a NULL
+ * pointer where there is work.  m = 0 does nothing. */
+typedef struct { bls_g1_affine a; bls_g2_affine b; bls_g1_affine c; } bls_groth16_proof;   /* 408 B: bellman's Proof<Bls12> */
+typedef struct {
+  bls_g1_affine alpha_g1, beta_g1, delta_g1;                            /* by value: host memory in both variants */
+  bls_g2_affine beta_g2, delta_g2;
+  const bls_g1_affine *h, *l, *a, *b_g1;                                /* host pointers for _batch, device pointers for _dev */
+  const bls_g2_affine* b_g2;
+  size_t h_len, l_len, a_len, b_len;                                    /* b_len: b_g1 and b_g2 have the same length */
+} bls_groth16_params;
+int bls_groth16_prove_batch(bls_ctx*, const bls_groth16_params* params, const bls_fr* a, const bls_fr* b, const bls_fr* c, size_t len,
+                            const bls_fr* input, size_t num_inputs, const bls_fr* aux, size_t num_aux, const uint32_t* a_aux_density,
+                            const uint32_t* b_input_density, const uint32_t* b_aux_density, const bls_fr* r, const bls_fr* s, size_t m,
+                            bls_groth16_proof* out);
 
 /* ------------------------------------------------------------------ device-pointer variants
  * Same semantics; every pointer is a device pointer on the context's device, the work is enqueued
@@ -303,6 +336,17 @@ int bls_fr_groth16_h_dev(bls_ctx*, const bls_fr* a, const bls_fr* b, const bls_f
 /* bls_fr_op_batch on device pointers: the same ops, NULL rules for b and ok, and results.  out may equal a or b.  The way
  * between Montgomery bls_fr and bls_fr_repr (FROM_REPR / INTO_REPR) for data that stays on the device. */
 int bls_fr_op_dev(bls_ctx*, int op, const bls_fr* a, const bls_fr* b, bls_fr* out, uint8_t* ok, size_t n, void* stream);
+/* bls_groth16_prove_batch on device pointers: a, b, c, input, aux, r, s, out and the params' query pointers; params and
+ * the density bitmaps stay in host memory (their popcounts set the multiexp lengths).  Same limits.  scratch:
+ * bls_groth16_prove_scratch_bytes(ctx, the same arguments) bytes (0 for invalid arguments): the vk points and bitmap words
+ * (copied with cudaMemcpyAsync on `stream`), the five sums and the r / s products, the scalars of the five multiexps, and
+ * one region for H's transforms and each multiexp in turn.  The call allocates nothing and does not synchronise. */
+size_t bls_groth16_prove_scratch_bytes(const bls_ctx*, const bls_groth16_params* params, size_t len, size_t num_inputs, size_t num_aux,
+                                       const uint32_t* a_aux_density, const uint32_t* b_input_density, const uint32_t* b_aux_density, size_t m);
+int bls_groth16_prove_dev(bls_ctx*, const bls_groth16_params* params, const bls_fr* a, const bls_fr* b, const bls_fr* c, size_t len,
+                          const bls_fr* input, size_t num_inputs, const bls_fr* aux, size_t num_aux, const uint32_t* a_aux_density,
+                          const uint32_t* b_input_density, const uint32_t* b_aux_density, const bls_fr* r, const bls_fr* s, size_t m,
+                          bls_groth16_proof* out, void* scratch, void* stream);
 
 /* ------------------------------------------------------------------ several GPUs behind ONE call
  * Engine::miller_loop takes ALL pairs of a product in one call (mod.rs:40-102), and a Rust / C caller is one process.

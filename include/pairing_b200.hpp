@@ -398,6 +398,40 @@ template <class Proj, class Aff, bool IS_G2> struct Curve {
 using G1 = Curve<G1Point, G1AffinePoint, false>;
 using G2 = Curve<G2Point, G2AffinePoint, true>;
 
+// ------------------------------------------------------------------------------------------------ Groth16 prover
+// bellman's groth16::create_proof for m proofs of one circuit (bls_groth16_prove_batch): Params holds the vk points and the
+// queries of the proving key; the assignments of the m proofs are back to back (a, b, c: m * len, input: m * num_inputs,
+// aux: m * num_aux, r, s: m); the densities are bit-vec's BitVec<u32> words of DensityTracker (shared by the m proofs).
+struct Groth16 {
+  using Proof = bls_groth16_proof;
+  struct Params {
+    G1AffinePoint alpha_g1, beta_g1, delta_g1;
+    G2AffinePoint beta_g2, delta_g2;
+    std::vector<G1AffinePoint> h, l, a, b_g1;
+    std::vector<G2AffinePoint> b_g2;
+  };
+  static std::vector<Proof> create_proof(Gpu& g, const Params& p, const std::vector<bls_fr>& a, const std::vector<bls_fr>& b,
+                                         const std::vector<bls_fr>& c, const std::vector<bls_fr>& input, const std::vector<bls_fr>& aux,
+                                         const std::vector<uint32_t>& a_aux_density, const std::vector<uint32_t>& b_input_density,
+                                         const std::vector<uint32_t>& b_aux_density, const std::vector<bls_fr>& r, const std::vector<bls_fr>& s,
+                                         size_t m) {
+    if (m == 0 ? !(a.empty() && input.empty() && aux.empty()) : (a.size() % m || input.size() % m || aux.size() % m))
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::create_proof: a, input or aux is not m rows");
+    if (b.size() != a.size() || c.size() != a.size() || r.size() != m || s.size() != m)
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::create_proof: b, c must match a and r, s hold m values");
+    if (p.b_g1.size() != p.b_g2.size()) throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::create_proof: b_g1 and b_g2 differ in length");
+    const size_t len = m ? a.size() / m : 0, ni = m ? input.size() / m : 0, na = m ? aux.size() / m : 0;
+    if (a_aux_density.size() < (na + 31) / 32 || b_aux_density.size() < (na + 31) / 32 || b_input_density.size() < (ni + 31) / 32)
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::create_proof: a density bitmap is shorter than its variables");
+    bls_groth16_params c_params{p.alpha_g1, p.beta_g1, p.delta_g1, p.beta_g2, p.delta_g2, p.h.data(), p.l.data(), p.a.data(),
+                                p.b_g1.data(), p.b_g2.data(), p.h.size(), p.l.size(), p.a.size(), p.b_g1.size()};
+    std::vector<Proof> out(m);
+    g.check(bls_groth16_prove_batch(g.ctx(), &c_params, a.data(), b.data(), c.data(), len, input.data(), ni, aux.data(), na, a_aux_density.data(),
+                                    b_input_density.data(), b_aux_density.data(), r.data(), s.data(), m, out.data()));
+    return out;
+  }
+};
+
 struct G1Affine {
   static std::vector<G1PreparedPoint> prepare(const std::vector<G1AffinePoint>& p) { return p; }   // ec.rs:924-935
   // CurveAffine::mul (ec.rs:174-177)

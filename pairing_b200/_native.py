@@ -5,6 +5,7 @@ entry point raises.  Nothing here imports or calls the oracle.
 """
 import ctypes
 import os
+from dataclasses import dataclass
 
 import numpy as np
 
@@ -53,6 +54,7 @@ SYMBOLS = [
     "bls_g1_msm_batch", "bls_g2_msm_batch", "bls_msm_batch_scratch_bytes", "bls_g1_msm_batch_dev", "bls_g2_msm_batch_dev",
     "bls_fr_fft_batch", "bls_fr_fft_scratch_bytes", "bls_fr_fft_dev",
     "bls_fr_groth16_h_batch", "bls_fr_groth16_h_scratch_bytes", "bls_fr_groth16_h_dev", "bls_fr_op_dev",
+    "bls_groth16_prove_batch", "bls_groth16_prove_scratch_bytes", "bls_groth16_prove_dev",
 ]
 
 
@@ -100,6 +102,8 @@ def load():
     lib.bls_fr_fft_scratch_bytes.argtypes = [vp, ci, sz]
     lib.bls_fr_groth16_h_scratch_bytes.restype = sz
     lib.bls_fr_groth16_h_scratch_bytes.argtypes = [vp, sz, sz]
+    lib.bls_groth16_prove_scratch_bytes.restype = sz
+    lib.bls_groth16_prove_scratch_bytes.argtypes = [vp, vp, sz, sz, sz, vp, vp, vp, sz]
     sig = {
         "bls_g2_prepare_batch": [vp, vp, vp, sz],
         "bls_miller_loop_batch": [vp, vp, vp, vp, sz],
@@ -184,6 +188,8 @@ def load():
         "bls_fr_groth16_h_batch": [vp, vp, vp, vp, sz, sz, vp],
         "bls_fr_groth16_h_dev": [vp, vp, vp, vp, sz, sz, vp, vp, vp],
         "bls_fr_op_dev": [vp, ci, vp, vp, vp, vp, sz, vp],
+        "bls_groth16_prove_batch": [vp, vp, vp, vp, vp, sz, vp, sz, vp, sz, vp, vp, vp, vp, vp, sz, vp],
+        "bls_groth16_prove_dev": [vp, vp, vp, vp, vp, sz, vp, sz, vp, sz, vp, vp, vp, vp, vp, sz, vp, vp, vp],
     }
     lib.bls_mgpu_create.restype = vp
     lib.bls_mgpu_create.argtypes = [ctypes.POINTER(ci), ci, ctypes.POINTER(ci)]
@@ -209,6 +215,60 @@ def _arr(a, w, name="array"):
 
 def _p(a):
     return None if a is None else a.ctypes.data_as(ctypes.c_void_p)
+
+
+W_PROOF = 2 * W_G1A + W_G2A        # bls_groth16_proof: A (G1Affine), B (G2Affine), C (G1Affine)
+
+
+@dataclass
+class Groth16Params:
+    """The part of bellman's groth16::Parameters that create_proof reads: the vk points alpha_g1, beta_g1, delta_g1 ((13,)
+    G1Affine rows), beta_g2, delta_g2 ((25,) G2Affine rows) and the queries h, l, a, b_g1 ((n, 13)) and b_g2 ((n, 25)).  numpy
+    uint64 arrays for Context.groth16_prove; for DeviceEngine.groth16_prove the queries are CUDA int64 tensors."""
+    alpha_g1: object
+    beta_g1: object
+    delta_g1: object
+    beta_g2: object
+    delta_g2: object
+    h: object
+    l: object
+    a: object
+    b_g1: object
+    b_g2: object
+
+
+class _Groth16ParamsC(ctypes.Structure):
+    _fields_ = [("alpha_g1", ctypes.c_uint64 * W_G1A), ("beta_g1", ctypes.c_uint64 * W_G1A), ("delta_g1", ctypes.c_uint64 * W_G1A),
+                ("beta_g2", ctypes.c_uint64 * W_G2A), ("delta_g2", ctypes.c_uint64 * W_G2A),
+                ("h", ctypes.c_void_p), ("l", ctypes.c_void_p), ("a", ctypes.c_void_p), ("b_g1", ctypes.c_void_p),
+                ("b_g2", ctypes.c_void_p), ("h_len", ctypes.c_size_t), ("l_len", ctypes.c_size_t), ("a_len", ctypes.c_size_t),
+                ("b_len", ctypes.c_size_t)]
+
+
+def groth16_params_c(params, ptr, length):
+    """the bls_groth16_params struct: vk rows by value, ptr(query) and length(query) for the five queries"""
+    c = _Groth16ParamsC()
+    for name, w in (("alpha_g1", W_G1A), ("beta_g1", W_G1A), ("delta_g1", W_G1A), ("beta_g2", W_G2A), ("delta_g2", W_G2A)):
+        row = np.ascontiguousarray(getattr(params, name), dtype=np.uint64).reshape(-1)
+        if row.shape != (w,):
+            raise ValueError("%s must be one row of %d uint64, got %r" % (name, w, row.shape))
+        getattr(c, name)[:] = [int(x) for x in row]
+    for name in ("h", "l", "a", "b_g1", "b_g2"):
+        setattr(c, name, ptr(getattr(params, name)))
+    if length(params.b_g1) != length(params.b_g2):
+        raise ValueError("b_g1 and b_g2 must have the same length")
+    c.h_len, c.l_len, c.a_len, c.b_len = (length(getattr(params, q)) for q in ("h", "l", "a", "b_g1"))
+    return c
+
+
+def density_words(d, bits, name):
+    """a numpy bool array of `bits` entries -> the uint32 words of bit-vec's BitVec<u32> (bit i at word i / 32, bit i % 32)"""
+    d = np.ascontiguousarray(d, dtype=bool)
+    if d.shape != (bits,):
+        raise ValueError("%s must be a bool array of %d entries, got %r" % (name, bits, d.shape))
+    b = np.packbits(d, bitorder="little")
+    b = np.concatenate([b, np.zeros(-len(b) % 4, dtype=np.uint8)])
+    return np.ascontiguousarray(b.view("<u4"))
 
 
 class Context:
@@ -610,6 +670,43 @@ class Context:
         if b == 0:
             raise ValueError("no Groth16 H of len = %d, m = %d" % (length, m))
         return b
+
+    def groth16_prove(self, params, a, b, c, input, aux, densities, r, s):
+        """bellman's groth16::create_proof for m proofs of one circuit (bls_groth16_prove_batch).  params: Groth16Params of
+        numpy rows; a, b, c (m, len, 4), input (m, num_inputs, 4), aux (m, num_aux, 4), r and s (m, 4), all Montgomery-form
+        Fr; densities = (a_aux_density, b_input_density, b_aux_density), numpy bool arrays of num_aux, num_inputs and num_aux
+        entries.  Returns the proofs (A (m, 13), B (m, 25), C (m, 13)) in affine form, views of one (m, 51) array."""
+        a, b, c, input, aux = (np.ascontiguousarray(x, dtype=np.uint64) for x in (a, b, c, input, aux))
+        r, s = (np.ascontiguousarray(x, dtype=np.uint64) for x in (r, s))
+        if a.ndim != 3 or a.shape[2] != W_FR or b.shape != a.shape or c.shape != a.shape:
+            raise ValueError("a, b and c must have one shape (m, len, 4) uint64, got %r, %r, %r" % (a.shape, b.shape, c.shape))
+        m, length = a.shape[:2]
+        for x, name in ((input, "input"), (aux, "aux")):
+            if x.ndim != 3 or x.shape[0] != m or x.shape[2] != W_FR:
+                raise ValueError("%s must have shape (%d, n, 4) uint64, got %r" % (name, m, x.shape))
+        for x, name in ((r, "r"), (s, "s")):
+            if x.shape != (m, W_FR):
+                raise ValueError("%s must have shape (%d, 4) uint64, got %r" % (name, m, x.shape))
+        ni, na = input.shape[1], aux.shape[1]
+        q = {}
+        for name, w in (("h", W_G1A), ("l", W_G1A), ("a", W_G1A), ("b_g1", W_G1A), ("b_g2", W_G2A)):
+            q[name] = _arr(getattr(params, name), w, name)
+        pc = groth16_params_c(Groth16Params(params.alpha_g1, params.beta_g1, params.delta_g1, params.beta_g2, params.delta_g2, **q), _p, len)
+        dw = [density_words(d, bits, name) for d, bits, name in zip(densities, (na, ni, na), ("a_aux_density", "b_input_density", "b_aux_density"))]
+        out = np.zeros((m, W_PROOF), dtype=np.uint64)
+        self._check(self._lib.bls_groth16_prove_batch(self._ctx, ctypes.byref(pc), _p(a), _p(b), _p(c), length, _p(input), ni, _p(aux), na,
+                                                      _p(dw[0]), _p(dw[1]), _p(dw[2]), _p(r), _p(s), m, _p(out)))
+        return out[:, :W_G1A], out[:, W_G1A:W_G1A + W_G2A], out[:, W_G1A + W_G2A:]
+
+    def groth16_prove_scratch_bytes(self, params_c, length, num_inputs, num_aux, density_words_, m):
+        """device scratch of bls_groth16_prove_dev; params_c from groth16_params_c, density_words_ the three uint32 word
+        arrays; raises for arguments the call would reject"""
+        n = int(self._lib.bls_groth16_prove_scratch_bytes(self._ctx, ctypes.byref(params_c), length, num_inputs, num_aux,
+                                                          *[_p(w) for w in density_words_], m))
+        if n == 0:
+            raise ValueError("no Groth16 proof of len = %d, num_inputs = %d, num_aux = %d, m = %d for these params and densities"
+                             % (length, num_inputs, num_aux, m))
+        return n
 
     def call_dev(self, name, *args):
         """Raw access to a `*_dev` entry point: args are ints (device pointers / sizes / stream)."""

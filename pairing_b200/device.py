@@ -4,6 +4,8 @@ torch is plumbing only (device memory, streams, torch.distributed); every kernel
 through the C ABI's `*_dev` entry points on torch's current stream.  Tensors are int64 with the
 ABI's u64 word layout, one row per element (same shapes as the numpy API: (n, 13) G1Affine, ...).
 """
+import ctypes
+
 import torch
 
 from . import _native as nat
@@ -232,6 +234,39 @@ class DeviceEngine:
         self.ctx.call_dev("bls_fr_groth16_h_dev", a.data_ptr(), b.data_ptr(), c.data_ptr(), length, m, out.data_ptr(), scr.data_ptr(),
                           self._stream())
         return out
+
+    def groth16_prove(self, params, a, b, c, input, aux, densities, r, s, out=None):
+        """bellman's groth16::create_proof for m proofs of one circuit on the device (bls_groth16_prove_dev): the arguments
+        of Context.groth16_prove as contiguous CUDA int64 tensors -- a, b, c (m, len, 4), input (m, num_inputs, 4), aux
+        (m, num_aux, 4), r, s (m, 4) and params' queries -- except params' vk rows and the densities (numpy bool arrays),
+        which stay on the host.  Returns (A (m, 13), B (m, 25), C (m, 13)), views of one (m, 51) tensor (`out` if given)."""
+        for t, name in ((a, "a"), (b, "b"), (c, "c"), (input, "input"), (aux, "aux")):
+            if not (t.is_cuda and t.dtype == torch.int64 and t.dim() == 3 and t.shape[2] == nat.W_FR and t.is_contiguous()):
+                raise ValueError("%s must be a contiguous CUDA int64 tensor of shape (m, n, 4)" % name)
+        m, length = a.shape[:2]
+        if b.shape != a.shape or c.shape != a.shape or input.shape[0] != m or aux.shape[0] != m:
+            raise ValueError("a, b, c must have one shape (m, len, 4) and input, aux m rows: %r %r %r %r %r"
+                             % tuple(tuple(x.shape) for x in (a, b, c, input, aux)))
+        for t, name in ((r, "r"), (s, "s")):
+            _check(t, nat.W_FR, name)
+            if t.shape[0] != m:
+                raise ValueError("%s must have %d rows" % (name, m))
+        for name, w in (("h", nat.W_G1A), ("l", nat.W_G1A), ("a", nat.W_G1A), ("b_g1", nat.W_G1A), ("b_g2", nat.W_G2A)):
+            _check(getattr(params, name), w, "params." + name)
+        ni, na = input.shape[1], aux.shape[1]
+        vk = [x.cpu().numpy() if isinstance(x, torch.Tensor) else x for x in (params.alpha_g1, params.beta_g1, params.delta_g1, params.beta_g2, params.delta_g2)]
+        pc = nat.groth16_params_c(nat.Groth16Params(*vk, params.h, params.l, params.a, params.b_g1, params.b_g2),
+                                  lambda t: t.data_ptr(), lambda t: t.shape[0])
+        dw = [nat.density_words(d, bits, name) for d, bits, name in zip(densities, (na, ni, na), ("a_aux_density", "b_input_density", "b_aux_density"))]
+        if out is None:
+            out = torch.empty((m, nat.W_PROOF), dtype=torch.int64, device=self.device)
+        elif not (out.is_cuda and out.dtype == torch.int64 and tuple(out.shape) == (m, nat.W_PROOF) and out.is_contiguous()):
+            raise ValueError("out must be a contiguous CUDA int64 tensor of shape (%d, %d)" % (m, nat.W_PROOF))
+        scr = self._buf("groth16", self.ctx.groth16_prove_scratch_bytes(pc, length, ni, na, dw, m))
+        self.ctx.call_dev("bls_groth16_prove_dev", ctypes.byref(pc), a.data_ptr(), b.data_ptr(), c.data_ptr(), length, input.data_ptr(), ni,
+                          aux.data_ptr(), na, *[nat._p(w) for w in dw], r.data_ptr(), s.data_ptr(), m, out.data_ptr(), scr.data_ptr(),
+                          self._stream())
+        return out[:, :nat.W_G1A], out[:, nat.W_G1A:nat.W_G1A + nat.W_G2A], out[:, nat.W_G1A + nat.W_G2A:]
 
     def fr_op(self, op, a, b=None, out=None):
         """Fr element-wise operation on (n, 4) tensors (bls_fr_op_batch's ops: "add", "mul", ..., "from_repr", "into_repr")

@@ -12,6 +12,14 @@ use std::os::raw::{c_char, c_int, c_void};
 #[repr(C)] #[derive(Copy, Clone)] pub struct bls_g2_affine { pub x: bls_fq2, pub y: bls_fq2, pub infinity: u64 }
 #[repr(C)] #[derive(Copy, Clone)] pub struct bls_g2 { pub x: bls_fq2, pub y: bls_fq2, pub z: bls_fq2 }
 #[repr(C)] #[derive(Copy, Clone)] pub struct bls_fr_repr { pub l: [u64; 4] }
+#[repr(C)] #[derive(Copy, Clone)] pub struct bls_groth16_proof { pub a: bls_g1_affine, pub b: bls_g2_affine, pub c: bls_g1_affine }
+#[repr(C)] pub struct bls_groth16_params {
+    pub alpha_g1: bls_g1_affine, pub beta_g1: bls_g1_affine, pub delta_g1: bls_g1_affine,
+    pub beta_g2: bls_g2_affine, pub delta_g2: bls_g2_affine,
+    pub h: *const bls_g1_affine, pub l: *const bls_g1_affine, pub a: *const bls_g1_affine, pub b_g1: *const bls_g1_affine,
+    pub b_g2: *const bls_g2_affine,
+    pub h_len: usize, pub l_len: usize, pub a_len: usize, pub b_len: usize,
+}
 #[repr(C)] #[derive(Copy, Clone)] pub struct bls_g2_prepared { pub coeffs: [[bls_fq2; 3]; 68], pub infinity: u64 }
 pub enum bls_ctx {}
 /// several devices of one node behind one call (include/pairing_b200.h, "several GPUs")
@@ -56,6 +64,10 @@ extern "C" {
     pub fn bls_g2_scale_by_cofactor_batch(ctx: *mut bls_ctx, input: *const bls_g2_affine, out: *mut bls_g2, n: usize) -> c_int;
     pub fn bls_fr_op_batch(ctx: *mut bls_ctx, op: c_int, a: *const bls_fr_repr, b: *const bls_fr_repr, out: *mut bls_fr_repr, ok: *mut u8, n: usize) -> c_int;
     pub fn bls_fr_fft_batch(ctx: *mut bls_ctx, kind: c_int, input: *const bls_fr_repr, out: *mut bls_fr_repr, log_n: c_int, m: usize) -> c_int;
+    pub fn bls_groth16_prove_batch(ctx: *mut bls_ctx, params: *const bls_groth16_params, a: *const bls_fr_repr, b: *const bls_fr_repr, c: *const bls_fr_repr, len: usize,
+                                   input: *const bls_fr_repr, num_inputs: usize, aux: *const bls_fr_repr, num_aux: usize, a_aux_density: *const u32,
+                                   b_input_density: *const u32, b_aux_density: *const u32, r: *const bls_fr_repr, s: *const bls_fr_repr, m: usize,
+                                   out: *mut bls_groth16_proof) -> c_int;
     pub fn bls_fr_groth16_h_batch(ctx: *mut bls_ctx, a: *const bls_fr_repr, b: *const bls_fr_repr, c: *const bls_fr_repr, len: usize, m: usize, h: *mut bls_fr_repr) -> c_int;
     pub fn bls_fq12_pow_batch(ctx: *mut bls_ctx, a: *const bls_fq12, k: *const bls_fr_repr, out: *mut bls_fq12, n: usize) -> c_int;
     pub fn bls_fq12_product(ctx: *mut bls_ctx, input: *const bls_fq12, n: usize, out1: *mut bls_fq12) -> c_int;

@@ -174,6 +174,40 @@ impl Gpu {
         Ok(h.iter().map(|r| FrRepr(r.l)).collect())
     }
 
+    /// bellman's `groth16::create_proof` for `m` proofs of one circuit, after synthesis: `a`, `b`, `c` are the proofs'
+    /// `ProvingAssignment` vectors back to back (`len = a.len() / m` each, input constraints included), `inputs` and `aux`
+    /// their `input_assignment` / `aux_assignment`, `densities` the words of the circuit's three `DensityTracker::bv`
+    /// (`a_aux`, `b_input`, `b_aux`: `BitVec<u32>` storage, shared by the proofs), `r` and `s` the blinding values.
+    /// Returns `Proof { a, b, c }` of every proof as `(A, B, C)`, bit-exact with bellman.
+    pub fn groth16_create_proof_batch(&self, params: &Groth16Params, a: &[Fr], b: &[Fr], c: &[Fr], inputs: &[Fr], aux: &[Fr],
+                                      densities: [&[u32]; 3], r: &[Fr], s: &[Fr], m: usize)
+                                      -> Result<Vec<(G1Affine, G2Affine, G1Affine)>, GpuError> {
+        assert!(m > 0 && a.len() % m == 0 && inputs.len() % m == 0 && aux.len() % m == 0 && b.len() == a.len() && c.len() == a.len());
+        assert!(r.len() == m && s.len() == m && params.b_g1.len() == params.b_g2.len());
+        let (len, ni, na) = (a.len() / m, inputs.len() / m, aux.len() / m);
+        let fr = |v: &[Fr]| -> Vec<bls_fr_repr> { v.iter().map(marshal::fr).collect() };
+        let (aa, bb, cc, ii, xx, rr, ss) = (fr(a), fr(b), fr(c), fr(inputs), fr(aux), fr(r), fr(s));
+        let g1s = |v: &[G1Affine]| -> Vec<bls_g1_affine> { v.iter().map(marshal::g1_affine).collect() };
+        let (h, l, qa, b1) = (g1s(&params.h), g1s(&params.l), g1s(&params.a), g1s(&params.b_g1));
+        let b2: Vec<bls_g2_affine> = params.b_g2.iter().map(marshal::g2_affine).collect();
+        let p = bls_groth16_params {
+            alpha_g1: marshal::g1_affine(&params.alpha_g1), beta_g1: marshal::g1_affine(&params.beta_g1),
+            delta_g1: marshal::g1_affine(&params.delta_g1), beta_g2: marshal::g2_affine(&params.beta_g2),
+            delta_g2: marshal::g2_affine(&params.delta_g2),
+            h: h.as_ptr(), l: l.as_ptr(), a: qa.as_ptr(), b_g1: b1.as_ptr(), b_g2: b2.as_ptr(),
+            h_len: h.len(), l_len: l.len(), a_len: qa.len(), b_len: b1.len(),
+        };
+        let zero1 = bls_g1_affine { x: marshal::FQ_ZERO, y: marshal::FQ_ZERO, infinity: 1 };
+        let zero2 = bls_g2_affine { x: bls_fq2 { c0: marshal::FQ_ZERO, c1: marshal::FQ_ZERO }, y: bls_fq2 { c0: marshal::FQ_ZERO, c1: marshal::FQ_ZERO }, infinity: 1 };
+        let mut out = vec![bls_groth16_proof { a: zero1, b: zero2, c: zero1 }; m];
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe {
+            bls_groth16_prove_batch(*ctx, &p, aa.as_ptr(), bb.as_ptr(), cc.as_ptr(), len, ii.as_ptr(), ni, xx.as_ptr(), na, densities[0].as_ptr(),
+                                    densities[1].as_ptr(), densities[2].as_ptr(), rr.as_ptr(), ss.as_ptr(), m, out.as_mut_ptr())
+        }, *ctx)?;
+        Ok(out.iter().map(|p| (marshal::g1_affine_back(&p.a), marshal::g2_affine_back(&p.b), marshal::g1_affine_back(&p.c))).collect())
+    }
+
     /// `let q = Q.prepare(); ps.iter().map(|p| Bls12::pairing(p, Q))` with the one `G2Prepared` staged on the device.
     pub fn pairing_shared_q(&self, p: &[G1Affine], q: &G2Affine) -> Result<Vec<Fq12>, GpuError> {
         let pp: Vec<bls_g1_affine> = p.iter().map(marshal::g1_affine).collect();
@@ -215,6 +249,13 @@ fn check(rc: i32, ctx: *mut bls_ctx) -> Result<(), GpuError> {
 
 /// Explicit field-by-field copies between the crate's types and the `#[repr(C)]` mirrors.  `Fq` is
 /// `Fq(FqRepr([u64; 6]))` in Montgomery form (fq.rs:699-700), which is exactly `bls_fq`.
+/// The part of bellman's `groth16::Parameters` that `create_proof` reads: the verifying key's alpha_g1, beta_g1, delta_g1,
+/// beta_g2, delta_g2 and the `h`, `l`, `a`, `b_g1`, `b_g2` queries.
+pub struct Groth16Params {
+    pub alpha_g1: G1Affine, pub beta_g1: G1Affine, pub delta_g1: G1Affine, pub beta_g2: G2Affine, pub delta_g2: G2Affine,
+    pub h: Vec<G1Affine>, pub l: Vec<G1Affine>, pub a: Vec<G1Affine>, pub b_g1: Vec<G1Affine>, pub b_g2: Vec<G2Affine>,
+}
+
 mod marshal {
     use super::ffi::*;
     use pairing::bls12_381::*;
@@ -237,6 +278,7 @@ mod marshal {
     pub fn fq12_back(x: &bls_fq12) -> Fq12 { Fq12 { c0: fq6_back(&x.c0), c1: fq6_back(&x.c1) } }
     pub fn g1_affine(p: &G1Affine) -> bls_g1_affine { bls_g1_affine { x: fq(&p.x), y: fq(&p.y), infinity: p.infinity as u64 } }
     pub fn g2_affine(p: &G2Affine) -> bls_g2_affine { bls_g2_affine { x: fq2(&p.x), y: fq2(&p.y), infinity: p.infinity as u64 } }
+    pub fn g2_affine_back(p: &bls_g2_affine) -> G2Affine { G2Affine { x: fq2_back(&p.x), y: fq2_back(&p.y), infinity: p.infinity != 0 } }
     pub fn g1_affine_back(p: &bls_g1_affine) -> G1Affine { G1Affine { x: fq_back(&p.x), y: fq_back(&p.y), infinity: p.infinity != 0 } }
     pub fn g1(p: &G1) -> bls_g1 { bls_g1 { x: fq(&p.x), y: fq(&p.y), z: fq(&p.z) } }
     pub fn g1_back(p: &bls_g1) -> G1 { G1 { x: fq_back(&p.x), y: fq_back(&p.y), z: fq_back(&p.z) } }
