@@ -273,6 +273,42 @@ int bls_groth16_prove_batch(bls_ctx*, const bls_groth16_params* params, const bl
                             const bls_fr* input, size_t num_inputs, const bls_fr* aux, size_t num_aux, const uint32_t* a_aux_density,
                             const uint32_t* b_input_density, const uint32_t* b_aux_density, const bls_fr* r, const bls_fr* s, size_t m,
                             bls_groth16_proof* out);
+/* Groth16 verification: bellman's groth16::{prepare_verifying_key, verify_proof} for proofs of one circuit.
+ * bls_groth16_pvk is bellman's PreparedVerifyingKey without ic (passed separately, like the prover's queries), plus the two
+ * negated G2 points in affine form.  Both prepared points start at a multiple of 16 bytes (the pads), so that the
+ * verification kernel can stage their coefficients by TMA bulk copies.  bls_groth16_prepare_verifying_key fills it from the
+ * vk points: alpha_g1_beta_g2 = pairing(alpha_g1, beta_g2), neg_gamma_g2 = prepare(-gamma_g2), neg_delta_g2 =
+ * prepare(-delta_g2), bit-exact with bellman; the pads are zero.  NULL pointers give BLS_ERR_INVALID_ARGUMENT. */
+typedef struct {
+  bls_g2_prepared neg_gamma_g2;                                      /* offset 0 */
+  uint64_t pad0;
+  bls_g2_prepared neg_delta_g2;                                      /* offset 19 600 */
+  uint64_t pad1;
+  bls_fq12 alpha_g1_beta_g2;                                         /* offset 39 200 */
+  bls_g2_affine neg_gamma_g2_affine, neg_delta_g2_affine;            /* offsets 39 776, 39 976 */
+} bls_groth16_pvk;                                                   /* 40 176 B */
+int bls_groth16_prepare_verifying_key(bls_ctx*, const bls_g1_affine* alpha_g1, const bls_g2_affine* beta_g2, const bls_g2_affine* gamma_g2,
+                                      const bls_g2_affine* delta_g2, bls_groth16_pvk* out);
+/* bellman's verify_proof for m proofs of one circuit.  ic holds the vk's num_inputs + 1 points; proof j's public inputs are
+ * inputs[j*num_inputs + i], Montgomery bls_fr without bellman's leading one, as verify_proof takes them.  With
+ * acc_j = ic[0] + sum_i x_ji ic[i + 1]:
+ *   ok[j] = 1  iff  final_exponentiation(miller_loop([(A_j, B_j), (acc_j, -gamma), (C_j, -delta)])) == alpha_g1_beta_g2,
+ * else 0 (a None from the final exponentiation gives 0).  A pair with a member at infinity (A_j, B_j, acc_j or C_j) contributes
+ * one, as in Engine::miller_loop.  Like bellman, the call does not validate points: decode proofs with
+ * bls_g*_decode_batch(checked = 1).  m <= 2^16 and m * (num_inputs + 1) <= 2^26 (bls_g1_msm_batch's limits); outside them,
+ * or for a NULL pointer where there is work, BLS_ERR_INVALID_ARGUMENT before any work.  m = 0 does nothing. */
+int bls_groth16_verify_batch(bls_ctx*, const bls_groth16_pvk* pvk, const bls_g1_affine* ic, size_t num_inputs, const bls_groth16_proof* proofs,
+                             const bls_fr* inputs, size_t m, uint8_t* ok);
+/* Randomized batch verification (bellperson's verify_proofs_batch): one verdict for m proofs, with the caller's randomizers
+ * rho[j] (canonical bls_fr_repr, < r; the library has no RNG).  With s_0 = sum_j rho_j and s_i = sum_j rho_j x_j(i-1) (mod r):
+ *   *ok1 = 1  iff  FE( prod_j ML(rho_j A_j, B_j) * ML(sum_i s_i ic_i, -gamma) * ML(sum_j rho_j C_j, -delta) )
+ *                  == alpha_g1_beta_g2 ^ (sum_j rho_j),
+ * exactly this equation; else 0.  A proof with rho_j = 0 is left out of it.  With random rho an invalid proof makes the
+ * verdict 0 except with probability about 1/r.  Limits are those of the multiexps and the product: m <= 2^26 and
+ * num_inputs + 1 <= 2^26, else BLS_ERR_INVALID_ARGUMENT, as for a NULL pointer where there is work.  m = 0 sets *ok1 = 1
+ * (the equation holds for the empty batch: both sides are one) when ok1 is not NULL, and does nothing else. */
+int bls_groth16_verify_rlc_batch(bls_ctx*, const bls_groth16_pvk* pvk, const bls_g1_affine* ic, size_t num_inputs, const bls_groth16_proof* proofs,
+                                 const bls_fr* inputs, const bls_fr_repr* rho, size_t m, uint8_t* ok1);
 
 /* ------------------------------------------------------------------ device-pointer variants
  * Same semantics; every pointer is a device pointer on the context's device, the work is enqueued
@@ -347,6 +383,17 @@ int bls_groth16_prove_dev(bls_ctx*, const bls_groth16_params* params, const bls_
                           const bls_fr* input, size_t num_inputs, const bls_fr* aux, size_t num_aux, const uint32_t* a_aux_density,
                           const uint32_t* b_input_density, const uint32_t* b_aux_density, const bls_fr* r, const bls_fr* s, size_t m,
                           bls_groth16_proof* out, void* scratch, void* stream);
+/* bls_groth16_verify_batch / bls_groth16_verify_rlc_batch on device pointers: pvk, ic, proofs, inputs, rho and ok / ok1 (one
+ * byte).  pvk must be 16-byte aligned.  Same limits.  scratch: bls_groth16_verify_scratch_bytes(ctx, num_inputs, m) (the msm
+ * scalars and sums and the msm's work region) or bls_groth16_verify_rlc_scratch_bytes(ctx, num_inputs, m) (the pairs of the
+ * product, the scalars s and the msm and product work regions) bytes, 0 for invalid arguments.  The calls allocate nothing
+ * and do not synchronise. */
+size_t bls_groth16_verify_scratch_bytes(const bls_ctx*, size_t num_inputs, size_t m);
+int bls_groth16_verify_dev(bls_ctx*, const bls_groth16_pvk* pvk, const bls_g1_affine* ic, size_t num_inputs, const bls_groth16_proof* proofs,
+                           const bls_fr* inputs, size_t m, uint8_t* ok, void* scratch, void* stream);
+size_t bls_groth16_verify_rlc_scratch_bytes(const bls_ctx*, size_t num_inputs, size_t m);
+int bls_groth16_verify_rlc_dev(bls_ctx*, const bls_groth16_pvk* pvk, const bls_g1_affine* ic, size_t num_inputs, const bls_groth16_proof* proofs,
+                               const bls_fr* inputs, const bls_fr_repr* rho, size_t m, uint8_t* ok1, void* scratch, void* stream);
 
 /* ------------------------------------------------------------------ several GPUs behind ONE call
  * Engine::miller_loop takes ALL pairs of a product in one call (mod.rs:40-102), and a Rust / C caller is one process.

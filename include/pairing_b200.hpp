@@ -19,6 +19,7 @@
 #pragma once
 #include <cstdint>
 #include <cstring>
+#include <memory>
 #include <optional>
 #include <stdexcept>
 #include <string>
@@ -429,6 +430,34 @@ struct Groth16 {
     g.check(bls_groth16_prove_batch(g.ctx(), &c_params, a.data(), b.data(), c.data(), len, input.data(), ni, aux.data(), na, a_aux_density.data(),
                                     b_input_density.data(), b_aux_density.data(), r.data(), s.data(), m, out.data()));
     return out;
+  }
+
+  // bellman's prepare_verifying_key (bls_groth16_prepare_verifying_key); ic stays with the caller
+  using PreparedVerifyingKey = bls_groth16_pvk;
+  static std::unique_ptr<PreparedVerifyingKey> prepare_verifying_key(Gpu& g, const G1AffinePoint& alpha_g1, const G2AffinePoint& beta_g2,
+                                                                     const G2AffinePoint& gamma_g2, const G2AffinePoint& delta_g2) {
+    std::unique_ptr<PreparedVerifyingKey> pvk(new PreparedVerifyingKey);
+    g.check(bls_groth16_prepare_verifying_key(g.ctx(), &alpha_g1, &beta_g2, &gamma_g2, &delta_g2, pvk.get()));
+    return pvk;
+  }
+  // bellman's verify_proof for m = proofs.size() proofs (bls_groth16_verify_batch): ic holds num_inputs + 1 points, inputs the
+  // m rows of num_inputs public inputs (without the leading one) back to back
+  static std::vector<bool> verify_proof(Gpu& g, const PreparedVerifyingKey& pvk, const std::vector<G1AffinePoint>& ic,
+                                        const std::vector<Proof>& proofs, const std::vector<bls_fr>& inputs) {
+    if (ic.empty() || inputs.size() != proofs.size() * (ic.size() - 1))
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::verify_proof: inputs must hold num_inputs = ic.size() - 1 values per proof");
+    std::vector<uint8_t> ok(proofs.size());
+    g.check(bls_groth16_verify_batch(g.ctx(), &pvk, ic.data(), ic.size() - 1, proofs.data(), inputs.data(), proofs.size(), ok.data()));
+    return std::vector<bool>(ok.begin(), ok.end());
+  }
+  // the randomized batch check (bls_groth16_verify_rlc_batch) with the caller's randomizers rho (canonical FrRepr, one per proof)
+  static bool verify_proofs_batch(Gpu& g, const PreparedVerifyingKey& pvk, const std::vector<G1AffinePoint>& ic, const std::vector<Proof>& proofs,
+                                  const std::vector<bls_fr>& inputs, const std::vector<bls_fr_repr>& rho) {
+    if (ic.empty() || inputs.size() != proofs.size() * (ic.size() - 1) || rho.size() != proofs.size())
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::verify_proofs_batch: inputs must hold ic.size() - 1 values and rho one value per proof");
+    uint8_t ok = 0;
+    g.check(bls_groth16_verify_rlc_batch(g.ctx(), &pvk, ic.data(), ic.size() - 1, proofs.data(), inputs.data(), rho.data(), proofs.size(), &ok));
+    return ok != 0;
   }
 };
 

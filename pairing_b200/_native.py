@@ -55,6 +55,8 @@ SYMBOLS = [
     "bls_fr_fft_batch", "bls_fr_fft_scratch_bytes", "bls_fr_fft_dev",
     "bls_fr_groth16_h_batch", "bls_fr_groth16_h_scratch_bytes", "bls_fr_groth16_h_dev", "bls_fr_op_dev",
     "bls_groth16_prove_batch", "bls_groth16_prove_scratch_bytes", "bls_groth16_prove_dev",
+    "bls_groth16_prepare_verifying_key", "bls_groth16_verify_batch", "bls_groth16_verify_scratch_bytes", "bls_groth16_verify_dev",
+    "bls_groth16_verify_rlc_batch", "bls_groth16_verify_rlc_scratch_bytes", "bls_groth16_verify_rlc_dev",
 ]
 
 
@@ -104,6 +106,9 @@ def load():
     lib.bls_fr_groth16_h_scratch_bytes.argtypes = [vp, sz, sz]
     lib.bls_groth16_prove_scratch_bytes.restype = sz
     lib.bls_groth16_prove_scratch_bytes.argtypes = [vp, vp, sz, sz, sz, vp, vp, vp, sz]
+    for name in ("bls_groth16_verify_scratch_bytes", "bls_groth16_verify_rlc_scratch_bytes"):
+        getattr(lib, name).restype = sz
+        getattr(lib, name).argtypes = [vp, sz, sz]
     sig = {
         "bls_g2_prepare_batch": [vp, vp, vp, sz],
         "bls_miller_loop_batch": [vp, vp, vp, vp, sz],
@@ -190,6 +195,11 @@ def load():
         "bls_fr_op_dev": [vp, ci, vp, vp, vp, vp, sz, vp],
         "bls_groth16_prove_batch": [vp, vp, vp, vp, vp, sz, vp, sz, vp, sz, vp, vp, vp, vp, vp, sz, vp],
         "bls_groth16_prove_dev": [vp, vp, vp, vp, vp, sz, vp, sz, vp, sz, vp, vp, vp, vp, vp, sz, vp, vp, vp],
+        "bls_groth16_prepare_verifying_key": [vp, vp, vp, vp, vp, vp],
+        "bls_groth16_verify_batch": [vp, vp, vp, sz, vp, vp, sz, vp],
+        "bls_groth16_verify_dev": [vp, vp, vp, sz, vp, vp, sz, vp, vp, vp],
+        "bls_groth16_verify_rlc_batch": [vp, vp, vp, sz, vp, vp, vp, sz, vp],
+        "bls_groth16_verify_rlc_dev": [vp, vp, vp, sz, vp, vp, vp, sz, vp, vp, vp],
     }
     lib.bls_mgpu_create.restype = vp
     lib.bls_mgpu_create.argtypes = [ctypes.POINTER(ci), ci, ctypes.POINTER(ci)]
@@ -259,6 +269,18 @@ def groth16_params_c(params, ptr, length):
         raise ValueError("b_g1 and b_g2 must have the same length")
     c.h_len, c.l_len, c.a_len, c.b_len = (length(getattr(params, q)) for q in ("h", "l", "a", "b_g1"))
     return c
+
+
+class Groth16PvkC(ctypes.Structure):
+    """bls_groth16_pvk: bellman's PreparedVerifyingKey without ic, plus -gamma_g2 and -delta_g2 in affine form.  The pads put
+    both prepared points at 16-byte aligned offsets."""
+    _fields_ = [("neg_gamma_g2", ctypes.c_uint64 * W_G2P), ("pad0", ctypes.c_uint64),
+                ("neg_delta_g2", ctypes.c_uint64 * W_G2P), ("pad1", ctypes.c_uint64),
+                ("alpha_g1_beta_g2", ctypes.c_uint64 * W_FQ12),
+                ("neg_gamma_g2_affine", ctypes.c_uint64 * W_G2A), ("neg_delta_g2_affine", ctypes.c_uint64 * W_G2A)]
+
+
+W_PVK = ctypes.sizeof(Groth16PvkC) // 8     # 5022 words
 
 
 def density_words(d, bits, name):
@@ -706,6 +728,60 @@ class Context:
         if n == 0:
             raise ValueError("no Groth16 proof of len = %d, num_inputs = %d, num_aux = %d, m = %d for these params and densities"
                              % (length, num_inputs, num_aux, m))
+        return n
+
+    def groth16_prepare_verifying_key(self, alpha_g1, beta_g2, gamma_g2, delta_g2):
+        """bellman's prepare_verifying_key (bls_groth16_prepare_verifying_key): alpha_g1 a (13,) G1Affine row, beta_g2,
+        gamma_g2, delta_g2 (25,) G2Affine rows -> the bls_groth16_pvk as a (5022,) uint64 array (Groth16PvkC's layout)."""
+        rows = []
+        for x, w, name in ((alpha_g1, W_G1A, "alpha_g1"), (beta_g2, W_G2A, "beta_g2"), (gamma_g2, W_G2A, "gamma_g2"), (delta_g2, W_G2A, "delta_g2")):
+            rows.append(_arr(np.reshape(x, (1, -1)), w, name))
+        out = np.zeros(W_PVK, dtype=np.uint64)
+        self._check(self._lib.bls_groth16_prepare_verifying_key(self._ctx, *[_p(r) for r in rows], _p(out)))
+        return out
+
+    def _verify_args(self, pvk, ic, proofs, inputs):
+        pvk = np.ascontiguousarray(pvk, dtype=np.uint64)
+        if pvk.shape != (W_PVK,):
+            raise ValueError("pvk must be a (%d,) uint64 array, got %r" % (W_PVK, pvk.shape))
+        ic, proofs = _arr(ic, W_G1A, "ic"), _arr(proofs, W_PROOF, "proofs")
+        m, ni = proofs.shape[0], ic.shape[0] - 1
+        inputs = np.ascontiguousarray(inputs, dtype=np.uint64)
+        if ni < 0 or inputs.shape != (m, ni, W_FR):
+            raise ValueError("ic must hold num_inputs + 1 points and inputs have shape (m, num_inputs, 4) = (%d, %d, 4), got %r, %r"
+                             % (m, max(ni, 0), ic.shape, inputs.shape))
+        return pvk, ic, proofs, inputs, m, ni
+
+    def groth16_verify(self, pvk, ic, proofs, inputs):
+        """bellman's verify_proof for m proofs of one circuit (bls_groth16_verify_batch): pvk from
+        groth16_prepare_verifying_key, ic (num_inputs + 1, 13), proofs (m, 51) rows (A, B, C), inputs (m, num_inputs, 4)
+        Montgomery-form Fr without the leading one -> (m,) bool array."""
+        pvk, ic, proofs, inputs, m, ni = self._verify_args(pvk, ic, proofs, inputs)
+        ok = np.zeros(m, dtype=np.uint8)
+        self._check(self._lib.bls_groth16_verify_batch(self._ctx, _p(pvk), _p(ic), ni, _p(proofs), _p(inputs), m, _p(ok)))
+        return ok.astype(bool)
+
+    def groth16_verify_rlc(self, pvk, ic, proofs, inputs, rho):
+        """the randomized batch check (bls_groth16_verify_rlc_batch): the arguments of groth16_verify and the randomizers
+        rho (m, 4) canonical FrRepr -> one bool (True for m = 0: the equation holds for the empty batch)"""
+        pvk, ic, proofs, inputs, m, ni = self._verify_args(pvk, ic, proofs, inputs)
+        rho = np.ascontiguousarray(rho, dtype=np.uint64)
+        if rho.shape != (m, W_FR):
+            raise ValueError("rho must have shape (%d, 4) uint64, got %r" % (m, rho.shape))
+        ok = np.zeros(1, dtype=np.uint8)
+        self._check(self._lib.bls_groth16_verify_rlc_batch(self._ctx, _p(pvk), _p(ic), ni, _p(proofs), _p(inputs), _p(rho), m, _p(ok)))
+        return bool(ok[0])
+
+    def groth16_verify_scratch_bytes(self, num_inputs, m):
+        n = int(self._lib.bls_groth16_verify_scratch_bytes(self._ctx, num_inputs, m))
+        if n == 0:
+            raise ValueError("no Groth16 verification of m = %d proofs with num_inputs = %d" % (m, num_inputs))
+        return n
+
+    def groth16_verify_rlc_scratch_bytes(self, num_inputs, m):
+        n = int(self._lib.bls_groth16_verify_rlc_scratch_bytes(self._ctx, num_inputs, m))
+        if n == 0:
+            raise ValueError("no randomized Groth16 check of m = %d proofs with num_inputs = %d" % (m, num_inputs))
         return n
 
     def call_dev(self, name, *args):

@@ -90,14 +90,6 @@ __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_PAIR_MINB) k_pair_miller_pre
 // bytes of line coefficients are staged ONCE per block in shared memory by a TMA bulk copy (cp.async.bulk, completion on
 // an mbarrier); every lane pair then reads them as shared-memory broadcasts and does only `ell` and the squarings
 // (5156 M per Miller loop instead of 6916 M with the G2 steps).
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ P2 ld_p2_smem(const uint64_t* p) {
-  P2 r;
-  const uint2* q = reinterpret_cast<const uint2*>(p + 6 * pair_c());
-#pragma unroll
-  for (int i = 0; i < 6; i++) { uint2 t = q[i]; r.v.v[2 * i] = t.x; r.v.v[2 * i + 1] = t.y; }
-  return r;
-}
 template <bool FINAL_EXP>
 __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_PAIR_MINB) k_pair_miller_shared_q(const uint64_t* p, const uint64_t* qp, uint64_t* out, size_t n) {
   __shared__ __align__(128) uint64_t s_coeffs[68 * 36];
@@ -121,8 +113,7 @@ __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_PAIR_MINB) k_pair_miller_sha
   const uint64_t* pi = p + G1A_W * i;
   const bool live = pi[12] == 0 && qp[G2P_W - 1] == 0;
   const Fp px = ld_fp(pi), py = ld_fp(pi + 6);
-  // wait for the bulk copy (phase 0 of the barrier)
-  asm volatile("{\n\t.reg .pred ready;\n\tWAIT_%=:\n\tmbarrier.try_wait.parity.shared::cta.b64 ready, [%0], 0;\n\t@ready bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" ::"r"(bar) : "memory");
+  mbar_wait_phase0(bar);                       // the bulk copy has landed
   P12 f;
   p12_one(f);
   PCoeffs c;
@@ -172,12 +163,6 @@ __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_PAIR_MINB) k_pair_final_exp(
 // which lie in the cyclotomic subgroup a^(q^4 - q^2 + 1) = 1.  One Frobenius test per operand -- a^(q^4) a == a^(q^2),
 // about 1 % of the work -- tells: when it holds for every lane pair of the WARP, the 252 squarings are Granger-Scott
 // cyclotomic squarings (6 Fq2 products instead of 12, the same value there); otherwise the warp squares generically.
-__device__ __forceinline__ bool p12_eq(const P12& a, const P12& b) {
-  const bool e = fp_eq(a.c0.c0.v, b.c0.c0.v) && fp_eq(a.c0.c1.v, b.c0.c1.v) && fp_eq(a.c0.c2.v, b.c0.c2.v) &&
-                 fp_eq(a.c1.c0.v, b.c1.c0.v) && fp_eq(a.c1.c1.v, b.c1.c1.v) && fp_eq(a.c1.c2.v, b.c1.c2.v);
-  const int eo = __shfl_xor_sync(0xffffffffu, (int)e, 1);
-  return e && eo;
-}
 __global__ void __launch_bounds__(BLS_PAIR_TPB, BLS_PAIR_MINB) k_pair_fq12_pow(const uint64_t* in, const uint64_t* k, uint64_t* out, size_t n) {
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   size_t i = t >> 1;

@@ -1,5 +1,5 @@
 // pair_io.cuh -- ABI <-> lane-pair register conversions and the launch shape shared by the lane-pair translation units
-// (kernels_pair.cu, kernels_mm.cu).
+// (kernels_pair.cu, kernels_mm.cu, kernels_groth16_verify.cu).
 #pragma once
 #include "abi_common.cuh"
 #include "pair_tower.cuh"
@@ -34,3 +34,17 @@ __device__ __forceinline__ void pcoeffs_set_one_if(bool dead, PCoeffs& c) {
 // G2Prepared::from_affine (mod.rs:168-358) on lane pairs: lane c writes coefficient c of every Fq2 of the 68 triples
 __device__ __forceinline__ void st_pcoeffs(uint64_t* p, const PCoeffs& c) { st_p2(p, c.c0); st_p2(p + 12, c.c1); st_p2(p + 24, c.c2); }
 __device__ __forceinline__ void ld_pcoeffs(PCoeffs& c, const uint64_t* p) { c.c0 = ld_p2(p); c.c1 = ld_p2(p + 12); c.c2 = ld_p2(p + 24); }
+
+// prepared coefficients staged in shared memory (a TMA bulk copy completing on an mbarrier): lane c reads coefficient c
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ P2 ld_p2_smem(const uint64_t* p) {
+  P2 r;
+  const uint2* q = reinterpret_cast<const uint2*>(p + 6 * pair_c());
+#pragma unroll
+  for (int i = 0; i < 6; i++) { uint2 t = q[i]; r.v.v[2 * i] = t.x; r.v.v[2 * i + 1] = t.y; }
+  return r;
+}
+// spin until phase 0 of the mbarrier at shared address `bar` has completed
+__device__ __forceinline__ void mbar_wait_phase0(uint32_t bar) {
+  asm volatile("{\n\t.reg .pred ready;\n\tWAIT_%=:\n\tmbarrier.try_wait.parity.shared::cta.b64 ready, [%0], 0;\n\t@ready bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}" ::"r"(bar) : "memory");
+}

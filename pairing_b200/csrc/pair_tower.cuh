@@ -477,6 +477,14 @@ __device__ __forceinline__ bool p12_is_zero(const P12& a) {
   return z && zo;
 }
 
+// both lanes learn whether the two Fq12 values are equal
+__device__ __forceinline__ bool p12_eq(const P12& a, const P12& b) {
+  const bool e = fp_eq(a.c0.c0.v, b.c0.c0.v) && fp_eq(a.c0.c1.v, b.c0.c1.v) && fp_eq(a.c0.c2.v, b.c0.c2.v) &&
+                 fp_eq(a.c1.c0.v, b.c1.c0.v) && fp_eq(a.c1.c1.v, b.c1.c1.v) && fp_eq(a.c1.c2.v, b.c1.c2.v);
+  const int eo = __shfl_xor_sync(0xffffffffu, (int)e, 1);
+  return e && eo;
+}
+
 // mod.rs:104-160
 // y0 = r^2 by the generic 12-product squaring.  The 6-product cyclotomic squaring gives the same value (r is in the cyclotomic
 // subgroup after the easy part) but lost: under bench.py's conditions (L2 flushed between launches) the fused kernel measured

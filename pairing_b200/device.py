@@ -268,6 +268,41 @@ class DeviceEngine:
                           self._stream())
         return out[:, :nat.W_G1A], out[:, nat.W_G1A:nat.W_G1A + nat.W_G2A], out[:, nat.W_G1A + nat.W_G2A:]
 
+    def _verify_args(self, pvk, ic, proofs, inputs):
+        if not (pvk.is_cuda and pvk.dtype == torch.int64 and tuple(pvk.shape) == (nat.W_PVK,) and pvk.is_contiguous()):
+            raise ValueError("pvk must be a contiguous CUDA int64 tensor of shape (%d,)" % nat.W_PVK)
+        _check(ic, nat.W_G1A, "ic"); _check(proofs, nat.W_PROOF, "proofs")
+        m, ni = proofs.shape[0], ic.shape[0] - 1
+        if not (inputs.is_cuda and inputs.dtype == torch.int64 and tuple(inputs.shape) == (m, max(ni, 0), nat.W_FR) and inputs.is_contiguous()) or ni < 0:
+            raise ValueError("ic must hold num_inputs + 1 points and inputs be a contiguous CUDA int64 tensor of shape (m, num_inputs, 4)")
+        return m, ni
+
+    def groth16_verify(self, pvk, ic, proofs, inputs, out=None):
+        """bellman's verify_proof for m proofs on the device (bls_groth16_verify_dev): pvk the (5022,) tensor of
+        Context.groth16_prepare_verifying_key, ic (num_inputs + 1, 13), proofs (m, 51), inputs (m, num_inputs, 4) -> (m,)
+        uint8 tensor, 1 where the proof verifies."""
+        m, ni = self._verify_args(pvk, ic, proofs, inputs)
+        if out is None:
+            out = torch.empty(m, dtype=torch.uint8, device=self.device)
+        scr = self._buf("groth16_verify", self.ctx.groth16_verify_scratch_bytes(ni, m))
+        self.ctx.call_dev("bls_groth16_verify_dev", pvk.data_ptr(), ic.data_ptr(), ni, proofs.data_ptr(), inputs.data_ptr(), m, out.data_ptr(),
+                          scr.data_ptr(), self._stream())
+        return out
+
+    def groth16_verify_rlc(self, pvk, ic, proofs, inputs, rho, out=None):
+        """the randomized batch check on the device (bls_groth16_verify_rlc_dev): groth16_verify's arguments and rho (m, 4)
+        canonical FrRepr -> (1,) uint8 tensor (1 for m = 0)"""
+        m, ni = self._verify_args(pvk, ic, proofs, inputs)
+        _check(rho, nat.W_FR, "rho")
+        if rho.shape[0] != m:
+            raise ValueError("rho must have %d rows" % m)
+        if out is None:
+            out = torch.zeros(1, dtype=torch.uint8, device=self.device)
+        scr = self._buf("groth16_verify_rlc", self.ctx.groth16_verify_rlc_scratch_bytes(ni, m))
+        self.ctx.call_dev("bls_groth16_verify_rlc_dev", pvk.data_ptr(), ic.data_ptr(), ni, proofs.data_ptr(), inputs.data_ptr(), rho.data_ptr(), m,
+                          out.data_ptr(), scr.data_ptr(), self._stream())
+        return out
+
     def fr_op(self, op, a, b=None, out=None):
         """Fr element-wise operation on (n, 4) tensors (bls_fr_op_batch's ops: "add", "mul", ..., "from_repr", "into_repr")
         -> (out, ok), ok an (n,) uint8 tensor, 0 for the inverse of zero or from_repr of a value >= r.  out may be a or b."""

@@ -21,6 +21,12 @@ use std::os::raw::{c_char, c_int, c_void};
     pub h_len: usize, pub l_len: usize, pub a_len: usize, pub b_len: usize,
 }
 #[repr(C)] #[derive(Copy, Clone)] pub struct bls_g2_prepared { pub coeffs: [[bls_fq2; 3]; 68], pub infinity: u64 }
+/// bellman's PreparedVerifyingKey without ic, plus -gamma_g2 and -delta_g2 in affine form; the pads keep both prepared points
+/// 16-byte aligned (40 176 bytes)
+#[repr(C)] #[derive(Copy, Clone)] pub struct bls_groth16_pvk {
+    pub neg_gamma_g2: bls_g2_prepared, pub pad0: u64, pub neg_delta_g2: bls_g2_prepared, pub pad1: u64,
+    pub alpha_g1_beta_g2: bls_fq12, pub neg_gamma_g2_affine: bls_g2_affine, pub neg_delta_g2_affine: bls_g2_affine,
+}
 pub enum bls_ctx {}
 /// several devices of one node behind one call (include/pairing_b200.h, "several GPUs")
 pub enum bls_mgpu {}
@@ -68,6 +74,12 @@ extern "C" {
                                    input: *const bls_fr_repr, num_inputs: usize, aux: *const bls_fr_repr, num_aux: usize, a_aux_density: *const u32,
                                    b_input_density: *const u32, b_aux_density: *const u32, r: *const bls_fr_repr, s: *const bls_fr_repr, m: usize,
                                    out: *mut bls_groth16_proof) -> c_int;
+    pub fn bls_groth16_prepare_verifying_key(ctx: *mut bls_ctx, alpha_g1: *const bls_g1_affine, beta_g2: *const bls_g2_affine, gamma_g2: *const bls_g2_affine,
+                                             delta_g2: *const bls_g2_affine, out: *mut bls_groth16_pvk) -> c_int;
+    pub fn bls_groth16_verify_batch(ctx: *mut bls_ctx, pvk: *const bls_groth16_pvk, ic: *const bls_g1_affine, num_inputs: usize, proofs: *const bls_groth16_proof,
+                                    inputs: *const bls_fr_repr, m: usize, ok: *mut u8) -> c_int;
+    pub fn bls_groth16_verify_rlc_batch(ctx: *mut bls_ctx, pvk: *const bls_groth16_pvk, ic: *const bls_g1_affine, num_inputs: usize, proofs: *const bls_groth16_proof,
+                                        inputs: *const bls_fr_repr, rho: *const bls_fr_repr, m: usize, ok1: *mut u8) -> c_int;
     pub fn bls_fr_groth16_h_batch(ctx: *mut bls_ctx, a: *const bls_fr_repr, b: *const bls_fr_repr, c: *const bls_fr_repr, len: usize, m: usize, h: *mut bls_fr_repr) -> c_int;
     pub fn bls_fq12_pow_batch(ctx: *mut bls_ctx, a: *const bls_fq12, k: *const bls_fr_repr, out: *mut bls_fq12, n: usize) -> c_int;
     pub fn bls_fq12_product(ctx: *mut bls_ctx, input: *const bls_fq12, n: usize, out1: *mut bls_fq12) -> c_int;

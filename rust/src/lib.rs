@@ -208,6 +208,45 @@ impl Gpu {
         Ok(out.iter().map(|p| (marshal::g1_affine_back(&p.a), marshal::g2_affine_back(&p.b), marshal::g1_affine_back(&p.c))).collect())
     }
 
+    /// bellman's `groth16::prepare_verifying_key` without `ic` (the caller keeps it): e(alpha_g1, beta_g2) and the prepared
+    /// -gamma_g2, -delta_g2, bit-exact with bellman.  Boxed: the struct is 40 176 bytes.
+    pub fn groth16_prepare_verifying_key(&self, alpha_g1: &G1Affine, beta_g2: &G2Affine, gamma_g2: &G2Affine, delta_g2: &G2Affine)
+                                         -> Result<Box<bls_groth16_pvk>, GpuError> {
+        let (a, b, g, d) = (marshal::g1_affine(alpha_g1), marshal::g2_affine(beta_g2), marshal::g2_affine(gamma_g2), marshal::g2_affine(delta_g2));
+        let mut out: Box<bls_groth16_pvk> = Box::new(unsafe { std::mem::zeroed() });
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_groth16_prepare_verifying_key(*ctx, &a, &b, &g, &d, &mut *out) }, *ctx)?;
+        Ok(out)
+    }
+
+    /// bellman's `groth16::verify_proof` for every proof: `ic` is the vk's `ic` (num_inputs + 1 points), `inputs` the proofs'
+    /// public inputs back to back (num_inputs each, without the leading one).  `true` where the proof verifies.
+    pub fn groth16_verify_proof_batch(&self, pvk: &bls_groth16_pvk, ic: &[G1Affine], proofs: &[(G1Affine, G2Affine, G1Affine)], inputs: &[Fr])
+                                      -> Result<Vec<bool>, GpuError> {
+        assert!(!ic.is_empty() && inputs.len() == proofs.len() * (ic.len() - 1));
+        let icc: Vec<bls_g1_affine> = ic.iter().map(marshal::g1_affine).collect();
+        let pr: Vec<bls_groth16_proof> = proofs.iter().map(|(a, b, c)| bls_groth16_proof { a: marshal::g1_affine(a), b: marshal::g2_affine(b), c: marshal::g1_affine(c) }).collect();
+        let xs: Vec<bls_fr_repr> = inputs.iter().map(marshal::fr).collect();
+        let mut ok = vec![0u8; proofs.len()];
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_groth16_verify_batch(*ctx, pvk, icc.as_ptr(), ic.len() - 1, pr.as_ptr(), xs.as_ptr(), proofs.len(), ok.as_mut_ptr()) }, *ctx)?;
+        Ok(ok.iter().map(|&b| b != 0).collect())
+    }
+
+    /// bellperson's `verify_proofs_batch` with the caller's randomizers `rho` (one per proof; 0 leaves a proof out): one verdict.
+    pub fn groth16_verify_proofs_batch(&self, pvk: &bls_groth16_pvk, ic: &[G1Affine], proofs: &[(G1Affine, G2Affine, G1Affine)], inputs: &[Fr],
+                                       rho: &[FrRepr]) -> Result<bool, GpuError> {
+        assert!(!ic.is_empty() && inputs.len() == proofs.len() * (ic.len() - 1) && rho.len() == proofs.len());
+        let icc: Vec<bls_g1_affine> = ic.iter().map(marshal::g1_affine).collect();
+        let pr: Vec<bls_groth16_proof> = proofs.iter().map(|(a, b, c)| bls_groth16_proof { a: marshal::g1_affine(a), b: marshal::g2_affine(b), c: marshal::g1_affine(c) }).collect();
+        let xs: Vec<bls_fr_repr> = inputs.iter().map(marshal::fr).collect();
+        let rs: Vec<bls_fr_repr> = rho.iter().map(|r| bls_fr_repr { l: r.0 }).collect();
+        let mut ok = 0u8;
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_groth16_verify_rlc_batch(*ctx, pvk, icc.as_ptr(), ic.len() - 1, pr.as_ptr(), xs.as_ptr(), rs.as_ptr(), proofs.len(), &mut ok) }, *ctx)?;
+        Ok(ok != 0)
+    }
+
     /// `let q = Q.prepare(); ps.iter().map(|p| Bls12::pairing(p, Q))` with the one `G2Prepared` staged on the device.
     pub fn pairing_shared_q(&self, p: &[G1Affine], q: &G2Affine) -> Result<Vec<Fq12>, GpuError> {
         let pp: Vec<bls_g1_affine> = p.iter().map(marshal::g1_affine).collect();
