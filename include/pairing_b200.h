@@ -309,6 +309,47 @@ int bls_groth16_verify_batch(bls_ctx*, const bls_groth16_pvk* pvk, const bls_g1_
  * (the equation holds for the empty batch: both sides are one) when ok1 is not NULL, and does nothing else. */
 int bls_groth16_verify_rlc_batch(bls_ctx*, const bls_groth16_pvk* pvk, const bls_g1_affine* ic, size_t num_inputs, const bls_groth16_proof* proofs,
                                  const bls_fr* inputs, const bls_fr_repr* rho, size_t m, uint8_t* ok1);
+/* Groth16 parameters: bellman's groth16::generate_parameters(circuit, g1, g2, alpha, beta, gamma, delta, tau), bit-exact, with
+ * the toxic waste and the bases supplied by the caller (generate_random_parameters is the caller drawing them).
+ * The circuit: num_inputs input variables (input 0 is ONE by bellman's convention, not enforced), num_aux aux variables and
+ * num_constraints constraints, the input_i * 0 = 0 constraints the generator appends included (the prover's len).  abc holds
+ * A, B and C as KeypairAssembly records them (at_inputs / at_aux ...), variable-major: variable v (inputs, then aux) owns
+ * the terms offsets[v] .. offsets[v + 1] - 1, each a constraint index and a Montgomery bls_fr coefficient.  Terms are not
+ * merged: a variable may have several terms in one constraint, and coefficients may be zero.
+ * With n the smallest power of two >= num_constraints (1 for 0 or 1), Lq = ifft(tau^0 .. tau^(n-1)) (the Lagrange basis at
+ * tau of the omega^q), u_v = sum coeff Lq[constraint] over A's terms of v, and v_v, w_v the same over B and C:
+ *   h[i]  = [tau^i (tau^n - 1) delta^-1] g1                for i < n - 1 (never filtered)
+ *   ic[i] = [(beta u_i + alpha v_i + w_i) gamma^-1] g1     for each input i
+ *   l[i]  = [(beta u + alpha v + w) delta^-1] g1          for each aux i
+ *   a     = [u_v] g1 over every variable, inputs then aux, identities dropped (the inputs too, as in bellman)
+ *   b_g1, b_g2 = [v_v] g1, [v_v] g2 over every variable, identities dropped (one length: g1, g2 are not the identity)
+ *   vk    = alpha_g1 = [alpha] g1, beta_g1 = [beta] g1, beta_g2 = [beta] g2, gamma_g2 = [gamma] g2, delta_g1, delta_g2
+ *   a_aux_density bit i = (u of aux i != 0), b_input_density bit i = (v of input i != 0), b_aux_density bit i = (v of aux
+ *   i != 0): BitVec<u32> words as bls_groth16_prove_* takes them, unused high bits of the last word zero
+ *   lens  = [a_len, b_len];  ok = 0 iff some l[i] is the identity (bellman's SynthesisError::UnconstrainedVariable; the rest of
+ *   the key is still written), else 1.
+ * Every point is a canonical affine row; the identity is (0, one, infinity = 1).  g1 and g2 must have order r (bellman's
+ * generators do), for which [k] g is the identity exactly when k = 0.
+ * BLS_ERR_INVALID_ARGUMENT, before any work: gamma or delta zero (bellman's UnexpectedIdentity from inverse()); a scalar
+ * >= r; g1 or g2 at infinity (a difference from bellman, whose key would then have b_g1 and b_g2 of different lengths); a
+ * NULL pointer where there is something to read or write; n > 2^26, num_inputs + num_aux > 2^26 (so that every query fits
+ * the prover's m * multiexp length <= 2^26) or a matrix with 2^31 terms or more, or with terms but no variables.  The host
+ * form also rejects offsets that do not rise from 0 to nnz, a constraint index >= num_constraints and a coefficient >= r.
+ * Shared with bellman: when an input's u_i(tau) = 0 (probability about 1/r, or an adversarial tau such as a domain point
+ * omega^k), a is shorter than num_inputs + popcount(a_aux_density); bls_groth16_prove_* rejects such a key. */
+typedef struct { const uint64_t* offsets; const uint32_t* constraint; const bls_fr* coeff; size_t nnz; } bls_r1cs_matrix;  /* offsets: nv + 1 */
+typedef struct { bls_g1_affine alpha_g1, beta_g1, delta_g1; bls_g2_affine beta_g2, gamma_g2, delta_g2; } bls_groth16_vk_points;  /* 114 u64 */
+typedef struct {                                   /* host pointers for _batch, device pointers for _dev */
+  bls_groth16_vk_points* vk;
+  bls_g1_affine *ic, *h, *l, *a, *b_g1;            /* num_inputs, n - 1, num_aux, and num_inputs + num_aux for a and b_g1 */
+  bls_g2_affine* b_g2;                             /* num_inputs + num_aux */
+  uint32_t *a_aux_density, *b_input_density, *b_aux_density;   /* ceil(num_aux / 32), ceil(num_inputs / 32), ceil(num_aux / 32) */
+  uint64_t* lens;                                  /* [a_len, b_len] */
+  uint8_t* ok;
+} bls_groth16_parameters_out;
+int bls_groth16_generate_parameters_batch(bls_ctx*, const bls_r1cs_matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux,
+                                          const bls_g1_affine* g1, const bls_g2_affine* g2, const bls_fr* alpha, const bls_fr* beta,
+                                          const bls_fr* gamma, const bls_fr* delta, const bls_fr* tau, const bls_groth16_parameters_out* out);
 
 /* ------------------------------------------------------------------ device-pointer variants
  * Same semantics; every pointer is a device pointer on the context's device, the work is enqueued
@@ -394,6 +435,20 @@ int bls_groth16_verify_dev(bls_ctx*, const bls_groth16_pvk* pvk, const bls_g1_af
 size_t bls_groth16_verify_rlc_scratch_bytes(const bls_ctx*, size_t num_inputs, size_t m);
 int bls_groth16_verify_rlc_dev(bls_ctx*, const bls_groth16_pvk* pvk, const bls_g1_affine* ic, size_t num_inputs, const bls_groth16_proof* proofs,
                                const bls_fr* inputs, const bls_fr_repr* rho, size_t m, uint8_t* ok1, void* scratch, void* stream);
+/* bls_groth16_generate_parameters_batch on device pointers: the matrices' offsets, constraint and coeff arrays and every
+ * pointer of `out`; abc itself, g1, g2 and the five scalars stay in host memory, so their checks happen before any work.
+ * The matrices' contents are NOT validated up front, but every device read stays inside the caller's buffers whatever they
+ * hold (offsets are clamped to nnz, a constraint index >= num_constraints or a coefficient >= r makes its term contribute
+ * zero) and a malformed matrix sets ok = 0.  Only the first a_len rows of a and b_len rows of b_g1 and b_g2 are written.
+ * scratch: bls_groth16_generate_parameters_scratch_bytes(ctx, abc, num_constraints, num_inputs, num_aux) bytes (0 for
+ * invalid arguments): the scalars, the Lagrange basis and its transform's work region, the QAP sums, the G1 and G2 scalars
+ * and points of the exponentiations, the two wNAF tables and the normalisation's work region.  The call allocates nothing
+ * and does not synchronise. */
+size_t bls_groth16_generate_parameters_scratch_bytes(const bls_ctx*, const bls_r1cs_matrix abc[3], size_t num_constraints, size_t num_inputs,
+                                                     size_t num_aux);
+int bls_groth16_generate_parameters_dev(bls_ctx*, const bls_r1cs_matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux,
+                                        const bls_g1_affine* g1, const bls_g2_affine* g2, const bls_fr* alpha, const bls_fr* beta, const bls_fr* gamma,
+                                        const bls_fr* delta, const bls_fr* tau, const bls_groth16_parameters_out* out, void* scratch, void* stream);
 
 /* ------------------------------------------------------------------ several GPUs behind ONE call
  * Engine::miller_loop takes ALL pairs of a product in one call (mod.rs:40-102), and a Rust / C caller is one process.

@@ -459,6 +459,48 @@ struct Groth16 {
     g.check(bls_groth16_verify_rlc_batch(g.ctx(), &pvk, ic.data(), ic.size() - 1, proofs.data(), inputs.data(), rho.data(), proofs.size(), &ok));
     return ok != 0;
   }
+
+  // bellman's groth16::generate_parameters (bls_groth16_generate_parameters_batch).  Each matrix is variable-major over
+  // num_inputs + num_aux variables (offsets of nv + 1 entries), as KeypairAssembly records A, B and C.  The queries come back
+  // trimmed to a_len and b_len, so the Parameters go to create_proof unchanged, with the density bitmaps next to them.
+  // Throws on bellman's UnconstrainedVariable (ok = 0).
+  struct Matrix {
+    std::vector<uint64_t> offsets;
+    std::vector<uint32_t> constraint;
+    std::vector<bls_fr> coeff;
+  };
+  struct Parameters : Params {
+    G2AffinePoint gamma_g2;
+    std::vector<G1AffinePoint> ic;
+    std::vector<uint32_t> a_aux_density, b_input_density, b_aux_density;
+  };
+  static Parameters generate_parameters(Gpu& g, const Matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux,
+                                        const G1AffinePoint& g1, const G2AffinePoint& g2, const bls_fr& alpha, const bls_fr& beta,
+                                        const bls_fr& gamma, const bls_fr& delta, const bls_fr& tau) {
+    const size_t nv = num_inputs + num_aux;
+    bls_r1cs_matrix m[3];
+    for (int i = 0; i < 3; i++) {
+      if (abc[i].offsets.size() != nv + 1 || abc[i].constraint.size() != abc[i].coeff.size())
+        throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::generate_parameters: offsets must hold nv + 1 entries and constraint one per coeff");
+      m[i] = bls_r1cs_matrix{abc[i].offsets.data(), abc[i].constraint.data(), abc[i].coeff.data(), abc[i].coeff.size()};
+    }
+    size_t n = 1;
+    while (n < num_constraints) n <<= 1;
+    Parameters p;
+    p.h.resize(n - 1); p.l.resize(num_aux); p.a.resize(nv); p.b_g1.resize(nv); p.b_g2.resize(nv); p.ic.resize(num_inputs);
+    p.a_aux_density.resize((num_aux + 31) / 32); p.b_input_density.resize((num_inputs + 31) / 32); p.b_aux_density.resize((num_aux + 31) / 32);
+    bls_groth16_vk_points vk;
+    uint64_t lens[2] = {0, 0};
+    uint8_t ok = 0;
+    bls_groth16_parameters_out out{&vk, p.ic.data(), p.h.data(), p.l.data(), p.a.data(), p.b_g1.data(), p.b_g2.data(), p.a_aux_density.data(),
+                                   p.b_input_density.data(), p.b_aux_density.data(), lens, &ok};
+    g.check(bls_groth16_generate_parameters_batch(g.ctx(), m, num_constraints, num_inputs, num_aux, &g1, &g2, &alpha, &beta, &gamma, &delta, &tau, &out));
+    if (!ok) throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::generate_parameters: UnconstrainedVariable (an l query point is the identity)");
+    p.alpha_g1 = vk.alpha_g1; p.beta_g1 = vk.beta_g1; p.delta_g1 = vk.delta_g1;
+    p.beta_g2 = vk.beta_g2; p.gamma_g2 = vk.gamma_g2; p.delta_g2 = vk.delta_g2;
+    p.a.resize(lens[0]); p.b_g1.resize(lens[1]); p.b_g2.resize(lens[1]);
+    return p;
+  }
 };
 
 struct G1Affine {

@@ -57,6 +57,7 @@ SYMBOLS = [
     "bls_groth16_prove_batch", "bls_groth16_prove_scratch_bytes", "bls_groth16_prove_dev",
     "bls_groth16_prepare_verifying_key", "bls_groth16_verify_batch", "bls_groth16_verify_scratch_bytes", "bls_groth16_verify_dev",
     "bls_groth16_verify_rlc_batch", "bls_groth16_verify_rlc_scratch_bytes", "bls_groth16_verify_rlc_dev",
+    "bls_groth16_generate_parameters_batch", "bls_groth16_generate_parameters_scratch_bytes", "bls_groth16_generate_parameters_dev",
 ]
 
 
@@ -109,6 +110,8 @@ def load():
     for name in ("bls_groth16_verify_scratch_bytes", "bls_groth16_verify_rlc_scratch_bytes"):
         getattr(lib, name).restype = sz
         getattr(lib, name).argtypes = [vp, sz, sz]
+    lib.bls_groth16_generate_parameters_scratch_bytes.restype = sz
+    lib.bls_groth16_generate_parameters_scratch_bytes.argtypes = [vp, vp, sz, sz, sz]
     sig = {
         "bls_g2_prepare_batch": [vp, vp, vp, sz],
         "bls_miller_loop_batch": [vp, vp, vp, vp, sz],
@@ -200,6 +203,8 @@ def load():
         "bls_groth16_verify_dev": [vp, vp, vp, sz, vp, vp, sz, vp, vp, vp],
         "bls_groth16_verify_rlc_batch": [vp, vp, vp, sz, vp, vp, vp, sz, vp],
         "bls_groth16_verify_rlc_dev": [vp, vp, vp, sz, vp, vp, vp, sz, vp, vp, vp],
+        "bls_groth16_generate_parameters_batch": [vp, vp, sz, sz, sz, vp, vp, vp, vp, vp, vp, vp, vp],
+        "bls_groth16_generate_parameters_dev": [vp, vp, sz, sz, sz, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp],
     }
     lib.bls_mgpu_create.restype = vp
     lib.bls_mgpu_create.argtypes = [ctypes.POINTER(ci), ci, ctypes.POINTER(ci)]
@@ -281,6 +286,73 @@ class Groth16PvkC(ctypes.Structure):
 
 
 W_PVK = ctypes.sizeof(Groth16PvkC) // 8     # 5022 words
+
+
+class R1csMatrixC(ctypes.Structure):
+    """bls_r1cs_matrix: one of A, B, C variable-major (offsets of num_inputs + num_aux + 1 entries, then the terms)"""
+    _fields_ = [("offsets", ctypes.c_void_p), ("constraint", ctypes.c_void_p), ("coeff", ctypes.c_void_p), ("nnz", ctypes.c_size_t)]
+
+
+class Groth16VkPointsC(ctypes.Structure):
+    """bls_groth16_vk_points"""
+    _fields_ = [("alpha_g1", ctypes.c_uint64 * W_G1A), ("beta_g1", ctypes.c_uint64 * W_G1A), ("delta_g1", ctypes.c_uint64 * W_G1A),
+                ("beta_g2", ctypes.c_uint64 * W_G2A), ("gamma_g2", ctypes.c_uint64 * W_G2A), ("delta_g2", ctypes.c_uint64 * W_G2A)]
+
+
+W_VK_POINTS = ctypes.sizeof(Groth16VkPointsC) // 8      # 114 words
+VK_POINT_ROWS = (("alpha_g1", 0, W_G1A), ("beta_g1", W_G1A, W_G1A), ("delta_g1", 2 * W_G1A, W_G1A),
+                 ("beta_g2", 3 * W_G1A, W_G2A), ("gamma_g2", 3 * W_G1A + W_G2A, W_G2A), ("delta_g2", 3 * W_G1A + 2 * W_G2A, W_G2A))
+
+
+class Groth16ParametersOutC(ctypes.Structure):
+    """bls_groth16_parameters_out"""
+    _fields_ = [(name, ctypes.c_void_p) for name in ("vk", "ic", "h", "l", "a", "b_g1", "b_g2", "a_aux_density", "b_input_density",
+                                                      "b_aux_density", "lens", "ok")]
+
+
+@dataclass
+class Groth16Parameters(Groth16Params):
+    """bellman's groth16::Parameters as generate_parameters makes them: Groth16Params (its queries trimmed to a_len and
+    b_len, so it goes to groth16_prove unchanged) plus gamma_g2 ((25,) G2Affine row), ic ((num_inputs, 13)), the density
+    bitmaps (a_aux_density, b_input_density, b_aux_density) as bool arrays and ok (False: bellman's UnconstrainedVariable)."""
+    gamma_g2: object = None
+    ic: object = None
+    densities: object = None
+    ok: bool = True
+
+
+def r1cs_matrices(abc, num_constraints, nv):
+    """abc = three (offsets, constraint, coeff) triples -> contiguous numpy arrays (uint64 (nv + 1,), uint32 (nnz,), uint64
+    (nnz, 4)) and the bls_r1cs_matrix[3] array pointing at them"""
+    if len(abc) != 3:
+        raise ValueError("abc must hold the three matrices A, B and C")
+    keep, mats = [], (R1csMatrixC * 3)()
+    for i, (off, cons, coeff) in enumerate(abc):
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        cons = np.ascontiguousarray(cons, dtype=np.uint32)
+        coeff = np.ascontiguousarray(coeff, dtype=np.uint64).reshape(-1, W_FR)
+        if off.shape != (nv + 1,) or cons.shape != (coeff.shape[0],):
+            raise ValueError("matrix %d: offsets must have %d entries and constraint one per coefficient row, got %r, %r, %r"
+                             % (i, nv + 1, off.shape, cons.shape, coeff.shape))
+        keep.append((off, cons, coeff))
+        mats[i] = R1csMatrixC(_p(off), _p(cons), _p(coeff), cons.shape[0])
+    return keep, mats
+
+
+def unpack_density(words, bits):
+    """the inverse of density_words: BitVec<u32> words -> a bool array of `bits` entries"""
+    b = np.unpackbits(np.ascontiguousarray(words, dtype="<u4").view(np.uint8), bitorder="little")
+    return b[:bits].astype(bool)
+
+
+def groth16_parameters(vk, ic, h, l, a, b_g1, b_g2, dens, lens, ok, ni, na):
+    """Groth16Parameters from the outputs of bls_groth16_generate_parameters_*: vk the 114 words of bls_groth16_vk_points,
+    the queries untrimmed, dens the three word arrays (numpy), lens (a_len, b_len)"""
+    rows = {name: vk[o:o + w] for name, o, w in VK_POINT_ROWS}
+    a_len, b_len = int(lens[0]), int(lens[1])
+    densities = (unpack_density(dens[0], na), unpack_density(dens[1], ni), unpack_density(dens[2], na))
+    return Groth16Parameters(rows["alpha_g1"], rows["beta_g1"], rows["delta_g1"], rows["beta_g2"], rows["delta_g2"], h, l, a[:a_len],
+                             b_g1[:b_len], b_g2[:b_len], gamma_g2=rows["gamma_g2"], ic=ic, densities=densities, ok=bool(ok))
 
 
 def density_words(d, bits, name):
@@ -782,6 +854,42 @@ class Context:
         n = int(self._lib.bls_groth16_verify_rlc_scratch_bytes(self._ctx, num_inputs, m))
         if n == 0:
             raise ValueError("no randomized Groth16 check of m = %d proofs with num_inputs = %d" % (m, num_inputs))
+        return n
+
+    def groth16_generate_parameters(self, abc, num_constraints, num_inputs, num_aux, g1, g2, alpha, beta, gamma, delta, tau):
+        """bellman's groth16::generate_parameters (bls_groth16_generate_parameters_batch): abc three (offsets, constraint,
+        coeff) numpy triples, A, B, C variable-major over num_inputs + num_aux variables (offsets uint64, constraint uint32,
+        coeff (nnz, 4) Montgomery Fr); g1 a (13,) G1Affine row, g2 a (25,) G2Affine row; alpha .. tau (4,) Montgomery Fr.
+        Returns a Groth16Parameters."""
+        ni, na = int(num_inputs), int(num_aux)
+        nv = ni + na
+        keep, mats = r1cs_matrices(abc, num_constraints, nv)
+        g1 = _arr(np.reshape(g1, (1, -1)), W_G1A, "g1")
+        g2 = _arr(np.reshape(g2, (1, -1)), W_G2A, "g2")
+        sc = []
+        for x, name in ((alpha, "alpha"), (beta, "beta"), (gamma, "gamma"), (delta, "delta"), (tau, "tau")):
+            sc.append(_arr(np.reshape(x, (1, -1)), W_FR, name))
+        n1 = (1 << max(int(num_constraints) - 1, 0).bit_length()) - 1
+        vk = np.zeros(W_VK_POINTS, dtype=np.uint64)
+        ic, h, l = (np.zeros((k, W_G1A), dtype=np.uint64) for k in (ni, n1, na))
+        a, b_g1 = (np.zeros((nv, W_G1A), dtype=np.uint64) for _ in range(2))
+        b_g2 = np.zeros((nv, W_G2A), dtype=np.uint64)
+        dens = [np.zeros((k + 31) // 32, dtype=np.uint32) for k in (na, ni, na)]
+        lens = np.zeros(2, dtype=np.uint64)
+        ok = np.zeros(1, dtype=np.uint8)
+        out = Groth16ParametersOutC(*[_p(x) for x in (vk, ic, h, l, a, b_g1, b_g2, *dens, lens, ok)])
+        self._check(self._lib.bls_groth16_generate_parameters_batch(self._ctx, mats, num_constraints, ni, na, _p(g1), _p(g2),
+                                                                    *[_p(x) for x in sc], ctypes.byref(out)))
+        del keep
+        return groth16_parameters(vk, ic, h, l, a, b_g1, b_g2, dens, lens, ok[0], ni, na)
+
+    def groth16_generate_parameters_scratch_bytes(self, mats, num_constraints, num_inputs, num_aux):
+        """device scratch of bls_groth16_generate_parameters_dev; mats a bls_r1cs_matrix[3] (R1csMatrixC * 3); raises for
+        arguments the call would reject"""
+        n = int(self._lib.bls_groth16_generate_parameters_scratch_bytes(self._ctx, mats, num_constraints, num_inputs, num_aux))
+        if n == 0:
+            raise ValueError("no Groth16 parameters for num_constraints = %d, num_inputs = %d, num_aux = %d and these matrices"
+                             % (num_constraints, num_inputs, num_aux))
         return n
 
     def call_dev(self, name, *args):

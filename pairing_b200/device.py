@@ -268,6 +268,41 @@ class DeviceEngine:
                           self._stream())
         return out[:, :nat.W_G1A], out[:, nat.W_G1A:nat.W_G1A + nat.W_G2A], out[:, nat.W_G1A + nat.W_G2A:]
 
+    def groth16_generate_parameters(self, abc, num_constraints, num_inputs, num_aux, g1, g2, alpha, beta, gamma, delta, tau):
+        """bellman's groth16::generate_parameters on the device (bls_groth16_generate_parameters_dev): abc three (offsets,
+        constraint, coeff) contiguous CUDA tensors -- int64 (nv + 1,), int32 (nnz,), int64 (nnz, 4) -- and g1, g2, alpha ..
+        tau as for Context.groth16_generate_parameters (host memory).  Returns a Groth16Parameters whose rows are CUDA int64
+        tensors and whose densities are numpy bool arrays, so it goes to groth16_prove unchanged.  Reading a_len and b_len to
+        trim the queries synchronises the stream."""
+        ni, na = int(num_inputs), int(num_aux)
+        nv = ni + na
+        if len(abc) != 3:
+            raise ValueError("abc must hold the three matrices A, B and C")
+        mats = (nat.R1csMatrixC * 3)()
+        for i, (off, cons, coeff) in enumerate(abc):
+            ok = all(t.is_cuda and t.is_contiguous() for t in (off, cons, coeff)) and off.dtype == torch.int64 and cons.dtype == torch.int32 \
+                and coeff.dtype == torch.int64 and tuple(off.shape) == (nv + 1,) and coeff.dim() == 2 and coeff.shape[1] == nat.W_FR \
+                and tuple(cons.shape) == (coeff.shape[0],)
+            if not ok:
+                raise ValueError("matrix %d: offsets, constraint, coeff must be contiguous CUDA tensors int64 (%d,), int32 (nnz,), int64 (nnz, 4)"
+                                 % (i, nv + 1))
+            mats[i] = nat.R1csMatrixC(off.data_ptr(), cons.data_ptr(), coeff.data_ptr(), cons.shape[0])
+        host = [nat._arr(nat.np.reshape(x, (1, -1)), w, name) for x, w, name in
+                ((g1, nat.W_G1A, "g1"), (g2, nat.W_G2A, "g2"), (alpha, nat.W_FR, "alpha"), (beta, nat.W_FR, "beta"), (gamma, nat.W_FR, "gamma"),
+                 (delta, nat.W_FR, "delta"), (tau, nat.W_FR, "tau"))]
+        n1 = (1 << max(int(num_constraints) - 1, 0).bit_length()) - 1
+        e = lambda *shape: torch.zeros(shape, dtype=torch.int64, device=self.device)
+        vk, ic, h, l, a, b_g1, b_g2 = e(nat.W_VK_POINTS), e(ni, nat.W_G1A), e(n1, nat.W_G1A), e(na, nat.W_G1A), e(nv, nat.W_G1A), e(nv, nat.W_G1A), e(nv, nat.W_G2A)
+        dens = [torch.zeros((k + 31) // 32, dtype=torch.int32, device=self.device) for k in (na, ni, na)]
+        lens = e(2)
+        ok = torch.zeros(1, dtype=torch.uint8, device=self.device)
+        out = nat.Groth16ParametersOutC(*[t.data_ptr() for t in (vk, ic, h, l, a, b_g1, b_g2, *dens, lens, ok)])
+        scr = self._buf("groth16_setup", self.ctx.groth16_generate_parameters_scratch_bytes(mats, num_constraints, ni, na))
+        self.ctx.call_dev("bls_groth16_generate_parameters_dev", mats, num_constraints, ni, na, *[nat._p(x) for x in host], ctypes.byref(out),
+                          scr.data_ptr(), self._stream())
+        words = [d.cpu().numpy().view(nat.np.uint32) for d in dens]
+        return nat.groth16_parameters(vk, ic, h, l, a, b_g1, b_g2, words, lens.cpu().numpy(), int(ok.cpu()[0]), ni, na)
+
     def _verify_args(self, pvk, ic, proofs, inputs):
         if not (pvk.is_cuda and pvk.dtype == torch.int64 and tuple(pvk.shape) == (nat.W_PVK,) and pvk.is_contiguous()):
             raise ValueError("pvk must be a contiguous CUDA int64 tensor of shape (%d,)" % nat.W_PVK)

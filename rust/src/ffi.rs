@@ -27,6 +27,19 @@ use std::os::raw::{c_char, c_int, c_void};
     pub neg_gamma_g2: bls_g2_prepared, pub pad0: u64, pub neg_delta_g2: bls_g2_prepared, pub pad1: u64,
     pub alpha_g1_beta_g2: bls_fq12, pub neg_gamma_g2_affine: bls_g2_affine, pub neg_delta_g2_affine: bls_g2_affine,
 }
+/// one of A, B, C variable-major, as KeypairAssembly records it: the terms of variable v are offsets[v] .. offsets[v + 1]
+#[repr(C)] pub struct bls_r1cs_matrix { pub offsets: *const u64, pub constraint: *const u32, pub coeff: *const bls_fr_repr, pub nnz: usize }
+#[repr(C)] #[derive(Copy, Clone)] pub struct bls_groth16_vk_points {
+    pub alpha_g1: bls_g1_affine, pub beta_g1: bls_g1_affine, pub delta_g1: bls_g1_affine,
+    pub beta_g2: bls_g2_affine, pub gamma_g2: bls_g2_affine, pub delta_g2: bls_g2_affine,
+}
+#[repr(C)] pub struct bls_groth16_parameters_out {
+    pub vk: *mut bls_groth16_vk_points,
+    pub ic: *mut bls_g1_affine, pub h: *mut bls_g1_affine, pub l: *mut bls_g1_affine, pub a: *mut bls_g1_affine, pub b_g1: *mut bls_g1_affine,
+    pub b_g2: *mut bls_g2_affine,
+    pub a_aux_density: *mut u32, pub b_input_density: *mut u32, pub b_aux_density: *mut u32,
+    pub lens: *mut u64, pub ok: *mut u8,
+}
 pub enum bls_ctx {}
 /// several devices of one node behind one call (include/pairing_b200.h, "several GPUs")
 pub enum bls_mgpu {}
@@ -80,6 +93,10 @@ extern "C" {
                                     inputs: *const bls_fr_repr, m: usize, ok: *mut u8) -> c_int;
     pub fn bls_groth16_verify_rlc_batch(ctx: *mut bls_ctx, pvk: *const bls_groth16_pvk, ic: *const bls_g1_affine, num_inputs: usize, proofs: *const bls_groth16_proof,
                                         inputs: *const bls_fr_repr, rho: *const bls_fr_repr, m: usize, ok1: *mut u8) -> c_int;
+    pub fn bls_groth16_generate_parameters_batch(ctx: *mut bls_ctx, abc: *const bls_r1cs_matrix, num_constraints: usize, num_inputs: usize,
+                                                 num_aux: usize, g1: *const bls_g1_affine, g2: *const bls_g2_affine, alpha: *const bls_fr_repr,
+                                                 beta: *const bls_fr_repr, gamma: *const bls_fr_repr, delta: *const bls_fr_repr, tau: *const bls_fr_repr,
+                                                 out: *const bls_groth16_parameters_out) -> c_int;
     pub fn bls_fr_groth16_h_batch(ctx: *mut bls_ctx, a: *const bls_fr_repr, b: *const bls_fr_repr, c: *const bls_fr_repr, len: usize, m: usize, h: *mut bls_fr_repr) -> c_int;
     pub fn bls_fq12_pow_batch(ctx: *mut bls_ctx, a: *const bls_fq12, k: *const bls_fr_repr, out: *mut bls_fq12, n: usize) -> c_int;
     pub fn bls_fq12_product(ctx: *mut bls_ctx, input: *const bls_fq12, n: usize, out1: *mut bls_fq12) -> c_int;

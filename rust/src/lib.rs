@@ -247,6 +247,55 @@ impl Gpu {
         Ok(ok != 0)
     }
 
+    /// bellman's `groth16::generate_parameters(circuit, g1, g2, alpha, beta, gamma, delta, tau)` from the circuit's three
+    /// matrices as `KeypairAssembly` records them, flattened variable-major (see INTEGRATION.md): `abc[k] = (offsets, constraint,
+    /// coeff)` with `offsets` of `num_inputs + num_aux + 1` entries.  `num_constraints` counts the input constraints the generator
+    /// appends.  Returns the parameters with their queries trimmed to `a_len` / `b_len`, `gamma_g2`, `ic` and the three density
+    /// bitmaps (`a_aux`, `b_input`, `b_aux` words, as `groth16_create_proof_batch` takes them); `Err` on bellman's
+    /// `UnconstrainedVariable`, reported as `BLS_ERR_INVALID_ARGUMENT`.
+    pub fn groth16_generate_parameters(&self, abc: [(&[u64], &[u32], &[Fr]); 3], num_constraints: usize, num_inputs: usize, num_aux: usize,
+                                       g1: &G1Affine, g2: &G2Affine, alpha: &Fr, beta: &Fr, gamma: &Fr, delta: &Fr, tau: &Fr)
+                                       -> Result<(Groth16Params, G2Affine, Vec<G1Affine>, [Vec<u32>; 3]), GpuError> {
+        let nv = num_inputs + num_aux;
+        let coeffs: Vec<Vec<bls_fr_repr>> = abc.iter().map(|m| m.2.iter().map(marshal::fr).collect()).collect();
+        let mats: Vec<bls_r1cs_matrix> = abc.iter().zip(coeffs.iter()).map(|(m, c)| {
+            assert!(m.0.len() == nv + 1 && m.1.len() == c.len());
+            bls_r1cs_matrix { offsets: m.0.as_ptr(), constraint: m.1.as_ptr(), coeff: c.as_ptr(), nnz: c.len() }
+        }).collect();
+        let n = num_constraints.max(1).next_power_of_two();
+        let zero1 = bls_g1_affine { x: marshal::FQ_ZERO, y: marshal::FQ_ZERO, infinity: 1 };
+        let zero2 = bls_g2_affine { x: marshal::FQ2_ZERO, y: marshal::FQ2_ZERO, infinity: 1 };
+        let mut vk = bls_groth16_vk_points { alpha_g1: zero1, beta_g1: zero1, delta_g1: zero1, beta_g2: zero2, gamma_g2: zero2, delta_g2: zero2 };
+        let (mut ic, mut h, mut l) = (vec![zero1; num_inputs], vec![zero1; n - 1], vec![zero1; num_aux]);
+        let (mut a, mut b1, mut b2) = (vec![zero1; nv], vec![zero1; nv], vec![zero2; nv]);
+        let mut dens = [vec![0u32; (num_aux + 31) / 32], vec![0u32; (num_inputs + 31) / 32], vec![0u32; (num_aux + 31) / 32]];
+        let (mut lens, mut ok) = ([0u64; 2], 0u8);
+        let out = bls_groth16_parameters_out {
+            vk: &mut vk, ic: ic.as_mut_ptr(), h: h.as_mut_ptr(), l: l.as_mut_ptr(), a: a.as_mut_ptr(), b_g1: b1.as_mut_ptr(), b_g2: b2.as_mut_ptr(),
+            a_aux_density: dens[0].as_mut_ptr(), b_input_density: dens[1].as_mut_ptr(), b_aux_density: dens[2].as_mut_ptr(),
+            lens: lens.as_mut_ptr(), ok: &mut ok,
+        };
+        let (gg1, gg2) = (marshal::g1_affine(g1), marshal::g2_affine(g2));
+        let sc: Vec<bls_fr_repr> = [alpha, beta, gamma, delta, tau].iter().map(|x| marshal::fr(x)).collect();
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe {
+            bls_groth16_generate_parameters_batch(*ctx, mats.as_ptr(), num_constraints, num_inputs, num_aux, &gg1, &gg2, &sc[0], &sc[1], &sc[2],
+                                                  &sc[3], &sc[4], &out)
+        }, *ctx)?;
+        if ok == 0 {
+            return Err(GpuError(-1, "UnconstrainedVariable: an l query point is the identity".to_string()));
+        }
+        let g1v = |v: &[bls_g1_affine]| -> Vec<G1Affine> { v.iter().map(marshal::g1_affine_back).collect() };
+        let params = Groth16Params {
+            alpha_g1: marshal::g1_affine_back(&vk.alpha_g1), beta_g1: marshal::g1_affine_back(&vk.beta_g1),
+            delta_g1: marshal::g1_affine_back(&vk.delta_g1), beta_g2: marshal::g2_affine_back(&vk.beta_g2),
+            delta_g2: marshal::g2_affine_back(&vk.delta_g2),
+            h: g1v(&h), l: g1v(&l), a: g1v(&a[..lens[0] as usize]), b_g1: g1v(&b1[..lens[1] as usize]),
+            b_g2: b2[..lens[1] as usize].iter().map(marshal::g2_affine_back).collect(),
+        };
+        Ok((params, marshal::g2_affine_back(&vk.gamma_g2), g1v(&ic), dens))
+    }
+
     /// `let q = Q.prepare(); ps.iter().map(|p| Bls12::pairing(p, Q))` with the one `G2Prepared` staged on the device.
     pub fn pairing_shared_q(&self, p: &[G1Affine], q: &G2Affine) -> Result<Vec<Fq12>, GpuError> {
         let pp: Vec<bls_g1_affine> = p.iter().map(marshal::g1_affine).collect();
