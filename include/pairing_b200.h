@@ -351,6 +351,47 @@ int bls_groth16_generate_parameters_batch(bls_ctx*, const bls_r1cs_matrix abc[3]
                                           const bls_g1_affine* g1, const bls_g2_affine* g2, const bls_fr* alpha, const bls_fr* beta,
                                           const bls_fr* gamma, const bls_fr* delta, const bls_fr* tau, const bls_groth16_parameters_out* out);
 
+/* ------------------------------------------------------------------ KZG polynomial commitments
+ * The SRS is srs[i] = [tau^i] g in G1 for i < srs_len (affine rows), plus h and [tau] h in G2; the caller supplies all of it
+ * (the library has no RNG and no setup file), and the Fiat-Shamir challenges z_j and randomizers rho_j as well.  Polynomials
+ * are in coefficient form, p(X) = sum_{i<n} p_i X^i, Montgomery bls_fr, canonical, m polynomials back to back (p[j*n + i]:
+ * the layout bls_fr_fft_* produces).  n is any length.  Points leave as canonical affine rows (the identity is (0, one,
+ * infinity = 1)), so outputs are bit-exact whatever the summation order.  m = 0 does nothing.  BLS_ERR_INVALID_ARGUMENT,
+ * before any work: a NULL pointer where there is work, an SRS shorter than the formula indexes, sizes over the limits.
+ *
+ * commit: c[j] = sum_{i<n} p_ji srs[i].  srs_len >= n; m <= 2^16 and m * n <= 2^26 (bls_g1_msm_batch's limits). */
+int bls_kzg_commit_batch(bls_ctx*, const bls_g1_affine* srs, size_t srs_len, const bls_fr* p, size_t n, size_t m, bls_g1_affine* c);
+/* open at z_j (Montgomery bls_fr): y[j] = p_j(z_j) (Montgomery bls_fr) and proof[j] = sum_{i<n-1} q_ji srs[i] with
+ * q_j(X) = (p_j(X) - y_j) / (X - z_j), q_i = sum_{k>i} p_k z^(k-i-1): the unique [q(tau)] g.  n = 0 gives y = 0 and the
+ * identity, n = 1 gives y = p_0 and the identity.  srs_len >= n - 1; the limits of commit. */
+int bls_kzg_open_batch(bls_ctx*, const bls_g1_affine* srs, size_t srs_len, const bls_fr* p, size_t n, const bls_fr* z, size_t m, bls_fr* y,
+                       bls_g1_affine* proof);
+/* The verifying key: prepare(h) at offset 0 and prepare(-tau h) at a 16-byte aligned offset (the pads; zero), so that the
+ * verification kernel can stage both coefficient arrays by bulk copies, then g, h and -tau h in affine form.  NULL pointers
+ * give BLS_ERR_INVALID_ARGUMENT. */
+typedef struct {
+  bls_g2_prepared h_prepared;                                        /* offset 0 */
+  uint64_t pad0;
+  bls_g2_prepared neg_tau_h_prepared;                                /* offset 19 600 */
+  uint64_t pad1;
+  bls_g1_affine g;                                                   /* offset 39 200 */
+  bls_g2_affine h, neg_tau_h;                                        /* offsets 39 304, 39 504 */
+} bls_kzg_pvk;                                                       /* 39 704 B */
+int bls_kzg_prepare_verifying_key(bls_ctx*, const bls_g1_affine* g, const bls_g2_affine* h, const bls_g2_affine* tau_h, bls_kzg_pvk* out);
+/* verify, one byte per proof:
+ *   ok[j] = 1  iff  FE(ML(C_j - y_j g + z_j proof_j, h) * ML(proof_j, -tau h)) == 1   (e(C - y g, h) == e(proof, tau h - z h)),
+ * else 0; also 0 when y_j or z_j is not < r (rejected, not reduced).  A pair with a member at infinity contributes one, as in
+ * Engine::miller_loop.  Points are not validated: decode them with bls_g*_decode_batch(checked = 1).  m <= 2^26. */
+int bls_kzg_verify_batch(bls_ctx*, const bls_kzg_pvk* pvk, const bls_g1_affine* c, const bls_fr* y, const bls_fr* z, const bls_g1_affine* proof,
+                         size_t m, uint8_t* ok);
+/* randomized check, one verdict for m proofs with the caller's randomizers rho[j] (canonical bls_fr_repr, < r):
+ *   *ok1 = 1  iff  FE(ML(sum_j rho_j (C_j - y_j g + z_j proof_j), h) * ML(sum_j rho_j proof_j, -tau h)) == 1,
+ * exactly this equation (for points of order r), else 0; 0 as well when some y_j or z_j is not < r.  rho_j = 0 leaves proof j
+ * out.  The first sum is one bls_g1_msm over the 2m + 1 bases [C_0 .. C_(m-1), proof_0 .. proof_(m-1), g], so m < 2^25
+ * (2m + 1 <= 2^26, bls_g1_msm's limit).  m = 0 sets *ok1 = 1 when ok1 is not NULL. */
+int bls_kzg_verify_rlc_batch(bls_ctx*, const bls_kzg_pvk* pvk, const bls_g1_affine* c, const bls_fr* y, const bls_fr* z, const bls_g1_affine* proof,
+                             const bls_fr_repr* rho, size_t m, uint8_t* ok1);
+
 /* ------------------------------------------------------------------ device-pointer variants
  * Same semantics; every pointer is a device pointer on the context's device, the work is enqueued
  * on `stream` (a cudaStream_t, NULL = the context's own stream) and NOT synchronised.  `scratch`
@@ -449,6 +490,23 @@ size_t bls_groth16_generate_parameters_scratch_bytes(const bls_ctx*, const bls_r
 int bls_groth16_generate_parameters_dev(bls_ctx*, const bls_r1cs_matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux,
                                         const bls_g1_affine* g1, const bls_g2_affine* g2, const bls_fr* alpha, const bls_fr* beta, const bls_fr* gamma,
                                         const bls_fr* delta, const bls_fr* tau, const bls_groth16_parameters_out* out, void* scratch, void* stream);
+/* bls_kzg_* on device pointers: srs, p, z, y, c / proof, pvk (16-byte aligned), rho and ok / ok1.  Same limits.  scratch:
+ * bls_kzg_*_scratch_bytes(ctx, ...) bytes, 0 for invalid arguments -- commit: the msm scalars, the m sums and the multiexp's
+ * work region; open: the quotient coefficients, the scan's upper levels (about m n / 31 elements), the sums and the
+ * multiexp's; verify: the m G1 terms, the range flags and the normalisation's; verify_rlc: the 2m + 1 bases and scalars, the
+ * two sums and the multiexp's.  The calls allocate nothing and do not synchronise. */
+size_t bls_kzg_commit_scratch_bytes(const bls_ctx*, size_t n, size_t m);
+int bls_kzg_commit_dev(bls_ctx*, const bls_g1_affine* srs, size_t srs_len, const bls_fr* p, size_t n, size_t m, bls_g1_affine* c, void* scratch,
+                       void* stream);
+size_t bls_kzg_open_scratch_bytes(const bls_ctx*, size_t n, size_t m);
+int bls_kzg_open_dev(bls_ctx*, const bls_g1_affine* srs, size_t srs_len, const bls_fr* p, size_t n, const bls_fr* z, size_t m, bls_fr* y,
+                     bls_g1_affine* proof, void* scratch, void* stream);
+size_t bls_kzg_verify_scratch_bytes(const bls_ctx*, size_t m);
+int bls_kzg_verify_dev(bls_ctx*, const bls_kzg_pvk* pvk, const bls_g1_affine* c, const bls_fr* y, const bls_fr* z, const bls_g1_affine* proof,
+                       size_t m, uint8_t* ok, void* scratch, void* stream);
+size_t bls_kzg_verify_rlc_scratch_bytes(const bls_ctx*, size_t m);
+int bls_kzg_verify_rlc_dev(bls_ctx*, const bls_kzg_pvk* pvk, const bls_g1_affine* c, const bls_fr* y, const bls_fr* z, const bls_g1_affine* proof,
+                           const bls_fr_repr* rho, size_t m, uint8_t* ok1, void* scratch, void* stream);
 
 /* ------------------------------------------------------------------ several GPUs behind ONE call
  * Engine::miller_loop takes ALL pairs of a product in one call (mod.rs:40-102), and a Rust / C caller is one process.

@@ -503,6 +503,53 @@ struct Groth16 {
   }
 };
 
+// ------------------------------------------------------------------------------------------------ KZG commitments
+// m polynomials of n coefficients (Montgomery bls_fr) back to back in p; srs[i] = [tau^i] g.  See pairing_b200.h.
+struct Kzg {
+  using PreparedVerifyingKey = bls_kzg_pvk;
+  static size_t rows(size_t coeffs, size_t n, const char* what) {
+    if (n == 0 ? coeffs != 0 : coeffs % n) throw Error(BLS_ERR_INVALID_ARGUMENT, what);
+    return n ? coeffs / n : 0;
+  }
+  // c[j] = sum_i p[j*n + i] srs[i]; with n = 0 the number of polynomials is m
+  static std::vector<G1AffinePoint> commit(Gpu& g, const std::vector<G1AffinePoint>& srs, const std::vector<bls_fr>& p, size_t n, size_t m = 0) {
+    if (n) m = rows(p.size(), n, "Kzg::commit: p must hold m rows of n coefficients");
+    std::vector<G1AffinePoint> c(m);
+    g.check(bls_kzg_commit_batch(g.ctx(), srs.data(), srs.size(), p.data(), n, m, c.data()));
+    return c;
+  }
+  struct Opening { std::vector<bls_fr> y; std::vector<G1AffinePoint> proof; };
+  // open polynomial j at z[j]: y[j] = p_j(z_j), proof[j] = [q_j(tau)] g
+  static Opening open(Gpu& g, const std::vector<G1AffinePoint>& srs, const std::vector<bls_fr>& p, size_t n, const std::vector<bls_fr>& z) {
+    if (p.size() != n * z.size()) throw Error(BLS_ERR_INVALID_ARGUMENT, "Kzg::open: p must hold z.size() rows of n coefficients");
+    Opening o{std::vector<bls_fr>(z.size()), std::vector<G1AffinePoint>(z.size())};
+    g.check(bls_kzg_open_batch(g.ctx(), srs.data(), srs.size(), p.data(), n, z.data(), z.size(), o.y.data(), o.proof.data()));
+    return o;
+  }
+  static std::unique_ptr<PreparedVerifyingKey> prepare_verifying_key(Gpu& g, const G1AffinePoint& g1, const G2AffinePoint& h, const G2AffinePoint& tau_h) {
+    std::unique_ptr<PreparedVerifyingKey> pvk(new PreparedVerifyingKey);
+    g.check(bls_kzg_prepare_verifying_key(g.ctx(), &g1, &h, &tau_h, pvk.get()));
+    return pvk;
+  }
+  static std::vector<bool> verify(Gpu& g, const PreparedVerifyingKey& pvk, const std::vector<G1AffinePoint>& c, const std::vector<bls_fr>& y,
+                                  const std::vector<bls_fr>& z, const std::vector<G1AffinePoint>& proof) {
+    if (y.size() != c.size() || z.size() != c.size() || proof.size() != c.size())
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Kzg::verify: c, y, z and proof must have one length");
+    std::vector<uint8_t> ok(c.size());
+    g.check(bls_kzg_verify_batch(g.ctx(), &pvk, c.data(), y.data(), z.data(), proof.data(), c.size(), ok.data()));
+    return std::vector<bool>(ok.begin(), ok.end());
+  }
+  // the randomized check with the caller's randomizers rho (canonical FrRepr, one per proof)
+  static bool verify_batch(Gpu& g, const PreparedVerifyingKey& pvk, const std::vector<G1AffinePoint>& c, const std::vector<bls_fr>& y,
+                           const std::vector<bls_fr>& z, const std::vector<G1AffinePoint>& proof, const std::vector<bls_fr_repr>& rho) {
+    if (y.size() != c.size() || z.size() != c.size() || proof.size() != c.size() || rho.size() != c.size())
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Kzg::verify_batch: c, y, z, proof and rho must have one length");
+    uint8_t ok = 0;
+    g.check(bls_kzg_verify_rlc_batch(g.ctx(), &pvk, c.data(), y.data(), z.data(), proof.data(), rho.data(), c.size(), &ok));
+    return ok != 0;
+  }
+};
+
 struct G1Affine {
   static std::vector<G1PreparedPoint> prepare(const std::vector<G1AffinePoint>& p) { return p; }   // ec.rs:924-935
   // CurveAffine::mul (ec.rs:174-177)

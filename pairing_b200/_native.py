@@ -58,6 +58,9 @@ SYMBOLS = [
     "bls_groth16_prepare_verifying_key", "bls_groth16_verify_batch", "bls_groth16_verify_scratch_bytes", "bls_groth16_verify_dev",
     "bls_groth16_verify_rlc_batch", "bls_groth16_verify_rlc_scratch_bytes", "bls_groth16_verify_rlc_dev",
     "bls_groth16_generate_parameters_batch", "bls_groth16_generate_parameters_scratch_bytes", "bls_groth16_generate_parameters_dev",
+    "bls_kzg_commit_batch", "bls_kzg_commit_scratch_bytes", "bls_kzg_commit_dev", "bls_kzg_open_batch", "bls_kzg_open_scratch_bytes",
+    "bls_kzg_open_dev", "bls_kzg_prepare_verifying_key", "bls_kzg_verify_batch", "bls_kzg_verify_scratch_bytes", "bls_kzg_verify_dev",
+    "bls_kzg_verify_rlc_batch", "bls_kzg_verify_rlc_scratch_bytes", "bls_kzg_verify_rlc_dev",
 ]
 
 
@@ -112,6 +115,10 @@ def load():
         getattr(lib, name).argtypes = [vp, sz, sz]
     lib.bls_groth16_generate_parameters_scratch_bytes.restype = sz
     lib.bls_groth16_generate_parameters_scratch_bytes.argtypes = [vp, vp, sz, sz, sz]
+    for name, args in (("bls_kzg_commit_scratch_bytes", [vp, sz, sz]), ("bls_kzg_open_scratch_bytes", [vp, sz, sz]),
+                       ("bls_kzg_verify_scratch_bytes", [vp, sz]), ("bls_kzg_verify_rlc_scratch_bytes", [vp, sz])):
+        getattr(lib, name).restype = sz
+        getattr(lib, name).argtypes = args
     sig = {
         "bls_g2_prepare_batch": [vp, vp, vp, sz],
         "bls_miller_loop_batch": [vp, vp, vp, vp, sz],
@@ -205,6 +212,15 @@ def load():
         "bls_groth16_verify_rlc_dev": [vp, vp, vp, sz, vp, vp, vp, sz, vp, vp, vp],
         "bls_groth16_generate_parameters_batch": [vp, vp, sz, sz, sz, vp, vp, vp, vp, vp, vp, vp, vp],
         "bls_groth16_generate_parameters_dev": [vp, vp, sz, sz, sz, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp],
+        "bls_kzg_commit_batch": [vp, vp, sz, vp, sz, sz, vp],
+        "bls_kzg_commit_dev": [vp, vp, sz, vp, sz, sz, vp, vp, vp],
+        "bls_kzg_open_batch": [vp, vp, sz, vp, sz, vp, sz, vp, vp],
+        "bls_kzg_open_dev": [vp, vp, sz, vp, sz, vp, sz, vp, vp, vp, vp],
+        "bls_kzg_prepare_verifying_key": [vp, vp, vp, vp, vp],
+        "bls_kzg_verify_batch": [vp, vp, vp, vp, vp, vp, sz, vp],
+        "bls_kzg_verify_dev": [vp, vp, vp, vp, vp, vp, sz, vp, vp, vp],
+        "bls_kzg_verify_rlc_batch": [vp, vp, vp, vp, vp, vp, vp, sz, vp],
+        "bls_kzg_verify_rlc_dev": [vp, vp, vp, vp, vp, vp, vp, sz, vp, vp, vp],
     }
     lib.bls_mgpu_create.restype = vp
     lib.bls_mgpu_create.argtypes = [ctypes.POINTER(ci), ci, ctypes.POINTER(ci)]
@@ -286,6 +302,27 @@ class Groth16PvkC(ctypes.Structure):
 
 
 W_PVK = ctypes.sizeof(Groth16PvkC) // 8     # 5022 words
+
+
+class KzgPvkC(ctypes.Structure):
+    """bls_kzg_pvk: prepare(h) and prepare(-tau h), the pads putting both at 16-byte aligned offsets, then g, h and -tau h in
+    affine form."""
+    _fields_ = [("h_prepared", ctypes.c_uint64 * W_G2P), ("pad0", ctypes.c_uint64),
+                ("neg_tau_h_prepared", ctypes.c_uint64 * W_G2P), ("pad1", ctypes.c_uint64),
+                ("g", ctypes.c_uint64 * W_G1A), ("h", ctypes.c_uint64 * W_G2A), ("neg_tau_h", ctypes.c_uint64 * W_G2A)]
+
+
+W_KZG_PVK = ctypes.sizeof(KzgPvkC) // 8     # 4963 words
+
+
+def kzg_poly_shape(shape, srs_rows, open_):
+    """(m, n) of an (m, n, 4) coefficient array, checked against an SRS of srs_rows rows (n rows for commit, n - 1 for open)"""
+    if len(shape) != 3 or shape[2] != W_FR:
+        raise ValueError("p must have shape (m, n, 4), got %r" % (tuple(shape),))
+    m, n = int(shape[0]), int(shape[1])
+    if srs_rows < (max(n - 1, 0) if open_ else n):
+        raise ValueError("the SRS has %d points, a polynomial of %d coefficients needs %d" % (srs_rows, n, max(n - 1, 0) if open_ else n))
+    return m, n
 
 
 class R1csMatrixC(ctypes.Structure):
@@ -891,6 +928,72 @@ class Context:
             raise ValueError("no Groth16 parameters for num_constraints = %d, num_inputs = %d, num_aux = %d and these matrices"
                              % (num_constraints, num_inputs, num_aux))
         return n
+
+    # ------------------------------------------------------------------ KZG commitments
+    def kzg_commit(self, srs, p):
+        """c[j] = sum_i p[j, i] srs[i] (bls_kzg_commit_batch): srs (>= n, 13) affine rows [tau^i] g, p (m, n, 4) Montgomery
+        coefficients -> (m, 13) affine rows."""
+        srs, p = _arr(srs, W_G1A, "srs"), np.ascontiguousarray(p, dtype=np.uint64)
+        m, n = kzg_poly_shape(p.shape, srs.shape[0], False)
+        out = np.zeros((m, W_G1A), dtype=np.uint64)
+        self._check(self._lib.bls_kzg_commit_batch(self._ctx, _p(srs), srs.shape[0], _p(p), n, m, _p(out)))
+        return out
+
+    def kzg_open(self, srs, p, z):
+        """open polynomial j at z[j] (bls_kzg_open_batch): srs (>= n - 1, 13), p (m, n, 4), z (m, 4) Montgomery Fr -> (y (m, 4)
+        Montgomery p_j(z_j), proof (m, 13) affine [q_j(tau)] g)."""
+        srs, p, z = _arr(srs, W_G1A, "srs"), np.ascontiguousarray(p, dtype=np.uint64), np.ascontiguousarray(z, dtype=np.uint64)
+        m, n = kzg_poly_shape(p.shape, srs.shape[0], True)
+        if z.shape != (m, W_FR):
+            raise ValueError("z must have shape (%d, 4) uint64, got %r" % (m, z.shape))
+        y, proof = np.zeros((m, W_FR), dtype=np.uint64), np.zeros((m, W_G1A), dtype=np.uint64)
+        self._check(self._lib.bls_kzg_open_batch(self._ctx, _p(srs), srs.shape[0], _p(p), n, _p(z), m, _p(y), _p(proof)))
+        return y, proof
+
+    def kzg_prepare_verifying_key(self, g, h, tau_h):
+        """bls_kzg_prepare_verifying_key: g a (13,) G1Affine row, h and tau_h (25,) G2Affine rows -> the bls_kzg_pvk as a
+        (4963,) uint64 array (KzgPvkC's layout)."""
+        rows = [_arr(np.reshape(x, (1, -1)), w, name) for x, w, name in ((g, W_G1A, "g"), (h, W_G2A, "h"), (tau_h, W_G2A, "tau_h"))]
+        out = np.zeros(W_KZG_PVK, dtype=np.uint64)
+        self._check(self._lib.bls_kzg_prepare_verifying_key(self._ctx, *[_p(r) for r in rows], _p(out)))
+        return out
+
+    def _kzg_verify_args(self, pvk, c, y, z, proof):
+        pvk = np.ascontiguousarray(pvk, dtype=np.uint64)
+        if pvk.shape != (W_KZG_PVK,):
+            raise ValueError("pvk must be a (%d,) uint64 array, got %r" % (W_KZG_PVK, pvk.shape))
+        c, proof, y, z = _arr(c, W_G1A, "c"), _arr(proof, W_G1A, "proof"), _arr(y, W_FR, "y"), _arr(z, W_FR, "z")
+        m = c.shape[0]
+        if not (proof.shape[0] == y.shape[0] == z.shape[0] == m):
+            raise ValueError("c, y, z and proof must have the same number of rows")
+        return pvk, c, y, z, proof, m
+
+    def kzg_verify(self, pvk, c, y, z, proof):
+        """bls_kzg_verify_batch: pvk from kzg_prepare_verifying_key, c and proof (m, 13) affine rows, y and z (m, 4) Montgomery
+        Fr -> (m,) bool array."""
+        pvk, c, y, z, proof, m = self._kzg_verify_args(pvk, c, y, z, proof)
+        ok = np.zeros(m, dtype=np.uint8)
+        self._check(self._lib.bls_kzg_verify_batch(self._ctx, _p(pvk), _p(c), _p(y), _p(z), _p(proof), m, _p(ok)))
+        return ok.astype(bool)
+
+    def kzg_verify_rlc(self, pvk, c, y, z, proof, rho):
+        """the randomized check (bls_kzg_verify_rlc_batch): kzg_verify's arguments and rho (m, 4) canonical FrRepr -> one bool
+        (True for m = 0)"""
+        pvk, c, y, z, proof, m = self._kzg_verify_args(pvk, c, y, z, proof)
+        rho = np.ascontiguousarray(rho, dtype=np.uint64)
+        if rho.shape != (m, W_FR):
+            raise ValueError("rho must have shape (%d, 4) uint64, got %r" % (m, rho.shape))
+        ok = np.zeros(1, dtype=np.uint8)
+        self._check(self._lib.bls_kzg_verify_rlc_batch(self._ctx, _p(pvk), _p(c), _p(y), _p(z), _p(proof), _p(rho), m, _p(ok)))
+        return bool(ok[0])
+
+    def kzg_scratch_bytes(self, what, *args):
+        """device scratch of bls_kzg_<what>_dev: what "commit" / "open" (args n, m), "verify" / "verify_rlc" (args m); raises
+        for arguments the call would reject"""
+        b = int(getattr(self._lib, "bls_kzg_%s_scratch_bytes" % what)(self._ctx, *args))
+        if b == 0:
+            raise ValueError("no KZG %s for %r" % (what, args))
+        return b
 
     def call_dev(self, name, *args):
         """Raw access to a `*_dev` entry point: args are ints (device pointers / sizes / stream)."""

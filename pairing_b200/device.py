@@ -338,6 +338,76 @@ class DeviceEngine:
                           out.data_ptr(), scr.data_ptr(), self._stream())
         return out
 
+    # ---------------------------------------------------------------- KZG commitments
+    def _kzg_poly(self, srs, p, open_):
+        _check(srs, nat.W_G1A, "srs")
+        if not (p.is_cuda and p.dtype == torch.int64 and p.is_contiguous()):
+            raise ValueError("p must be a contiguous CUDA int64 tensor of shape (m, n, 4)")
+        return nat.kzg_poly_shape(tuple(p.shape), srs.shape[0], open_)
+
+    def kzg_commit(self, srs, p, out=None):
+        """c[j] = sum_i p[j, i] srs[i] on the device (bls_kzg_commit_dev): srs (>= n, 13), p (m, n, 4) Montgomery -> (m, 13)."""
+        m, n = self._kzg_poly(srs, p, False)
+        if out is None:
+            out = torch.empty((m, nat.W_G1A), dtype=torch.int64, device=self.device)
+        _check(out, nat.W_G1A, "out")
+        scr = self._buf("kzg", self.ctx.kzg_scratch_bytes("commit", n, m))
+        self.ctx.call_dev("bls_kzg_commit_dev", srs.data_ptr(), srs.shape[0], p.data_ptr(), n, m, out.data_ptr(), scr.data_ptr(), self._stream())
+        return out
+
+    def kzg_open(self, srs, p, z):
+        """open polynomial j at z[j] on the device (bls_kzg_open_dev): srs (>= n - 1, 13), p (m, n, 4), z (m, 4) Montgomery ->
+        (y (m, 4) Montgomery, proof (m, 13) affine)."""
+        m, n = self._kzg_poly(srs, p, True)
+        _check(z, nat.W_FR, "z")
+        if z.shape[0] != m:
+            raise ValueError("z must have %d rows" % m)
+        y = torch.empty((m, nat.W_FR), dtype=torch.int64, device=self.device)
+        proof = torch.empty((m, nat.W_G1A), dtype=torch.int64, device=self.device)
+        scr = self._buf("kzg", self.ctx.kzg_scratch_bytes("open", n, m))
+        self.ctx.call_dev("bls_kzg_open_dev", srs.data_ptr(), srs.shape[0], p.data_ptr(), n, z.data_ptr(), m, y.data_ptr(), proof.data_ptr(),
+                          scr.data_ptr(), self._stream())
+        return y, proof
+
+    def kzg_prepare_verifying_key(self, g, h, tau_h):
+        """the (4963,) bls_kzg_pvk of Context.kzg_prepare_verifying_key as a CUDA tensor (rows in host or device memory)"""
+        rows = [x.cpu().numpy() if isinstance(x, torch.Tensor) else x for x in (g, h, tau_h)]
+        return torch.from_numpy(self.ctx.kzg_prepare_verifying_key(*rows).view(nat.np.int64)).to(self.device)
+
+    def _kzg_verify_args(self, pvk, c, y, z, proof):
+        if not (pvk.is_cuda and pvk.dtype == torch.int64 and tuple(pvk.shape) == (nat.W_KZG_PVK,) and pvk.is_contiguous()):
+            raise ValueError("pvk must be a contiguous CUDA int64 tensor of shape (%d,)" % nat.W_KZG_PVK)
+        _check(c, nat.W_G1A, "c"); _check(proof, nat.W_G1A, "proof"); _check(y, nat.W_FR, "y"); _check(z, nat.W_FR, "z")
+        m = c.shape[0]
+        if not (proof.shape[0] == y.shape[0] == z.shape[0] == m):
+            raise ValueError("c, y, z and proof must have the same number of rows")
+        return m
+
+    def kzg_verify(self, pvk, c, y, z, proof, out=None):
+        """bls_kzg_verify_dev: pvk (4963,), c and proof (m, 13), y and z (m, 4) Montgomery -> (m,) uint8 tensor, 1 where the
+        opening verifies."""
+        m = self._kzg_verify_args(pvk, c, y, z, proof)
+        if out is None:
+            out = torch.empty(m, dtype=torch.uint8, device=self.device)
+        scr = self._buf("kzg_verify", self.ctx.kzg_scratch_bytes("verify", m))
+        self.ctx.call_dev("bls_kzg_verify_dev", pvk.data_ptr(), c.data_ptr(), y.data_ptr(), z.data_ptr(), proof.data_ptr(), m, out.data_ptr(),
+                          scr.data_ptr(), self._stream())
+        return out
+
+    def kzg_verify_rlc(self, pvk, c, y, z, proof, rho, out=None):
+        """the randomized check on the device (bls_kzg_verify_rlc_dev): kzg_verify's arguments and rho (m, 4) canonical
+        FrRepr -> (1,) uint8 tensor (1 for m = 0)"""
+        m = self._kzg_verify_args(pvk, c, y, z, proof)
+        _check(rho, nat.W_FR, "rho")
+        if rho.shape[0] != m:
+            raise ValueError("rho must have %d rows" % m)
+        if out is None:
+            out = torch.zeros(1, dtype=torch.uint8, device=self.device)
+        scr = self._buf("kzg_verify_rlc", self.ctx.kzg_scratch_bytes("verify_rlc", m))
+        self.ctx.call_dev("bls_kzg_verify_rlc_dev", pvk.data_ptr(), c.data_ptr(), y.data_ptr(), z.data_ptr(), proof.data_ptr(), rho.data_ptr(), m,
+                          out.data_ptr(), scr.data_ptr(), self._stream())
+        return out
+
     def fr_op(self, op, a, b=None, out=None):
         """Fr element-wise operation on (n, 4) tensors (bls_fr_op_batch's ops: "add", "mul", ..., "from_repr", "into_repr")
         -> (out, ok), ok an (n,) uint8 tensor, 0 for the inverse of zero or from_repr of a value >= r.  out may be a or b."""

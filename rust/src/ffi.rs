@@ -27,6 +27,11 @@ use std::os::raw::{c_char, c_int, c_void};
     pub neg_gamma_g2: bls_g2_prepared, pub pad0: u64, pub neg_delta_g2: bls_g2_prepared, pub pad1: u64,
     pub alpha_g1_beta_g2: bls_fq12, pub neg_gamma_g2_affine: bls_g2_affine, pub neg_delta_g2_affine: bls_g2_affine,
 }
+/// KZG verifying key: prepare(h) and prepare(-tau h) at 16-byte aligned offsets (the pads), then g, h, -tau h (39 704 bytes)
+#[repr(C)] #[derive(Copy, Clone)] pub struct bls_kzg_pvk {
+    pub h_prepared: bls_g2_prepared, pub pad0: u64, pub neg_tau_h_prepared: bls_g2_prepared, pub pad1: u64,
+    pub g: bls_g1_affine, pub h: bls_g2_affine, pub neg_tau_h: bls_g2_affine,
+}
 /// one of A, B, C variable-major, as KeypairAssembly records it: the terms of variable v are offsets[v] .. offsets[v + 1]
 #[repr(C)] pub struct bls_r1cs_matrix { pub offsets: *const u64, pub constraint: *const u32, pub coeff: *const bls_fr_repr, pub nnz: usize }
 #[repr(C)] #[derive(Copy, Clone)] pub struct bls_groth16_vk_points {
@@ -97,6 +102,16 @@ extern "C" {
                                                  num_aux: usize, g1: *const bls_g1_affine, g2: *const bls_g2_affine, alpha: *const bls_fr_repr,
                                                  beta: *const bls_fr_repr, gamma: *const bls_fr_repr, delta: *const bls_fr_repr, tau: *const bls_fr_repr,
                                                  out: *const bls_groth16_parameters_out) -> c_int;
+    pub fn bls_kzg_commit_batch(ctx: *mut bls_ctx, srs: *const bls_g1_affine, srs_len: usize, p: *const bls_fr_repr, n: usize, m: usize,
+                                c: *mut bls_g1_affine) -> c_int;
+    pub fn bls_kzg_open_batch(ctx: *mut bls_ctx, srs: *const bls_g1_affine, srs_len: usize, p: *const bls_fr_repr, n: usize, z: *const bls_fr_repr,
+                              m: usize, y: *mut bls_fr_repr, proof: *mut bls_g1_affine) -> c_int;
+    pub fn bls_kzg_prepare_verifying_key(ctx: *mut bls_ctx, g: *const bls_g1_affine, h: *const bls_g2_affine, tau_h: *const bls_g2_affine,
+                                         out: *mut bls_kzg_pvk) -> c_int;
+    pub fn bls_kzg_verify_batch(ctx: *mut bls_ctx, pvk: *const bls_kzg_pvk, c: *const bls_g1_affine, y: *const bls_fr_repr, z: *const bls_fr_repr,
+                                proof: *const bls_g1_affine, m: usize, ok: *mut u8) -> c_int;
+    pub fn bls_kzg_verify_rlc_batch(ctx: *mut bls_ctx, pvk: *const bls_kzg_pvk, c: *const bls_g1_affine, y: *const bls_fr_repr, z: *const bls_fr_repr,
+                                    proof: *const bls_g1_affine, rho: *const bls_fr_repr, m: usize, ok1: *mut u8) -> c_int;
     pub fn bls_fr_groth16_h_batch(ctx: *mut bls_ctx, a: *const bls_fr_repr, b: *const bls_fr_repr, c: *const bls_fr_repr, len: usize, m: usize, h: *mut bls_fr_repr) -> c_int;
     pub fn bls_fq12_pow_batch(ctx: *mut bls_ctx, a: *const bls_fq12, k: *const bls_fr_repr, out: *mut bls_fq12, n: usize) -> c_int;
     pub fn bls_fq12_product(ctx: *mut bls_ctx, input: *const bls_fq12, n: usize, out1: *mut bls_fq12) -> c_int;

@@ -247,6 +247,69 @@ impl Gpu {
         Ok(ok != 0)
     }
 
+    /// KZG commitments `c[j] = sum_i p[j n + i] srs[i]` for `p.len() / n` polynomials of `n` coefficients (`srs[i] = [tau^i] g`).
+    pub fn kzg_commit(&self, srs: &[G1Affine], p: &[Fr], n: usize) -> Result<Vec<G1Affine>, GpuError> {
+        assert!(n > 0 && p.len() % n == 0);
+        let s: Vec<bls_g1_affine> = srs.iter().map(marshal::g1_affine).collect();
+        let pp: Vec<bls_fr_repr> = p.iter().map(marshal::fr).collect();
+        let m = p.len() / n;
+        let zero1 = bls_g1_affine { x: marshal::FQ_ZERO, y: marshal::FQ_ZERO, infinity: 1 };
+        let mut c = vec![zero1; m];
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_kzg_commit_batch(*ctx, s.as_ptr(), s.len(), pp.as_ptr(), n, m, c.as_mut_ptr()) }, *ctx)?;
+        Ok(c.iter().map(marshal::g1_affine_back).collect())
+    }
+
+    /// KZG openings: polynomial j (`n` coefficients) at `z[j]` -> (`p_j(z_j)`, `[q_j(tau)] g`), q_j = (p_j - p_j(z_j)) / (X - z_j).
+    pub fn kzg_open(&self, srs: &[G1Affine], p: &[Fr], n: usize, z: &[Fr]) -> Result<Vec<(Fr, G1Affine)>, GpuError> {
+        assert!(p.len() == n * z.len());
+        let s: Vec<bls_g1_affine> = srs.iter().map(marshal::g1_affine).collect();
+        let pp: Vec<bls_fr_repr> = p.iter().map(marshal::fr).collect();
+        let zz: Vec<bls_fr_repr> = z.iter().map(marshal::fr).collect();
+        let m = z.len();
+        let zero1 = bls_g1_affine { x: marshal::FQ_ZERO, y: marshal::FQ_ZERO, infinity: 1 };
+        let mut y = vec![bls_fr_repr { l: [0; 4] }; m];
+        let mut proof = vec![zero1; m];
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_kzg_open_batch(*ctx, s.as_ptr(), s.len(), pp.as_ptr(), n, zz.as_ptr(), m, y.as_mut_ptr(), proof.as_mut_ptr()) }, *ctx)?;
+        Ok(y.iter().zip(proof.iter()).map(|(y, w)| (marshal::fr_back(y), marshal::g1_affine_back(w))).collect())
+    }
+
+    /// The KZG verifying key from `g`, `h` and `[tau] h`.  Boxed: the struct is 39 704 bytes.
+    pub fn kzg_prepare_verifying_key(&self, g: &G1Affine, h: &G2Affine, tau_h: &G2Affine) -> Result<Box<bls_kzg_pvk>, GpuError> {
+        let (a, b, t) = (marshal::g1_affine(g), marshal::g2_affine(h), marshal::g2_affine(tau_h));
+        let mut out: Box<bls_kzg_pvk> = Box::new(unsafe { std::mem::zeroed() });
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_kzg_prepare_verifying_key(*ctx, &a, &b, &t, &mut *out) }, *ctx)?;
+        Ok(out)
+    }
+
+    /// `e(C_j - y_j g, h) == e(proof_j, tau h - z_j h)` for every opening `(C_j, z_j, y_j, proof_j)`.
+    pub fn kzg_verify(&self, pvk: &bls_kzg_pvk, openings: &[(G1Affine, Fr, Fr, G1Affine)]) -> Result<Vec<bool>, GpuError> {
+        let c: Vec<bls_g1_affine> = openings.iter().map(|o| marshal::g1_affine(&o.0)).collect();
+        let z: Vec<bls_fr_repr> = openings.iter().map(|o| marshal::fr(&o.1)).collect();
+        let y: Vec<bls_fr_repr> = openings.iter().map(|o| marshal::fr(&o.2)).collect();
+        let w: Vec<bls_g1_affine> = openings.iter().map(|o| marshal::g1_affine(&o.3)).collect();
+        let mut ok = vec![0u8; openings.len()];
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_kzg_verify_batch(*ctx, pvk, c.as_ptr(), y.as_ptr(), z.as_ptr(), w.as_ptr(), openings.len(), ok.as_mut_ptr()) }, *ctx)?;
+        Ok(ok.iter().map(|&b| b != 0).collect())
+    }
+
+    /// The randomized check of `kzg_verify`'s openings with the caller's randomizers `rho` (one per opening; 0 leaves one out).
+    pub fn kzg_verify_batch(&self, pvk: &bls_kzg_pvk, openings: &[(G1Affine, Fr, Fr, G1Affine)], rho: &[FrRepr]) -> Result<bool, GpuError> {
+        assert!(rho.len() == openings.len());
+        let c: Vec<bls_g1_affine> = openings.iter().map(|o| marshal::g1_affine(&o.0)).collect();
+        let z: Vec<bls_fr_repr> = openings.iter().map(|o| marshal::fr(&o.1)).collect();
+        let y: Vec<bls_fr_repr> = openings.iter().map(|o| marshal::fr(&o.2)).collect();
+        let w: Vec<bls_g1_affine> = openings.iter().map(|o| marshal::g1_affine(&o.3)).collect();
+        let rs: Vec<bls_fr_repr> = rho.iter().map(|r| bls_fr_repr { l: r.0 }).collect();
+        let mut ok = 0u8;
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_kzg_verify_rlc_batch(*ctx, pvk, c.as_ptr(), y.as_ptr(), z.as_ptr(), w.as_ptr(), rs.as_ptr(), openings.len(), &mut ok) }, *ctx)?;
+        Ok(ok != 0)
+    }
+
     /// bellman's `groth16::generate_parameters(circuit, g1, g2, alpha, beta, gamma, delta, tau)` from the circuit's three
     /// matrices as `KeypairAssembly` records them, flattened variable-major (see INTEGRATION.md): `abc[k] = (offsets, constraint,
     /// coeff)` with `offsets` of `num_inputs + num_aux + 1` entries.  `num_constraints` counts the input constraints the generator
