@@ -391,6 +391,33 @@ int bls_kzg_verify_batch(bls_ctx*, const bls_kzg_pvk* pvk, const bls_g1_affine* 
  * (2m + 1 <= 2^26, bls_g1_msm's limit).  m = 0 sets *ok1 = 1 when ok1 is not NULL. */
 int bls_kzg_verify_rlc_batch(bls_ctx*, const bls_kzg_pvk* pvk, const bls_g1_affine* c, const bls_fr* y, const bls_fr* z, const bls_g1_affine* proof,
                              const bls_fr_repr* rho, size_t m, uint8_t* ok1);
+/* Openings at every point of the domain (FK20, Feist-Khovratovich "Fast amortized KZG proofs"): for m polynomials of
+ * n = 2^log_n coefficients (p[j*n + i], as above) and the domain's root omega (that of bls_fr_fft_*),
+ *   y[j*n + k] = p_j(omega^k)   and   proof[j*n + k] = what bls_kzg_open_batch(srs, p_j, z = omega^k) returns,
+ * bit for bit, for O(n log n) scalar multiplications per polynomial instead of n multiexps of length n.
+ * prepare (once per SRS and n): table (2n affine rows) = the point FFT of size 2n of w, w_t = srs[2n - 1 - t] for
+ * n < t < 2n and the identity for t <= n; srs_len >= n - 1, as for open.  n = 1 gives two identity rows.
+ * open_all: y = FFT_n(p) over Fr; c-hat = FFT_2n(p zero-padded) (2n)^-1; H = the first n of IFFT_2n(c-hat_i table_i) (without
+ * its n^-1); proof = FFT_n(H).  n = 1 gives y = p_0 and the identity.  log_n <= 24 and m * 2^(log_n + 1) <= 2^26, else
+ * BLS_ERR_INVALID_ARGUMENT, as for a NULL pointer where there is work; m = 0 does nothing.  The SRS points must have order r
+ * (see the point FFT below). */
+int bls_kzg_open_all_prepare(bls_ctx*, const bls_g1_affine* srs, size_t srs_len, int log_n, bls_g1_affine* table);
+int bls_kzg_open_all_batch(bls_ctx*, const bls_g1_affine* table, const bls_fr* p, int log_n, size_t m, bls_fr* y, bls_g1_affine* proof);
+
+/* ------------------------------------------------------------------ point FFT
+ * bellman's EvaluationDomain<Point<G>> transforms (fft, ifft, coset_fft, icoset_fft with group_mul_assign a scalar
+ * multiplication): those of bls_fr_fft_* with Fr products replaced by scalar multiplications, the same kinds, omega, g = 7 and
+ * n^-1.  E.g. BLS_FFT: out[i] = sum_j omega^(ij) in[j]; BLS_ICOSET_FFT: out[i] = g^-i n^-1 sum_j omega^(-ij) in[j].  The
+ * powers-of-tau rows [tau^i] g go to the Lagrange basis [L_i(tau)] g by BLS_IFFT.
+ * m rows of n = 2^log_n points back to back, natural order in and out; in == out is allowed.  Outputs are canonical affine
+ * rows (the identity is (0, one, infinity = 1)), so they are bit-exact whatever the butterfly order.
+ * Results are defined for inputs of order dividing r (subgroup points and the identity): any correct evaluation order, and
+ * the folding of n^-1 g^-i into one scalar, give the same element for them.  For other inputs the call returns BLS_OK with
+ * unspecified rows; like bellman, it validates nothing (decode with bls_g*_decode_batch(checked = 1)).
+ * log_n <= 26 and m * 2^log_n <= 2^26 (the multiexp's limits); outside them, for a bad kind, or a NULL pointer where there is
+ * work, BLS_ERR_INVALID_ARGUMENT before any work.  m = 0 does nothing. */
+int bls_g1_fft_batch(bls_ctx*, int kind, const bls_g1_affine* in, bls_g1_affine* out, int log_n, size_t m);
+int bls_g2_fft_batch(bls_ctx*, int kind, const bls_g2_affine* in, bls_g2_affine* out, int log_n, size_t m);
 
 /* ------------------------------------------------------------------ device-pointer variants
  * Same semantics; every pointer is a device pointer on the context's device, the work is enqueued
@@ -507,6 +534,21 @@ int bls_kzg_verify_dev(bls_ctx*, const bls_kzg_pvk* pvk, const bls_g1_affine* c,
 size_t bls_kzg_verify_rlc_scratch_bytes(const bls_ctx*, size_t m);
 int bls_kzg_verify_rlc_dev(bls_ctx*, const bls_kzg_pvk* pvk, const bls_g1_affine* c, const bls_fr* y, const bls_fr* z, const bls_g1_affine* proof,
                            const bls_fr_repr* rho, size_t m, uint8_t* ok1, void* scratch, void* stream);
+/* bls_kzg_open_all_* on device pointers: srs, table, p, y and proof.  Same limits.  scratch: prepare, the w rows and the point
+ * FFT's scratch for one row of 2n; open_all, c-hat (m 2n Fr), the Jacobian rows of the transforms (m 2n + m n points), the
+ * twiddles, the normalisation's and the Fr FFT's work regions.  0 for invalid arguments.  The calls allocate nothing and do not
+ * synchronise. */
+size_t bls_kzg_open_all_prepare_scratch_bytes(const bls_ctx*, int log_n);
+int bls_kzg_open_all_prepare_dev(bls_ctx*, const bls_g1_affine* srs, size_t srs_len, int log_n, bls_g1_affine* table, void* scratch, void* stream);
+size_t bls_kzg_open_all_scratch_bytes(const bls_ctx*, int log_n, size_t m);
+int bls_kzg_open_all_dev(bls_ctx*, const bls_g1_affine* table, const bls_fr* p, int log_n, size_t m, bls_fr* y, bls_g1_affine* proof,
+                         void* scratch, void* stream);
+/* bls_g*_fft_batch on device pointers, same arguments and limits.  scratch: bls_point_fft_scratch_bytes(ctx, degree, log_n, m)
+ * bytes (degree 1 = G1, 2 = G2; 0 for invalid arguments; the same for every kind): the m * 2^log_n Jacobian points the stages
+ * run on, the twiddles, the coset scaling and the normalisation's work region.  The call allocates nothing. */
+size_t bls_point_fft_scratch_bytes(const bls_ctx*, int degree, int log_n, size_t m);
+int bls_g1_fft_dev(bls_ctx*, int kind, const bls_g1_affine* in, bls_g1_affine* out, int log_n, size_t m, void* scratch, void* stream);
+int bls_g2_fft_dev(bls_ctx*, int kind, const bls_g2_affine* in, bls_g2_affine* out, int log_n, size_t m, void* scratch, void* stream);
 
 /* ------------------------------------------------------------------ several GPUs behind ONE call
  * Engine::miller_loop takes ALL pairs of a product in one call (mod.rs:40-102), and a Rust / C caller is one process.

@@ -548,6 +548,39 @@ struct Kzg {
     g.check(bls_kzg_verify_rlc_batch(g.ctx(), &pvk, c.data(), y.data(), z.data(), proof.data(), rho.data(), c.size(), &ok));
     return ok != 0;
   }
+  // openings at every omega^k (FK20): the table (2n rows) once per SRS and n = 2^log_n, then y[j*n + k] = p_j(omega^k) and
+  // proof[j*n + k] = open(srs, p_j, omega^k).proof for the m = p.size() / n polynomials of p
+  static std::vector<G1AffinePoint> open_all_prepare(Gpu& g, const std::vector<G1AffinePoint>& srs, int log_n) {
+    if (log_n < 0 || log_n > 24) throw Error(BLS_ERR_INVALID_ARGUMENT, "Kzg::open_all_prepare: log_n must be in 0..24");
+    std::vector<G1AffinePoint> table(size_t(2) << log_n);
+    g.check(bls_kzg_open_all_prepare(g.ctx(), srs.data(), srs.size(), log_n, table.data()));
+    return table;
+  }
+  static Opening open_all(Gpu& g, const std::vector<G1AffinePoint>& table, const std::vector<bls_fr>& p, int log_n) {
+    if (log_n < 0 || log_n > 24 || table.size() != (size_t(2) << log_n))
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Kzg::open_all: the table must hold 2n rows, n = 2^log_n <= 2^24");
+    const size_t m = rows(p.size(), size_t(1) << log_n, "Kzg::open_all: p must hold m rows of n coefficients");
+    Opening o{std::vector<bls_fr>(p.size()), std::vector<G1AffinePoint>(p.size())};
+    g.check(bls_kzg_open_all_batch(g.ctx(), table.data(), p.data(), log_n, m, o.y.data(), o.proof.data()));
+    return o;
+  }
+};
+
+// ------------------------------------------------------------------------------------------------ point FFT
+// bellman's EvaluationDomain<Point<G>>: a.size() = m * 2^log_n affine points of m rows back to back, natural order; the
+// results are canonical affine rows.  Defined for points of order r (see pairing_b200.h).
+struct PointFft {
+  template <class Aff, class Fn> static std::vector<Aff> run(Gpu& g, Fn fn, int kind, const std::vector<Aff>& a, int log_n) {
+    if (log_n < 0 || log_n > 26 || a.size() % (size_t(1) << log_n)) throw std::invalid_argument("PointFft: a.size() is not a multiple of 2^log_n");
+    std::vector<Aff> out(a.size());
+    g.check(fn(g.ctx(), kind, a.data(), out.data(), log_n, a.size() >> log_n));
+    return out;
+  }
+  static std::vector<G1AffinePoint> g1(Gpu& g, int kind, const std::vector<G1AffinePoint>& a, int log_n) { return run(g, bls_g1_fft_batch, kind, a, log_n); }
+  static std::vector<G2AffinePoint> g2(Gpu& g, int kind, const std::vector<G2AffinePoint>& a, int log_n) { return run(g, bls_g2_fft_batch, kind, a, log_n); }
+  // the Lagrange basis [L_i(tau)] g of the powers-of-tau rows [tau^i] g, i < 2^log_n
+  static std::vector<G1AffinePoint> g1_lagrange(Gpu& g, const std::vector<G1AffinePoint>& powers, int log_n) { return g1(g, BLS_IFFT, powers, log_n); }
+  static std::vector<G2AffinePoint> g2_lagrange(Gpu& g, const std::vector<G2AffinePoint>& powers, int log_n) { return g2(g, BLS_IFFT, powers, log_n); }
 };
 
 struct G1Affine {

@@ -61,6 +61,9 @@ SYMBOLS = [
     "bls_kzg_commit_batch", "bls_kzg_commit_scratch_bytes", "bls_kzg_commit_dev", "bls_kzg_open_batch", "bls_kzg_open_scratch_bytes",
     "bls_kzg_open_dev", "bls_kzg_prepare_verifying_key", "bls_kzg_verify_batch", "bls_kzg_verify_scratch_bytes", "bls_kzg_verify_dev",
     "bls_kzg_verify_rlc_batch", "bls_kzg_verify_rlc_scratch_bytes", "bls_kzg_verify_rlc_dev",
+    "bls_kzg_open_all_prepare", "bls_kzg_open_all_prepare_scratch_bytes", "bls_kzg_open_all_prepare_dev",
+    "bls_kzg_open_all_batch", "bls_kzg_open_all_scratch_bytes", "bls_kzg_open_all_dev",
+    "bls_g1_fft_batch", "bls_g2_fft_batch", "bls_point_fft_scratch_bytes", "bls_g1_fft_dev", "bls_g2_fft_dev",
 ]
 
 
@@ -117,6 +120,10 @@ def load():
     lib.bls_groth16_generate_parameters_scratch_bytes.argtypes = [vp, vp, sz, sz, sz]
     for name, args in (("bls_kzg_commit_scratch_bytes", [vp, sz, sz]), ("bls_kzg_open_scratch_bytes", [vp, sz, sz]),
                        ("bls_kzg_verify_scratch_bytes", [vp, sz]), ("bls_kzg_verify_rlc_scratch_bytes", [vp, sz])):
+        getattr(lib, name).restype = sz
+        getattr(lib, name).argtypes = args
+    for name, args in (("bls_point_fft_scratch_bytes", [vp, ci, ci, sz]), ("bls_kzg_open_all_prepare_scratch_bytes", [vp, ci]),
+                       ("bls_kzg_open_all_scratch_bytes", [vp, ci, sz])):
         getattr(lib, name).restype = sz
         getattr(lib, name).argtypes = args
     sig = {
@@ -221,6 +228,14 @@ def load():
         "bls_kzg_verify_dev": [vp, vp, vp, vp, vp, vp, sz, vp, vp, vp],
         "bls_kzg_verify_rlc_batch": [vp, vp, vp, vp, vp, vp, vp, sz, vp],
         "bls_kzg_verify_rlc_dev": [vp, vp, vp, vp, vp, vp, vp, sz, vp, vp, vp],
+        "bls_kzg_open_all_prepare": [vp, vp, sz, ci, vp],
+        "bls_kzg_open_all_prepare_dev": [vp, vp, sz, ci, vp, vp, vp],
+        "bls_kzg_open_all_batch": [vp, vp, vp, ci, sz, vp, vp],
+        "bls_kzg_open_all_dev": [vp, vp, vp, ci, sz, vp, vp, vp, vp],
+        "bls_g1_fft_batch": [vp, ci, vp, vp, ci, sz],
+        "bls_g2_fft_batch": [vp, ci, vp, vp, ci, sz],
+        "bls_g1_fft_dev": [vp, ci, vp, vp, ci, sz, vp, vp],
+        "bls_g2_fft_dev": [vp, ci, vp, vp, ci, sz, vp, vp],
     }
     lib.bls_mgpu_create.restype = vp
     lib.bls_mgpu_create.argtypes = [ctypes.POINTER(ci), ci, ctypes.POINTER(ci)]
@@ -323,6 +338,19 @@ def kzg_poly_shape(shape, srs_rows, open_):
     if srs_rows < (max(n - 1, 0) if open_ else n):
         raise ValueError("the SRS has %d points, a polynomial of %d coefficients needs %d" % (srs_rows, n, max(n - 1, 0) if open_ else n))
     return m, n
+
+
+def open_all_shape(shape, table_rows):
+    """(m, n, log_n) of an (m, n, 4) coefficient array, n a power of two, checked against a table of table_rows rows (2n)"""
+    if len(shape) != 3 or shape[2] != W_FR:
+        raise ValueError("p must have shape (m, n, 4), got %r" % (tuple(shape),))
+    m, n = int(shape[0]), int(shape[1])
+    log_n = n.bit_length() - 1
+    if n != 1 << log_n:
+        raise ValueError("the polynomial length must be a power of two, got %d" % n)
+    if table_rows != 2 * n:
+        raise ValueError("the table has %d rows, the domain of %d needs %d" % (table_rows, n, 2 * n))
+    return m, n, log_n
 
 
 class R1csMatrixC(ctypes.Structure):
@@ -987,8 +1015,58 @@ class Context:
         self._check(self._lib.bls_kzg_verify_rlc_batch(self._ctx, _p(pvk), _p(c), _p(y), _p(z), _p(proof), _p(rho), m, _p(ok)))
         return bool(ok[0])
 
+    def kzg_open_all_prepare(self, srs, log_n):
+        """the FK20 table of an SRS for the domain of n = 2^log_n (bls_kzg_open_all_prepare): srs (>= n - 1, 13) affine rows
+        [tau^i] g -> (2n, 13) affine rows"""
+        srs = _arr(srs, W_G1A, "srs")
+        n = 1 << log_n
+        if srs.shape[0] < n - 1:
+            raise ValueError("the SRS has %d points, the domain of %d needs %d" % (srs.shape[0], n, n - 1))
+        out = np.zeros((2 * n, W_G1A), dtype=np.uint64)
+        self._check(self._lib.bls_kzg_open_all_prepare(self._ctx, _p(srs), srs.shape[0], log_n, _p(out)))
+        return out
+
+    def kzg_open_all(self, table, p):
+        """open every polynomial at every omega^k (bls_kzg_open_all_batch): table (2n, 13) from kzg_open_all_prepare, p (m, n, 4)
+        Montgomery coefficients, n a power of two -> (y (m, n, 4) Montgomery p_j(omega^k), proof (m, n, 13) affine rows)."""
+        table, p = _arr(table, W_G1A, "table"), np.ascontiguousarray(p, dtype=np.uint64)
+        m, n, log_n = open_all_shape(p.shape, table.shape[0])
+        y, proof = np.zeros((m, n, W_FR), dtype=np.uint64), np.zeros((m, n, W_G1A), dtype=np.uint64)
+        self._check(self._lib.bls_kzg_open_all_batch(self._ctx, _p(table), _p(p), log_n, m, _p(y), _p(proof)))
+        return y, proof
+
+    def _point_fft(self, fn, w, kind, a):
+        kind = FFT_KINDS[kind]
+        a = np.ascontiguousarray(a, dtype=np.uint64)
+        if a.ndim not in (2, 3) or a.shape[-1] != w:
+            raise ValueError("a must have shape (n, %d) or (m, n, %d) uint64, got %r" % (w, w, a.shape))
+        n = a.shape[-2]
+        log_n = n.bit_length() - 1
+        if n != 1 << log_n:
+            raise ValueError("the row length must be a power of two, got %d" % n)
+        out = np.zeros_like(a)
+        self._check(fn(self._ctx, kind, _p(a), _p(out), log_n, a.shape[0] if a.ndim == 3 else 1))
+        return out
+
+    def g1_fft(self, kind, a):
+        """bellman's EvaluationDomain<Point<G1>> transforms: kind "fft" | "ifft" | "coset_fft" | "icoset_fft" on one row (n, 13)
+        or m rows (m, n, 13) of affine points, n a power of two -> canonical affine rows of the same shape"""
+        return self._point_fft(self._lib.bls_g1_fft_batch, W_G1A, kind, a)
+
+    def g2_fft(self, kind, a):
+        """g1_fft over G2: (n, 25) or (m, n, 25) affine rows"""
+        return self._point_fft(self._lib.bls_g2_fft_batch, W_G2A, kind, a)
+
+    def point_fft_scratch_bytes(self, degree, log_n, m=1):
+        """device scratch of bls_g<degree>_fft_dev for m rows of 2^log_n; raises for arguments the call would reject"""
+        b = int(self._lib.bls_point_fft_scratch_bytes(self._ctx, degree, log_n, m))
+        if b == 0:
+            raise ValueError("no point FFT of degree %r, log_n = %d, m = %d" % (degree, log_n, m))
+        return b
+
     def kzg_scratch_bytes(self, what, *args):
-        """device scratch of bls_kzg_<what>_dev: what "commit" / "open" (args n, m), "verify" / "verify_rlc" (args m); raises
+        """device scratch of bls_kzg_<what>_dev: what "commit" / "open" (args n, m), "verify" / "verify_rlc" (args m),
+        "open_all_prepare" (args log_n), "open_all" (args log_n, m); raises
         for arguments the call would reject"""
         b = int(getattr(self._lib, "bls_kzg_%s_scratch_bytes" % what)(self._ctx, *args))
         if b == 0:

@@ -369,6 +369,62 @@ class DeviceEngine:
                           scr.data_ptr(), self._stream())
         return y, proof
 
+    def kzg_open_all_prepare(self, srs, log_n, out=None):
+        """the FK20 table on the device (bls_kzg_open_all_prepare_dev): srs (>= n - 1, 13), n = 2^log_n -> (2n, 13)"""
+        _check(srs, nat.W_G1A, "srs")
+        n = 1 << log_n
+        if srs.shape[0] < n - 1:
+            raise ValueError("the SRS has %d points, the domain of %d needs %d" % (srs.shape[0], n, n - 1))
+        if out is None:
+            out = torch.empty((2 * n, nat.W_G1A), dtype=torch.int64, device=self.device)
+        _check(out, nat.W_G1A, "out")
+        if out.shape[0] != 2 * n:
+            raise ValueError("out must have %d rows" % (2 * n))
+        scr = self._buf("kzg_open_all_prepare", self.ctx.kzg_scratch_bytes("open_all_prepare", log_n))
+        self.ctx.call_dev("bls_kzg_open_all_prepare_dev", srs.data_ptr(), srs.shape[0], log_n, out.data_ptr(), scr.data_ptr(), self._stream())
+        return out
+
+    def kzg_open_all(self, table, p):
+        """open every polynomial at every omega^k on the device (bls_kzg_open_all_dev): table (2n, 13), p (m, n, 4) Montgomery ->
+        (y (m, n, 4) Montgomery, proof (m, n, 13) affine)"""
+        _check(table, nat.W_G1A, "table")
+        if not (p.is_cuda and p.dtype == torch.int64 and p.is_contiguous()):
+            raise ValueError("p must be a contiguous CUDA int64 tensor of shape (m, n, 4)")
+        m, n, log_n = nat.open_all_shape(tuple(p.shape), table.shape[0])
+        y = torch.empty((m, n, nat.W_FR), dtype=torch.int64, device=self.device)
+        proof = torch.empty((m, n, nat.W_G1A), dtype=torch.int64, device=self.device)
+        scr = self._buf("kzg_open_all", self.ctx.kzg_scratch_bytes("open_all", log_n, m))
+        self.ctx.call_dev("bls_kzg_open_all_dev", table.data_ptr(), p.data_ptr(), log_n, m, y.data_ptr(), proof.data_ptr(), scr.data_ptr(),
+                          self._stream())
+        return y, proof
+
+    def _point_fft(self, g2, a, kind, out):
+        w = nat.W_G2A if g2 else nat.W_G1A
+        if not (a.is_cuda and a.dtype == torch.int64 and a.dim() in (2, 3) and a.shape[-1] == w and a.is_contiguous()):
+            raise ValueError("a must be a contiguous CUDA int64 tensor of shape (n, %d) or (m, n, %d)" % (w, w))
+        n = a.shape[-2]
+        log_n = n.bit_length() - 1
+        if n != 1 << log_n:
+            raise ValueError("the row length must be a power of two, got %d" % n)
+        m = a.shape[0] if a.dim() == 3 else 1
+        if out is None:
+            out = torch.empty_like(a)
+        elif not (out.is_cuda and out.dtype == torch.int64 and out.shape == a.shape and out.is_contiguous()):
+            raise ValueError("out must be a contiguous CUDA int64 tensor of shape %r" % (tuple(a.shape),))
+        scr = self._buf("point_fft", self.ctx.point_fft_scratch_bytes(2 if g2 else 1, log_n, m))
+        self.ctx.call_dev("bls_g2_fft_dev" if g2 else "bls_g1_fft_dev", nat.FFT_KINDS[kind], a.data_ptr(), out.data_ptr(), log_n, m,
+                          scr.data_ptr(), self._stream())
+        return out
+
+    def g1_fft(self, a, kind="fft", out=None):
+        """bellman's EvaluationDomain<Point<G1>> transforms on the device: kind "fft" | "ifft" | "coset_fft" | "icoset_fft" on
+        (n, 13) or (m, n, 13) affine rows, n a power of two -> canonical affine rows.  out may be `a` itself (in place)."""
+        return self._point_fft(False, a, kind, out)
+
+    def g2_fft(self, a, kind="fft", out=None):
+        """g1_fft over G2: (n, 25) or (m, n, 25) affine rows"""
+        return self._point_fft(True, a, kind, out)
+
     def kzg_prepare_verifying_key(self, g, h, tau_h):
         """the (4963,) bls_kzg_pvk of Context.kzg_prepare_verifying_key as a CUDA tensor (rows in host or device memory)"""
         rows = [x.cpu().numpy() if isinstance(x, torch.Tensor) else x for x in (g, h, tau_h)]

@@ -112,6 +112,11 @@ extern "C" {
                                 proof: *const bls_g1_affine, m: usize, ok: *mut u8) -> c_int;
     pub fn bls_kzg_verify_rlc_batch(ctx: *mut bls_ctx, pvk: *const bls_kzg_pvk, c: *const bls_g1_affine, y: *const bls_fr_repr, z: *const bls_fr_repr,
                                     proof: *const bls_g1_affine, rho: *const bls_fr_repr, m: usize, ok1: *mut u8) -> c_int;
+    pub fn bls_kzg_open_all_prepare(ctx: *mut bls_ctx, srs: *const bls_g1_affine, srs_len: usize, log_n: c_int, table: *mut bls_g1_affine) -> c_int;
+    pub fn bls_kzg_open_all_batch(ctx: *mut bls_ctx, table: *const bls_g1_affine, p: *const bls_fr_repr, log_n: c_int, m: usize, y: *mut bls_fr_repr,
+                                  proof: *mut bls_g1_affine) -> c_int;
+    pub fn bls_g1_fft_batch(ctx: *mut bls_ctx, kind: c_int, input: *const bls_g1_affine, out: *mut bls_g1_affine, log_n: c_int, m: usize) -> c_int;
+    pub fn bls_g2_fft_batch(ctx: *mut bls_ctx, kind: c_int, input: *const bls_g2_affine, out: *mut bls_g2_affine, log_n: c_int, m: usize) -> c_int;
     pub fn bls_fr_groth16_h_batch(ctx: *mut bls_ctx, a: *const bls_fr_repr, b: *const bls_fr_repr, c: *const bls_fr_repr, len: usize, m: usize, h: *mut bls_fr_repr) -> c_int;
     pub fn bls_fq12_pow_batch(ctx: *mut bls_ctx, a: *const bls_fq12, k: *const bls_fr_repr, out: *mut bls_fq12, n: usize) -> c_int;
     pub fn bls_fq12_product(ctx: *mut bls_ctx, input: *const bls_fq12, n: usize, out1: *mut bls_fq12) -> c_int;

@@ -310,6 +310,52 @@ impl Gpu {
         Ok(ok != 0)
     }
 
+    /// The FK20 table (2n rows) of `srs` for the domain of `n = 2^log_n`, for `kzg_open_all`.
+    pub fn kzg_open_all_prepare(&self, srs: &[G1Affine], log_n: u32) -> Result<Vec<G1Affine>, GpuError> {
+        let s: Vec<bls_g1_affine> = srs.iter().map(marshal::g1_affine).collect();
+        let zero1 = bls_g1_affine { x: marshal::FQ_ZERO, y: marshal::FQ_ZERO, infinity: 1 };
+        let mut table = vec![zero1; 2usize << log_n];
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_kzg_open_all_prepare(*ctx, s.as_ptr(), s.len(), log_n as i32, table.as_mut_ptr()) }, *ctx)?;
+        Ok(table.iter().map(marshal::g1_affine_back).collect())
+    }
+
+    /// KZG openings of every polynomial of `p` (`p.len() / n` rows of `n = 2^log_n` coefficients) at every `omega^k`:
+    /// entry `j n + k` is (`p_j(omega^k)`, the proof `kzg_open` returns for `z = omega^k`).
+    pub fn kzg_open_all(&self, table: &[G1Affine], p: &[Fr], log_n: u32) -> Result<Vec<(Fr, G1Affine)>, GpuError> {
+        let n = 1usize << log_n;
+        assert!(table.len() == 2 * n && p.len() % n == 0);
+        let t: Vec<bls_g1_affine> = table.iter().map(marshal::g1_affine).collect();
+        let pp: Vec<bls_fr_repr> = p.iter().map(marshal::fr).collect();
+        let zero1 = bls_g1_affine { x: marshal::FQ_ZERO, y: marshal::FQ_ZERO, infinity: 1 };
+        let mut y = vec![bls_fr_repr { l: [0; 4] }; p.len()];
+        let mut proof = vec![zero1; p.len()];
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_kzg_open_all_batch(*ctx, t.as_ptr(), pp.as_ptr(), log_n as i32, p.len() / n, y.as_mut_ptr(), proof.as_mut_ptr()) }, *ctx)?;
+        Ok(y.iter().zip(proof.iter()).map(|(y, w)| (marshal::fr_back(y), marshal::g1_affine_back(w))).collect())
+    }
+
+    /// bellman's `EvaluationDomain<Point<G1>>` transforms (`kind`: 0 fft, 1 ifft, 2 coset_fft, 3 icoset_fft) of the
+    /// `a.len() / 2^log_n` rows of `a`; `ifft` of `[tau^i] g` is the Lagrange basis `[L_i(tau)] g`.
+    pub fn g1_fft(&self, kind: i32, a: &[G1Affine], log_n: u32) -> Result<Vec<G1Affine>, GpuError> {
+        assert!(a.len() % (1usize << log_n) == 0);
+        let x: Vec<bls_g1_affine> = a.iter().map(marshal::g1_affine).collect();
+        let mut out = x.clone();
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_g1_fft_batch(*ctx, kind as i32, x.as_ptr(), out.as_mut_ptr(), log_n as i32, a.len() >> log_n) }, *ctx)?;
+        Ok(out.iter().map(marshal::g1_affine_back).collect())
+    }
+
+    /// `g1_fft` over G2.
+    pub fn g2_fft(&self, kind: i32, a: &[G2Affine], log_n: u32) -> Result<Vec<G2Affine>, GpuError> {
+        assert!(a.len() % (1usize << log_n) == 0);
+        let x: Vec<bls_g2_affine> = a.iter().map(marshal::g2_affine).collect();
+        let mut out = x.clone();
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_g2_fft_batch(*ctx, kind as i32, x.as_ptr(), out.as_mut_ptr(), log_n as i32, a.len() >> log_n) }, *ctx)?;
+        Ok(out.iter().map(marshal::g2_affine_back).collect())
+    }
+
     /// bellman's `groth16::generate_parameters(circuit, g1, g2, alpha, beta, gamma, delta, tau)` from the circuit's three
     /// matrices as `KeypairAssembly` records them, flattened variable-major (see INTEGRATION.md): `abc[k] = (offsets, constraint,
     /// coeff)` with `offsets` of `num_inputs + num_aux + 1` entries.  `num_constraints` counts the input constraints the generator
