@@ -423,7 +423,8 @@ int bls_g2_fft_batch(bls_ctx*, int kind, const bls_g2_affine* in, bls_g2_affine*
  * Same semantics; every pointer is a device pointer on the context's device, the work is enqueued
  * on `stream` (a cudaStream_t, NULL = the context's own stream) and NOT synchronised.  `scratch`
  * arguments are caller-provided device buffers of the stated size (so no allocation happens on the
- * timed path). */
+ * timed path).  A scratch pointer must be 256-byte aligned, as cudaMalloc and torch return it: the
+ * calls place their regions at multiples of 256 bytes from it, and some kernels use vector loads. */
 int bls_g2_prepare_dev(bls_ctx*, const bls_g2_affine* q, bls_g2_prepared* out, size_t n, void* stream);
 int bls_miller_loop_dev(bls_ctx*, const bls_g1_affine* p, const bls_g2_affine* q, bls_fq12* out, size_t n, void* stream);
 int bls_miller_loop_prepared_dev(bls_ctx*, const bls_g1_affine* p, const bls_g2_prepared* q, bls_fq12* out, size_t n, void* stream);
