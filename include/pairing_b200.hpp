@@ -28,6 +28,7 @@
 #include <vector>
 
 #include "pairing_b200.h"
+#include "pairing_b200_mpc.h"
 
 namespace pairing_b200 {
 
@@ -477,11 +478,71 @@ struct Groth16 {
   static Parameters generate_parameters(Gpu& g, const Matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux,
                                         const G1AffinePoint& g1, const G2AffinePoint& g2, const bls_fr& alpha, const bls_fr& beta,
                                         const bls_fr& gamma, const bls_fr& delta, const bls_fr& tau) {
+    return build_key(abc, num_constraints, num_inputs, num_aux, "Groth16::generate_parameters",
+                     "UnconstrainedVariable (an l query point is the identity)", [&](const bls_r1cs_matrix* m, const bls_groth16_parameters_out* out) {
+      g.check(bls_groth16_generate_parameters_batch(g.ctx(), m, num_constraints, num_inputs, num_aux, &g1, &g2, &alpha, &beta, &gamma, &delta, &tau, out));
+    });
+  }
+
+  // phase2's MPCParameters::new (bls_groth16_mpc_new_batch): the circuit's key from powersoftau's prepare_phase2 rows for the
+  // domain of num_constraints (phase1.n of them; h: n - 1), before any contribution.  Throws on UnconstrainedVariable and on a
+  // transcript whose b_g1 and b_g2 disagree on the identity (ok = 0).
+  struct Phase1 {
+    G1AffinePoint alpha_g1, beta_g1;
+    G2AffinePoint beta_g2;
+    std::vector<G1AffinePoint> coeffs_g1, alpha_coeffs_g1, beta_coeffs_g1;
+    std::vector<G2AffinePoint> coeffs_g2;
+    std::vector<G1AffinePoint> h;
+  };
+  static Parameters mpc_new(Gpu& g, const Matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux, const Phase1& phase1,
+                            const G1AffinePoint& g1, const G2AffinePoint& g2) {
+    const size_t n = phase1.coeffs_g1.size();
+    if (phase1.alpha_coeffs_g1.size() != n || phase1.beta_coeffs_g1.size() != n || phase1.coeffs_g2.size() != n || phase1.h.size() + 1 != n)
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::mpc_new: the transcript needs n rows per coefficient set and n - 1 h rows");
+    const bls_groth16_phase1 ph{phase1.alpha_g1, phase1.beta_g1, phase1.beta_g2, phase1.coeffs_g1.data(), phase1.alpha_coeffs_g1.data(),
+                                phase1.beta_coeffs_g1.data(), phase1.coeffs_g2.data(), phase1.h.data(), n};
+    return build_key(abc, num_constraints, num_inputs, num_aux, "Groth16::mpc_new",
+                     "UnconstrainedVariable (an l query point is the identity) or b_g1 and b_g2 disagreeing on the identity", [&](const bls_r1cs_matrix* m, const bls_groth16_parameters_out* out) {
+      g.check(bls_groth16_mpc_new_batch(g.ctx(), m, num_constraints, num_inputs, num_aux, &ph, &g1, &g2, out));
+    });
+  }
+
+  // phase2's MPCParameters::contribute (bls_groth16_mpc_contribute_batch) for the caller's secret delta, s and r =
+  // hash_to_g2(transcript): h and l multiplied by delta^-1, delta_g1 and delta_g2 by delta, in place.  Returns the public key.
+  static bls_groth16_mpc_pubkey mpc_contribute(Gpu& g, Parameters& p, const bls_fr& delta, const G1AffinePoint& s, const G2AffinePoint& r) {
+    bls_groth16_vk_points vk{p.alpha_g1, p.beta_g1, p.delta_g1, p.beta_g2, p.gamma_g2, p.delta_g2};
+    bls_groth16_mpc_pubkey pk;
+    g.check(bls_groth16_mpc_contribute_batch(g.ctx(), &delta, &s, &r, &vk, p.h.data(), p.h.size(), p.l.data(), p.l.size(), p.h.data(), p.l.data(), &pk));
+    p.delta_g1 = vk.delta_g1;
+    p.delta_g2 = vk.delta_g2;
+    return pk;
+  }
+
+  // phase2's MPCParameters::verify (bls_groth16_mpc_verify_batch): before = the key of mpc_new, after = the contributed key,
+  // pks the contributions in order, rho_h / rho_l the caller's randomizers (one per h and l row).
+  static bool mpc_verify(Gpu& g, const Parameters& before, const Parameters& after, const std::vector<bls_groth16_mpc_pubkey>& pks,
+                         const std::vector<bls_fr_repr>& rho_h, const std::vector<bls_fr_repr>& rho_l) {
+    if (rho_h.size() != before.h.size() || rho_l.size() != before.l.size())
+      throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::mpc_verify: one randomizer per h and l row");
+    auto key = [](const Parameters& p) {
+      return bls_groth16_key{{p.alpha_g1, p.beta_g1, p.delta_g1, p.beta_g2, p.gamma_g2, p.delta_g2}, p.ic.data(), p.h.data(), p.l.data(), p.a.data(),
+                             p.b_g1.data(), p.b_g2.data(), p.ic.size(), p.h.size(), p.l.size(), p.a.size(), p.b_g1.size()};
+    };
+    const bls_groth16_key kb = key(before), ka = key(after);
+    uint8_t ok = 0;
+    g.check(bls_groth16_mpc_verify_batch(g.ctx(), &kb, &ka, pks.data(), pks.size(), rho_h.data(), rho_l.data(), &ok));
+    return ok != 0;
+  }
+
+ private:
+  template <class Call>
+  static Parameters build_key(const Matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux, const char* who, const char* not_ok,
+                              Call call) {
     const size_t nv = num_inputs + num_aux;
     bls_r1cs_matrix m[3];
     for (int i = 0; i < 3; i++) {
       if (abc[i].offsets.size() != nv + 1 || abc[i].constraint.size() != abc[i].coeff.size())
-        throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::generate_parameters: offsets must hold nv + 1 entries and constraint one per coeff");
+        throw Error(BLS_ERR_INVALID_ARGUMENT, std::string(who) + ": offsets must hold nv + 1 entries and constraint one per coeff");
       m[i] = bls_r1cs_matrix{abc[i].offsets.data(), abc[i].constraint.data(), abc[i].coeff.data(), abc[i].coeff.size()};
     }
     size_t n = 1;
@@ -494,8 +555,8 @@ struct Groth16 {
     uint8_t ok = 0;
     bls_groth16_parameters_out out{&vk, p.ic.data(), p.h.data(), p.l.data(), p.a.data(), p.b_g1.data(), p.b_g2.data(), p.a_aux_density.data(),
                                    p.b_input_density.data(), p.b_aux_density.data(), lens, &ok};
-    g.check(bls_groth16_generate_parameters_batch(g.ctx(), m, num_constraints, num_inputs, num_aux, &g1, &g2, &alpha, &beta, &gamma, &delta, &tau, &out));
-    if (!ok) throw Error(BLS_ERR_INVALID_ARGUMENT, "Groth16::generate_parameters: UnconstrainedVariable (an l query point is the identity)");
+    call(m, &out);
+    if (!ok) throw Error(BLS_ERR_INVALID_ARGUMENT, std::string(who) + ": " + not_ok);
     p.alpha_g1 = vk.alpha_g1; p.beta_g1 = vk.beta_g1; p.delta_g1 = vk.delta_g1;
     p.beta_g2 = vk.beta_g2; p.gamma_g2 = vk.gamma_g2; p.delta_g2 = vk.delta_g2;
     p.a.resize(lens[0]); p.b_g1.resize(lens[1]); p.b_g2.resize(lens[1]);

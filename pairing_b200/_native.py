@@ -4,6 +4,7 @@ The product path has no CPU fallback: if the CUDA library is missing or no devic
 entry point raises.  Nothing here imports or calls the oracle.
 """
 import ctypes
+import dataclasses
 import os
 from dataclasses import dataclass
 
@@ -65,6 +66,10 @@ SYMBOLS = [
     "bls_kzg_open_all_batch", "bls_kzg_open_all_scratch_bytes", "bls_kzg_open_all_dev",
     "bls_g1_fft_batch", "bls_g2_fft_batch", "bls_point_fft_scratch_bytes", "bls_g1_fft_dev", "bls_g2_fft_dev",
 ]
+# every symbol include/pairing_b200_mpc.h declares (tests/test_gpu_groth16_mpc.py checks that header against this list)
+MPC_SYMBOLS = ["bls_groth16_mpc_new_batch", "bls_groth16_mpc_new_scratch_bytes", "bls_groth16_mpc_new_dev",
+               "bls_groth16_mpc_contribute_batch", "bls_groth16_mpc_contribute_scratch_bytes", "bls_groth16_mpc_contribute_dev",
+               "bls_groth16_mpc_verify_batch", "bls_groth16_mpc_verify_scratch_bytes", "bls_groth16_mpc_verify_dev"]
 
 
 class BlsError(RuntimeError):
@@ -116,8 +121,13 @@ def load():
     for name in ("bls_groth16_verify_scratch_bytes", "bls_groth16_verify_rlc_scratch_bytes"):
         getattr(lib, name).restype = sz
         getattr(lib, name).argtypes = [vp, sz, sz]
-    lib.bls_groth16_generate_parameters_scratch_bytes.restype = sz
-    lib.bls_groth16_generate_parameters_scratch_bytes.argtypes = [vp, vp, sz, sz, sz]
+    for name in ("bls_groth16_generate_parameters_scratch_bytes", "bls_groth16_mpc_new_scratch_bytes"):
+        getattr(lib, name).restype = sz
+        getattr(lib, name).argtypes = [vp, vp, sz, sz, sz]
+    lib.bls_groth16_mpc_contribute_scratch_bytes.restype = sz
+    lib.bls_groth16_mpc_contribute_scratch_bytes.argtypes = [vp, sz, sz]
+    lib.bls_groth16_mpc_verify_scratch_bytes.restype = sz
+    lib.bls_groth16_mpc_verify_scratch_bytes.argtypes = [vp, vp, vp, sz]
     for name, args in (("bls_kzg_commit_scratch_bytes", [vp, sz, sz]), ("bls_kzg_open_scratch_bytes", [vp, sz, sz]),
                        ("bls_kzg_verify_scratch_bytes", [vp, sz]), ("bls_kzg_verify_rlc_scratch_bytes", [vp, sz])):
         getattr(lib, name).restype = sz
@@ -236,6 +246,12 @@ def load():
         "bls_g2_fft_batch": [vp, ci, vp, vp, ci, sz],
         "bls_g1_fft_dev": [vp, ci, vp, vp, ci, sz, vp, vp],
         "bls_g2_fft_dev": [vp, ci, vp, vp, ci, sz, vp, vp],
+        "bls_groth16_mpc_new_batch": [vp, vp, sz, sz, sz, vp, vp, vp, vp],
+        "bls_groth16_mpc_new_dev": [vp, vp, sz, sz, sz, vp, vp, vp, vp, vp, vp],
+        "bls_groth16_mpc_contribute_batch": [vp, vp, vp, vp, vp, vp, sz, vp, sz, vp, vp, vp],
+        "bls_groth16_mpc_contribute_dev": [vp, vp, vp, vp, vp, vp, sz, vp, sz, vp, vp, vp, vp, vp],
+        "bls_groth16_mpc_verify_batch": [vp, vp, vp, vp, sz, vp, vp, vp],
+        "bls_groth16_mpc_verify_dev": [vp, vp, vp, vp, sz, vp, vp, vp, vp, vp],
     }
     lib.bls_mgpu_create.restype = vp
     lib.bls_mgpu_create.argtypes = [ctypes.POINTER(ci), ci, ctypes.POINTER(ci)]
@@ -384,6 +400,87 @@ class Groth16Parameters(Groth16Params):
     ic: object = None
     densities: object = None
     ok: bool = True
+
+
+@dataclass
+class Groth16Phase1:
+    """powersoftau's prepare_phase2 output for a domain of n points (bls_groth16_phase1): alpha_g1, beta_g1 ((13,) G1Affine
+    rows), beta_g2 ((25,)), the rows coeffs_g1, alpha_coeffs_g1, beta_coeffs_g1 ((n, 13)), coeffs_g2 ((n, 25)) and h
+    ((n - 1, 13)).  numpy uint64 arrays for Context.groth16_mpc_new, CUDA int64 tensors (the rows) for DeviceEngine's."""
+    alpha_g1: object
+    beta_g1: object
+    beta_g2: object
+    coeffs_g1: object
+    alpha_coeffs_g1: object
+    beta_coeffs_g1: object
+    coeffs_g2: object
+    h: object
+
+
+class Groth16Phase1C(ctypes.Structure):
+    """bls_groth16_phase1"""
+    _fields_ = [("alpha_g1", ctypes.c_uint64 * W_G1A), ("beta_g1", ctypes.c_uint64 * W_G1A), ("beta_g2", ctypes.c_uint64 * W_G2A),
+                ("coeffs_g1", ctypes.c_void_p), ("alpha_coeffs_g1", ctypes.c_void_p), ("beta_coeffs_g1", ctypes.c_void_p),
+                ("coeffs_g2", ctypes.c_void_p), ("h", ctypes.c_void_p), ("n", ctypes.c_size_t)]
+
+
+W_MPC_PUBKEY = 3 * W_G1A + 2 * W_G2A      # bls_groth16_mpc_pubkey: delta_after, s, s_delta (G1), r, r_delta (G2)
+MPC_PUBKEY_ROWS = (("delta_after", 0, W_G1A), ("s", W_G1A, W_G1A), ("s_delta", 2 * W_G1A, W_G1A), ("r", 3 * W_G1A, W_G2A),
+                   ("r_delta", 3 * W_G1A + W_G2A, W_G2A))
+
+
+class Groth16KeyC(ctypes.Structure):
+    """bls_groth16_key: bellman's Parameters<Bls12>, the vk by value and the queries by pointer"""
+    _fields_ = [("vk", Groth16VkPointsC)] + [(n, ctypes.c_void_p) for n in ("ic", "h", "l", "a", "b_g1", "b_g2")] + \
+               [(n, ctypes.c_size_t) for n in ("ic_len", "h_len", "l_len", "a_len", "b_len")]
+
+
+def vk_points(params, row=lambda x: x):
+    """the 114 words of bls_groth16_vk_points from a Groth16Parameters' vk rows (row(x) turns a row into numpy)"""
+    return np.concatenate([np.ascontiguousarray(row(getattr(params, name)), dtype=np.uint64).reshape(-1) for name, _, _ in VK_POINT_ROWS])
+
+
+def groth16_key_c(params, ptr, length, row=lambda x: x):
+    """the bls_groth16_key struct of a Groth16Parameters: vk by value, ptr(query) and length(query)"""
+    c = Groth16KeyC()
+    vk = vk_points(params, row)
+    ctypes.memmove(ctypes.byref(c.vk), vk.ctypes.data, vk.nbytes)
+    for name in ("ic", "h", "l", "a", "b_g1", "b_g2"):
+        setattr(c, name, ptr(getattr(params, name)))
+    if length(params.b_g1) != length(params.b_g2):
+        raise ValueError("b_g1 and b_g2 must have the same length")
+    c.ic_len, c.h_len, c.l_len, c.a_len, c.b_len = (length(getattr(params, q)) for q in ("ic", "h", "l", "a", "b_g1"))
+    return c
+
+
+def contributed(params, vk, h, l):
+    """params with the delta points of vk (114 words) and the new h and l queries"""
+    rows = {name: vk[o:o + w] for name, o, w in VK_POINT_ROWS}
+    return dataclasses.replace(params, delta_g1=rows["delta_g1"], delta_g2=rows["delta_g2"], h=h, l=l)
+
+
+def domain_size(num_constraints):
+    """n of the constraint system's domain: the smallest power of two >= num_constraints, 1 for 0 or 1 constraints"""
+    return 1 << max(int(num_constraints) - 1, 0).bit_length()
+
+
+def groth16_phase1_c(phase1, num_constraints, ptr, length):
+    """the bls_groth16_phase1 struct: the vk points by value, ptr(rows) for the row sets; raises when a row set does not have
+    the domain's n (h: n - 1) rows"""
+    c = Groth16Phase1C()
+    for name, w in (("alpha_g1", W_G1A), ("beta_g1", W_G1A), ("beta_g2", W_G2A)):
+        row = np.ascontiguousarray(getattr(phase1, name), dtype=np.uint64).reshape(-1)
+        if row.shape != (w,):
+            raise ValueError("%s must be one row of %d uint64, got %r" % (name, w, row.shape))
+        getattr(c, name)[:] = [int(x) for x in row]
+    n = domain_size(num_constraints)
+    for name in ("coeffs_g1", "alpha_coeffs_g1", "beta_coeffs_g1", "coeffs_g2", "h"):
+        rows = getattr(phase1, name)
+        if length(rows) != (n - 1 if name == "h" else n):
+            raise ValueError("%s must have %d rows for %d constraints, got %d" % (name, n - 1 if name == "h" else n, num_constraints, length(rows)))
+        setattr(c, name, ptr(rows))
+    c.n = n
+    return c
 
 
 def r1cs_matrices(abc, num_constraints, nv):
@@ -934,7 +1031,17 @@ class Context:
         sc = []
         for x, name in ((alpha, "alpha"), (beta, "beta"), (gamma, "gamma"), (delta, "delta"), (tau, "tau")):
             sc.append(_arr(np.reshape(x, (1, -1)), W_FR, name))
-        n1 = (1 << max(int(num_constraints) - 1, 0).bit_length()) - 1
+        bufs, out = self._parameters_out(num_constraints, ni, na)
+        self._check(self._lib.bls_groth16_generate_parameters_batch(self._ctx, mats, num_constraints, ni, na, _p(g1), _p(g2),
+                                                                    *[_p(x) for x in sc], ctypes.byref(out)))
+        del keep
+        return groth16_parameters(*bufs[:-1], bufs[-1][0], ni, na)
+
+    @staticmethod
+    def _parameters_out(num_constraints, ni, na):
+        """zeroed host buffers of a key (vk, ic, h, l, a, b_g1, b_g2, densities, lens, ok) and the bls_groth16_parameters_out
+        pointing at them"""
+        nv, n1 = ni + na, domain_size(num_constraints) - 1
         vk = np.zeros(W_VK_POINTS, dtype=np.uint64)
         ic, h, l = (np.zeros((k, W_G1A), dtype=np.uint64) for k in (ni, n1, na))
         a, b_g1 = (np.zeros((nv, W_G1A), dtype=np.uint64) for _ in range(2))
@@ -943,10 +1050,71 @@ class Context:
         lens = np.zeros(2, dtype=np.uint64)
         ok = np.zeros(1, dtype=np.uint8)
         out = Groth16ParametersOutC(*[_p(x) for x in (vk, ic, h, l, a, b_g1, b_g2, *dens, lens, ok)])
-        self._check(self._lib.bls_groth16_generate_parameters_batch(self._ctx, mats, num_constraints, ni, na, _p(g1), _p(g2),
-                                                                    *[_p(x) for x in sc], ctypes.byref(out)))
+        return (vk, ic, h, l, a, b_g1, b_g2, dens, lens, ok), out
+
+    def groth16_mpc_new(self, abc, num_constraints, num_inputs, num_aux, phase1, g1, g2):
+        """phase2's MPCParameters::new (bls_groth16_mpc_new_batch): the circuit's key from a phase-1 transcript, before any
+        contribution.  abc, num_constraints, num_inputs, num_aux, g1 and g2 as for groth16_generate_parameters; phase1 a
+        Groth16Phase1 of numpy rows for the domain of num_constraints.  Returns a Groth16Parameters (ok False: an l row at the
+        identity, or b_g1 and b_g2 disagreeing on the identity)."""
+        ni, na = int(num_inputs), int(num_aux)
+        keep, mats = r1cs_matrices(abc, num_constraints, ni + na)
+        g1 = _arr(np.reshape(g1, (1, -1)), W_G1A, "g1")
+        g2 = _arr(np.reshape(g2, (1, -1)), W_G2A, "g2")
+        rows = {name: _arr(getattr(phase1, name), W_G2A if name == "coeffs_g2" else W_G1A, name)
+                for name in ("coeffs_g1", "alpha_coeffs_g1", "beta_coeffs_g1", "coeffs_g2", "h")}
+        ph = groth16_phase1_c(Groth16Phase1(phase1.alpha_g1, phase1.beta_g1, phase1.beta_g2, **rows), num_constraints, _p, len)
+        bufs, out = self._parameters_out(num_constraints, ni, na)
+        self._check(self._lib.bls_groth16_mpc_new_batch(self._ctx, mats, num_constraints, ni, na, ctypes.byref(ph), _p(g1), _p(g2),
+                                                        ctypes.byref(out)))
+        del keep, rows
+        return groth16_parameters(*bufs[:-1], bufs[-1][0], ni, na)
+
+    def groth16_mpc_contribute(self, params, delta, s, r):
+        """phase2's MPCParameters::contribute (bls_groth16_mpc_contribute_batch): params a Groth16Parameters (numpy), delta a
+        (4,) Montgomery Fr (canonical, nonzero), s a (13,) G1Affine row, r a (25,) G2Affine row (hash_to_g2 of the caller's
+        transcript).  Returns (the contributed Groth16Parameters, the (89,) bls_groth16_mpc_pubkey words)."""
+        delta = _arr(np.reshape(delta, (1, -1)), W_FR, "delta")
+        s = _arr(np.reshape(s, (1, -1)), W_G1A, "s")
+        r = _arr(np.reshape(r, (1, -1)), W_G2A, "r")
+        vk = vk_points(params)
+        h, l = _arr(params.h, W_G1A, "h").copy(), _arr(params.l, W_G1A, "l").copy()
+        pk = np.zeros(W_MPC_PUBKEY, dtype=np.uint64)
+        self._check(self._lib.bls_groth16_mpc_contribute_batch(self._ctx, _p(delta), _p(s), _p(r), _p(vk), _p(h), len(h), _p(l), len(l), _p(h),
+                                                               _p(l), _p(pk)))
+        return contributed(params, vk, h, l), pk
+
+    def groth16_mpc_contribute_scratch_bytes(self, h_len, l_len):
+        n = int(self._lib.bls_groth16_mpc_contribute_scratch_bytes(self._ctx, h_len, l_len))
+        if n == 0:
+            raise ValueError("no contribution for h_len = %d, l_len = %d" % (h_len, l_len))
+        return n
+
+    def groth16_mpc_verify(self, before, after, pubkeys, rho_h, rho_l):
+        """phase2's MPCParameters::verify (bls_groth16_mpc_verify_batch): before the key of groth16_mpc_new, after the
+        contributed key, pubkeys (k, 89) words, rho_h (h_len, 4) and rho_l (l_len, 4) canonical randomizers.  Returns a bool."""
+        keep = [np.ascontiguousarray(getattr(k, q), dtype=np.uint64) for k in (before, after) for q in ("ic", "h", "l", "a", "b_g1", "b_g2")]
+        kb, ka = (groth16_key_c(k, _p, len) for k in (before, after))
+        pk = _arr(np.reshape(pubkeys, (-1, W_MPC_PUBKEY)), W_MPC_PUBKEY, "pubkeys")
+        rh, rl = _arr(np.reshape(rho_h, (-1, W_FR)), W_FR, "rho_h"), _arr(np.reshape(rho_l, (-1, W_FR)), W_FR, "rho_l")
+        ok = np.zeros(1, dtype=np.uint8)
+        self._check(self._lib.bls_groth16_mpc_verify_batch(self._ctx, ctypes.byref(kb), ctypes.byref(ka), _p(pk), len(pk), _p(rh), _p(rl), _p(ok)))
         del keep
-        return groth16_parameters(vk, ic, h, l, a, b_g1, b_g2, dens, lens, ok[0], ni, na)
+        return bool(ok[0])
+
+    def groth16_mpc_verify_scratch_bytes(self, before_c, after_c, k):
+        n = int(self._lib.bls_groth16_mpc_verify_scratch_bytes(self._ctx, ctypes.byref(before_c), ctypes.byref(after_c), k))
+        if n == 0:
+            raise ValueError("no verification for these keys and k = %d" % k)
+        return n
+
+    def groth16_mpc_new_scratch_bytes(self, mats, num_constraints, num_inputs, num_aux):
+        """device scratch of bls_groth16_mpc_new_dev; mats a bls_r1cs_matrix[3]; raises for arguments the call would reject"""
+        n = int(self._lib.bls_groth16_mpc_new_scratch_bytes(self._ctx, mats, num_constraints, num_inputs, num_aux))
+        if n == 0:
+            raise ValueError("no phase-2 key for num_constraints = %d, num_inputs = %d, num_aux = %d and these matrices"
+                             % (num_constraints, num_inputs, num_aux))
+        return n
 
     def groth16_generate_parameters_scratch_bytes(self, mats, num_constraints, num_inputs, num_aux):
         """device scratch of bls_groth16_generate_parameters_dev; mats a bls_r1cs_matrix[3] (R1csMatrixC * 3); raises for

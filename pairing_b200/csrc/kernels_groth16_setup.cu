@@ -28,8 +28,12 @@
 //      (rank = prefix of the word + popcount below the bit) with the identities dropped, and `ok`.
 // g1 and g2 have order r (bellman's generators), so [k]g is the identity exactly when k = 0: the filters are decided on the
 // scalars, which is bellman's rule on the points.
+//
+// bls_groth16_mpc_new_* (phase 2 of the ceremony, include/pairing_b200_mpc.h) shares steps 6 and 7: its sums are points
+// from the start (k_mpc_qap, k_mpc_fix and k_mpc_combine below), so the filters are decided on the Jacobian sums.
 #include "curve_io.cuh"
 #include "fr.cuh"
+#include "../../include/pairing_b200_mpc.h"
 
 #define GS_TPB 128
 #define GS_SCAN_TPB 1024
@@ -386,6 +390,218 @@ __global__ void __launch_bounds__(GS_TPB) k_gs_emit(const uint64_t* p1, const ui
   gs_emit_row<Fp>(dst, p1 + (size_t)G1_W * t);
 }
 
+// ---- phase 2 of the ceremony (bls_groth16_mpc_new_*) ----------------------------------------------------------------------
+// The group-valued k_gs_qap: the same per-chunk walk over the CSR terms, with c [L_q(tau)] (a scalar multiplication of the
+// transcript's row q) in place of c L_q(tau).  Points cannot be added atomically, so a run of a variable that crosses chunk
+// boundaries goes to one of the chunk's two boundary slots (0: the variable started in an earlier chunk, 1: it starts here
+// and goes on), and k_mpc_fix adds the slots up.  One launch per (matrix, transcript row set):
+//   G1: A x coeffs -> a, A x beta_coeffs, B x coeffs -> b_g1, B x alpha_coeffs, C x coeffs; G2: B x coeffs_g2 -> b_g2.
+// k_mpc_combine then adds the three ext parts, and decides densities and flags on the Jacobian sums (z = 0 is exact).
+#define MPC_CHUNK 12                       /* terms per thread: 4 groups of MPC_K_G1, 6 of MPC_K_G2 */
+#define MPC_K_G1 3                         /* points per thread of the wNAF runner, as the library's wNAF kernels */
+#define MPC_K_G2 2
+#define MPC_MAXT 8                         /* wNAF table entries: window <= 4 */
+#define MPC_INCONSISTENT 4u                /* flags bit: bg1_v and bg2_v disagree on being the identity */
+
+template <class F, int K> struct MpcTables {
+  Jac<F> t[K][MPC_MAXT];
+  __device__ __forceinline__ Jac<F> get(int j, int e) const { return t[j][e]; }
+};
+
+// c (Montgomery) as the integer min(c, r - c); neg when r - c was taken.  -1 and -2^k become 1 and 2^k: the window and the
+// doublings follow the short value.  [r - c](-P) = [c] P holds for P of order r.
+__device__ __forceinline__ Scalar mpc_signed(const Fr& c, bool& neg) {
+  const Fr x = gs_into_repr(c), y = gs_into_repr(fr_neg(c));
+  neg = !fr_geq(y, x);
+  Scalar s;
+#pragma unroll
+  for (int i = 0; i < 8; i++) s.v[i] = neg ? y.v[i] : x.v[i];
+  return s;
+}
+
+// a boundary or complete run of variable v from chunk k: complete variables go to sums[v], the others to a boundary slot
+template <class F>
+__device__ __forceinline__ void mpc_flush(const GsMat& M, size_t v, size_t k, size_t chunks, const Jac<F>& sum, uint64_t* sums, uint64_t* bnd) {
+  const int PW = 3 * FW<F>::W;
+  size_t kf = M.ov(v) / MPC_CHUNK;
+  if (kf >= chunks) kf = chunks - 1;
+  const size_t o1 = M.ov(v + 1);
+  if (o1 && kf == (o1 - 1) / MPC_CHUNK) st_jac(sums + (size_t)PW * v, sum);
+  else st_jac(bnd + (size_t)PW * (2 * k + (kf < k ? 0 : 1)), sum);
+}
+
+// Thread k sums c [rows[q]] over the terms kC .. kC + C - 1 of M, K terms at a time through the decoupled wNAF runner.
+template <class F, bool IS_G2, int K>
+__global__ void __launch_bounds__(GS_TPB, IS_G2 ? 3 : 4)
+    k_mpc_qap(GsMat M, size_t nv, size_t nc, const uint64_t* rows, uint64_t* sums, uint64_t* bnd, uint32_t* flags) {
+  const int W = FW<F>::W, PW = 3 * W;
+  const size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const size_t chunks = (M.nnz + MPC_CHUNK - 1) / MPC_CHUNK;
+  // no early return: the runner votes with __ballot_sync, so every lane runs the same number of groups
+  const bool active = k < chunks && nv != 0;
+  const size_t e0 = k * MPC_CHUNK, e1 = !active ? e0 : e0 + MPC_CHUNK < M.nnz ? e0 + MPC_CHUNK : M.nnz;
+  Jac<F> sum;
+  pt_set_zero(sum);
+  if (active) {
+    st_jac(bnd + (size_t)PW * 2 * k, sum);
+    st_jac(bnd + (size_t)PW * (2 * k + 1), sum);
+  }
+  uint32_t bad = 0;
+  bool open = false;                                        // sum holds terms of v
+  size_t v = active ? gs_last_at(M, 0, nv - 1, e0) : 0;
+  size_t o1 = active ? M.ov(v + 1) : 0;
+#pragma unroll 1
+  for (size_t g = e0; g < e0 + MPC_CHUNK; g += K) {
+    MpcTables<F, K> table;
+    int8_t digits[K][260];
+    WnafState<K> st;
+    Jac<F> res[K];
+    bool neg[K];
+#pragma unroll 1
+    for (int j = 0; j < K; j++) {
+      const size_t e = g + j;
+      Scalar s;
+#pragma unroll
+      for (int i = 0; i < 8; i++) s.v[i] = 0;
+      Jac<F> b;
+      pt_set_zero(b);
+      neg[j] = false;
+      if (e < e1) {
+        const uint32_t q = M.cons[e];
+        const Fr c = gs_ld_fr(M.coeff + 4 * e);
+        if (q >= nc || fr_geq(c, fr_modulus())) bad = 1;   // a malformed term contributes the identity
+        else {
+          s = mpc_signed(c, neg[j]);
+          Aff<F> a;
+          ld_aff(a, rows + (size_t)(2 * W + 1) * q);
+          if (!a.inf) { b.x = a.x; b.y = a.y; f_set_one(b.z); }
+        }
+      }
+      const int w = IS_G2 ? g2_window_for_bits(scalar_num_bits(s)) : g1_window_for_bits(scalar_num_bits(s)), tsize = 1 << (w - 1);
+      Jac<F> dbl = b;
+      pt_double(dbl);
+#pragma unroll 1
+      for (int t = 0; t < MPC_MAXT; t++) {
+        if (t < tsize) { table.t[j][t] = b; if (t + 1 < tsize) pt_add(b, dbl); }
+      }
+      st.i[j] = wnaf_form(digits[j], s, w) - 1;
+      st.found[j] = false; st.doubled[j] = false;
+      pt_set_zero(res[j]);
+    }
+    pt_wnaf_run_lazy<F, K>(res, table, digits, st);
+#pragma unroll 1
+    for (int j = 0; j < K; j++) {
+      const size_t e = g + j;
+      if (e >= e1) break;
+      while (e >= o1 && v + 1 < nv) {                       // the run of v ends before term e
+        if (open) mpc_flush<F>(M, v, k, chunks, sum, sums, bnd);
+        open = false;
+        pt_set_zero(sum);
+        v = gs_last_at(M, v + 1, nv - 1, e);
+        o1 = M.ov(v + 1);
+      }
+      if (e >= o1) continue;                                // past the last variable: only malformed offsets get here
+      if (neg[j]) pt_negate(res[j]);
+      pt_add(sum, res[j]);
+      open = true;
+    }
+  }
+  if (open) mpc_flush<F>(M, v, k, chunks, sum, sums, bnd);
+  if (bad) atomicOr(flags, GS_BAD_CSR);
+}
+
+// One block per variable: the identity for a variable without terms; for one whose terms cross chunk boundaries, slot 1 of
+// its first chunk plus slot 0 of every later chunk it reaches, strided over the block's threads.  A variable with all terms in
+// one chunk was stored by k_mpc_qap.
+template <class F>
+__global__ void __launch_bounds__(GS_TPB) k_mpc_fix(GsMat M, size_t nv, uint64_t* bnd, uint64_t* sums) {
+  const int PW = 3 * FW<F>::W;
+  const size_t v = blockIdx.x;
+  const int tid = threadIdx.x;
+  if (v >= nv) return;                                      // block-uniform, as every return before the barrier
+  Jac<F> s;
+  pt_set_zero(s);
+  const size_t o0 = M.ov(v), o1 = M.ov(v + 1);
+  if (o1 <= o0) {
+    if (tid == 0) st_jac(sums + (size_t)PW * v, s);
+    return;
+  }
+  const size_t chunks = (M.nnz + MPC_CHUNK - 1) / MPC_CHUNK, kl = (o1 - 1) / MPC_CHUNK;
+  size_t kf = o0 / MPC_CHUNK;
+  if (kf >= chunks) kf = chunks - 1;
+  if (kf == kl) return;
+  if (tid == 0) ld_jac(s, bnd + (size_t)PW * (2 * kf + 1));
+#pragma unroll 1
+  for (size_t k = kf + 1 + tid; k <= kl; k += GS_TPB) {
+    Jac<F> t;
+    ld_jac(t, bnd + (size_t)PW * 2 * k);
+    pt_add(s, t);
+  }
+  // each thread's partial into the slot of the first chunk it read (no other thread reads it), then thread 0 adds them up
+  const size_t span = kl - kf;
+  if (tid && (size_t)tid < span) st_jac(bnd + (size_t)PW * 2 * (kf + 1 + tid), s);
+  __syncthreads();
+  if (tid) return;
+#pragma unroll 1
+  for (size_t l = 1; l < GS_TPB && l < span; l++) {
+    Jac<F> t;
+    ld_jac(t, bnd + (size_t)PW * 2 * (kf + 1 + l));
+    pt_add(s, t);
+  }
+  st_jac(sums + (size_t)PW * v, s);
+}
+
+// One thread per variable: ext = A x beta_coeffs + B x alpha_coeffs + C x coeffs into the ic | l block of the G1 batch, the
+// density ballots (a != O, bg1 != O), and the flags: malformed offsets, an l row at the identity (phase2's
+// UnconstrainedVariable), bg1 and bg2 disagreeing on the identity.
+__global__ void __launch_bounds__(GS_TPB) k_mpc_combine(GsMats mats, size_t ni, size_t nv, const uint64_t* x1, uint64_t* ext, const uint64_t* a,
+                                                        const uint64_t* b1, const uint64_t* b2, uint32_t* wa, uint32_t* wb, uint32_t* flags) {
+  const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  bool nz_a = false, nz_b = false;
+  if (t < nv) {
+    uint32_t bad = 0;
+#pragma unroll
+    for (int m = 0; m < 3; m++) {
+      const GsMat& M = mats.m[m];
+      const uint64_t lo = M.off[t], hi = M.off[t + 1];
+      if (lo > hi || hi > M.nnz || (t == 0 && lo != 0) || (t + 1 == nv && hi != M.nnz)) bad |= GS_BAD_CSR;
+    }
+    Jac<Fp> e, x;
+    ld_jac(e, x1 + (size_t)G1_W * t);
+    ld_jac(x, x1 + (size_t)G1_W * (nv + t));
+    pt_add(e, x);
+    ld_jac(x, x1 + (size_t)G1_W * (2 * nv + t));
+    pt_add(e, x);
+    st_jac(ext + (size_t)G1_W * t, e);
+    if (t >= ni && pt_is_zero(e)) bad |= GS_UNCONSTRAINED;
+    Fp z;
+    ld_F(z, a + (size_t)G1_W * t + 2 * FW<Fp>::W);
+    nz_a = !f_is_zero(z);
+    ld_F(z, b1 + (size_t)G1_W * t + 2 * FW<Fp>::W);
+    nz_b = !f_is_zero(z);
+    Fp2 z2;
+    ld_F(z2, b2 + (size_t)G2_W * t + 2 * FW<Fp2>::W);
+    if (nz_b == f_is_zero(z2)) bad |= MPC_INCONSISTENT;
+    if (bad) atomicOr(flags, bad);
+  }
+  const uint32_t ba = __ballot_sync(0xffffffffu, nz_a), bb = __ballot_sync(0xffffffffu, nz_b);
+  if ((threadIdx.x & 31) == 0 && t < nv) { wa[t >> 5] = ba; wb[t >> 5] = bb; }
+}
+
+// affine rows -> Jacobian rows (the identity as (0, 1, 0))
+template <class F>
+__global__ void __launch_bounds__(GS_TPB) k_mpc_load(const uint64_t* in, size_t count, uint64_t* out) {
+  const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= count) return;
+  const int W = FW<F>::W;
+  Aff<F> a;
+  ld_aff(a, in + (size_t)(2 * W + 1) * t);
+  Jac<F> r;
+  pt_set_zero(r);
+  if (!a.inf) { r.x = a.x; r.y = a.y; f_set_one(r.z); }
+  st_jac(out + (size_t)(3 * W) * t, r);
+}
+
 // ---- host side ----------------------------------------------------------------------------------------------------------
 
 static size_t gs_align(size_t x) { return (x + 255) & ~(size_t)255; }
@@ -431,6 +647,14 @@ static bool gs_fr_canonical_nonzero(const bls_fr* x, bool& zero) {
   return false;
 }
 
+static bool gs_out_ok(const bls_groth16_parameters_out* out, size_t ni, size_t na, const GsPlan& p) {
+  if (!out || !out->vk || !out->lens || !out->ok) return false;
+  if ((ni && (!out->ic || !out->b_input_density)) || (na && (!out->l || !out->a_aux_density || !out->b_aux_density))) return false;
+  if (p.n1 && !out->h) return false;
+  if (p.nv && (!out->a || !out->b_g1 || !out->b_g2)) return false;
+  return true;
+}
+
 static bool gs_args_ok(const bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc, size_t ni, size_t na, const bls_g1_affine* g1,
                        const bls_g2_affine* g2, const bls_fr* const sc[5], const bls_groth16_parameters_out* out, GsPlan& p) {
   if (!gs_shape_ok(ctx, abc, nc, ni, na, p)) return false;
@@ -440,11 +664,7 @@ static bool gs_args_ok(const bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc
     if (!sc[i] || !gs_fr_canonical_nonzero(sc[i], zero)) return false;
     if (zero && (i == GS_GAMMA || i == GS_DELTA)) return false;            // bellman's UnexpectedIdentity from inverse()
   }
-  if (!out || !out->vk || !out->lens || !out->ok) return false;
-  if ((ni && (!out->ic || !out->b_input_density)) || (na && (!out->l || !out->a_aux_density || !out->b_aux_density))) return false;
-  if (p.n1 && !out->h) return false;
-  if (p.nv && (!out->a || !out->b_g1 || !out->b_g2)) return false;
-  return true;
+  return gs_out_ok(out, ni, na, p);
 }
 
 static size_t gs_layout(bls_ctx* ctx, GsPlan& p) {
@@ -564,13 +784,11 @@ static bool gs_matrices_ok(const bls_r1cs_matrix* abc, size_t nc, size_t nv) {
   return true;
 }
 
-static int gs_host(bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc, size_t ni, size_t na, const bls_g1_affine* g1, const bls_g2_affine* g2,
-                   const bls_fr* const sc5[5], const bls_groth16_parameters_out* out) {
-  GsPlan p;
-  if (!gs_args_ok(ctx, abc, nc, ni, na, g1, g2, sc5, out, p)) return BLS_ERR_INVALID_ARGUMENT;
-  if (!gs_matrices_ok(abc, nc, p.nv)) return BLS_ERR_INVALID_ARGUMENT;
-  USE_DEVICE(ctx);
-  if (!gs_layout(ctx, p)) return BLS_ERR_CUDA;
+// The host forms: the matrices and a staging buffer for the outputs on the device, dev(matrices, outputs, scratch) for the
+// _dev form's work, then the outputs back (of the queries a, b_g1 and b_g2 only the rows the compaction wrote).
+template <class Dev>
+static int gs_host_run(bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t ni, size_t na, const GsPlan& p, size_t scratch,
+                       const bls_groth16_parameters_out* out, Dev dev) {
   const size_t ga = sizeof(bls_g1_affine), g2a = sizeof(bls_g2_affine), nv = p.nv;
   H2D(o0, abc[0].offsets, (nv + 1) * sizeof(uint64_t));
   H2D(o1, abc[1].offsets, (nv + 1) * sizeof(uint64_t));
@@ -589,7 +807,7 @@ static int gs_host(bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc, size_t n
                f_b1 = take(nv * ga), f_b2 = take(nv * g2a), f_da = take(wx * 4), f_dbi = take(wi * 4), f_dba = take(wx * 4), f_lens = take(16),
                f_ok = take(1);
   DALLOC(dout, o);
-  DALLOC(dscr, p.total);
+  DALLOC(dscr, scratch);
   char* d = (char*)dout.p;
   bls_groth16_parameters_out dp{(bls_groth16_vk_points*)(d + f_vk), (bls_g1_affine*)(d + f_ic), (bls_g1_affine*)(d + f_h), (bls_g1_affine*)(d + f_l),
                                 (bls_g1_affine*)(d + f_a), (bls_g1_affine*)(d + f_b1), (bls_g2_affine*)(d + f_b2), (uint32_t*)(d + f_da),
@@ -597,7 +815,7 @@ static int gs_host(bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc, size_t n
   bls_r1cs_matrix dm[3] = {{(const uint64_t*)o0.p, (const uint32_t*)c0.p, (const bls_fr*)k0.p, abc[0].nnz},
                            {(const uint64_t*)o1.p, (const uint32_t*)c1.p, (const bls_fr*)k1.p, abc[1].nnz},
                            {(const uint64_t*)o2.p, (const uint32_t*)c2.p, (const bls_fr*)k2.p, abc[2].nnz}};
-  TRY(gs_dev_impl(ctx, dm, nc, ni, na, g1, g2, sc5, &dp, dscr.p, ctx->stream));
+  TRY(dev(dm, &dp, dscr.p));
   uint64_t lens[2];
   CK(cudaMemcpyAsync(lens, dp.lens, sizeof(lens), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaMemcpyAsync(out->vk, dp.vk, sizeof(bls_groth16_vk_points), cudaMemcpyDeviceToHost, ctx->stream));
@@ -622,6 +840,154 @@ static int gs_host(bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc, size_t n
   return BLS_OK;
 }
 
+static int gs_host(bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc, size_t ni, size_t na, const bls_g1_affine* g1, const bls_g2_affine* g2,
+                   const bls_fr* const sc5[5], const bls_groth16_parameters_out* out) {
+  GsPlan p;
+  if (!gs_args_ok(ctx, abc, nc, ni, na, g1, g2, sc5, out, p)) return BLS_ERR_INVALID_ARGUMENT;
+  if (!gs_matrices_ok(abc, nc, p.nv)) return BLS_ERR_INVALID_ARGUMENT;
+  USE_DEVICE(ctx);
+  if (!gs_layout(ctx, p)) return BLS_ERR_CUDA;
+  return gs_host_run(ctx, abc, ni, na, p, p.total, out, [&](const bls_r1cs_matrix* dm, const bls_groth16_parameters_out* dp, void* scr) {
+    return gs_dev_impl(ctx, dm, nc, ni, na, g1, g2, sc5, dp, scr, ctx->stream);
+  });
+}
+
+// ---- phase 2: bls_groth16_mpc_new_* ----
+namespace {
+struct MpcPlan {
+  GsPlan g;                                      // shape, n, N1 = 3 + nv + n1 + 2 nv, N2 = 3 + nv, density words
+  size_t chunks_max;                             // k_mpc_qap chunks of the longest matrix
+  size_t off_flags, off_pts, off_p1, off_p2, off_x1, off_bnd, off_words, off_bn, total;
+};
+}  // namespace
+
+static bool mpc_args_ok(const bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc, size_t ni, size_t na, const bls_groth16_phase1* ph,
+                        const bls_g1_affine* g1, const bls_g2_affine* g2, const bls_groth16_parameters_out* out, MpcPlan& p) {
+  if (!gs_shape_ok(ctx, abc, nc, ni, na, p.g)) return false;
+  if (!g1 || !g2 || g1->infinity || g2->infinity || !ph || ph->n != p.g.n) return false;
+  if ((abc[0].nnz || abc[1].nnz || abc[2].nnz) && (!ph->coeffs_g1 || !ph->alpha_coeffs_g1 || !ph->beta_coeffs_g1 || !ph->coeffs_g2)) return false;
+  if (p.g.n1 && !ph->h) return false;
+  return gs_out_ok(out, ni, na, p.g);
+}
+
+static size_t mpc_layout(bls_ctx* ctx, const bls_r1cs_matrix* abc, MpcPlan& p) {
+  p.chunks_max = 0;
+  for (int m = 0; m < 3; m++) {
+    const size_t c = (abc[m].nnz + MPC_CHUNK - 1) / MPC_CHUNK;
+    p.chunks_max = c > p.chunks_max ? c : p.chunks_max;
+  }
+  size_t o = 0;
+  auto take = [&](size_t bytes) { size_t at = o; o += gs_align(bytes ? bytes : 1); return at; };
+  p.off_flags = take(sizeof(uint32_t));
+  p.off_pts = take(3 * sizeof(bls_g1_affine) + 3 * sizeof(bls_g2_affine));
+  p.off_p1 = take(p.g.N1 * sizeof(bls_g1));
+  p.off_p2 = take(p.g.N2 * sizeof(bls_g2));
+  p.off_x1 = take(3 * p.g.nv * sizeof(bls_g1));
+  p.off_bnd = take(2 * p.chunks_max * sizeof(bls_g2));
+  p.off_words = take(4 * p.g.words * sizeof(uint32_t));
+  const size_t b1 = bls_batch_normalization_scratch_bytes(ctx, 1, p.g.N1), b2 = bls_batch_normalization_scratch_bytes(ctx, 2, p.g.N2);
+  if (!b1 || !b2) return 0;
+  p.off_bn = take(b1 > b2 ? b1 : b2);
+  p.total = o;
+  return o;
+}
+
+static int mpc_dev_impl(bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc, size_t ni, size_t na, const bls_groth16_phase1* ph,
+                        const bls_g1_affine* g1, const bls_g2_affine* g2, const bls_groth16_parameters_out* out, void* scratch, void* stream) {
+  MpcPlan p;
+  if (!mpc_args_ok(ctx, abc, nc, ni, na, ph, g1, g2, out, p) || !scratch) return BLS_ERR_INVALID_ARGUMENT;
+  USE_DEVICE(ctx);
+  if (!mpc_layout(ctx, abc, p)) return BLS_ERR_CUDA;
+  cudaStream_t st = pick(ctx, stream);
+  char* base = (char*)scratch;
+  auto at = [&](size_t off) { return (uint64_t*)(base + off); };
+  const size_t nv = p.g.nv, n1 = p.g.n1;
+  uint32_t* flags = (uint32_t*)(base + p.off_flags);
+  uint64_t *pts = at(p.off_pts), *p1 = at(p.off_p1), *p2 = at(p.off_p2), *x1 = at(p.off_x1), *bnd = at(p.off_bnd);
+  uint32_t *wa = (uint32_t*)(base + p.off_words), *wb = wa + p.g.words, *pa = wb + p.g.words, *pb = pa + p.g.words;
+  // G1 batch [alpha, beta, delta | ic | l | h | a | b], G2 batch [beta, gamma, delta | b]: k_gs_emit's layout
+  uint64_t *p1_ext = p1 + G1_W * 3, *p1_h = p1_ext + G1_W * nv, *p1_a = p1_h + G1_W * n1, *p1_b = p1_a + G1_W * nv, *p2_b = p2 + G2_W * 3;
+
+  // vk points in one copy (a pageable source has been staged when cudaMemcpyAsync returns): alpha_g1, beta_g1, delta_g1 = g1,
+  // then beta_g2, gamma_g2 = delta_g2 = g2
+  uint64_t up[3 * G1A_W + 3 * G2A_W];
+  memcpy(up, &ph->alpha_g1, sizeof(bls_g1_affine));
+  memcpy(up + G1A_W, &ph->beta_g1, sizeof(bls_g1_affine));
+  memcpy(up + 2 * G1A_W, g1, sizeof(bls_g1_affine));
+  memcpy(up + 3 * G1A_W, &ph->beta_g2, sizeof(bls_g2_affine));
+  memcpy(up + 3 * G1A_W + G2A_W, g2, sizeof(bls_g2_affine));
+  memcpy(up + 3 * G1A_W + 2 * G2A_W, g2, sizeof(bls_g2_affine));
+  CK(cudaMemcpyAsync(pts, up, sizeof(up), cudaMemcpyHostToDevice, st));
+  CK(cudaMemsetAsync(flags, 0, sizeof(uint32_t), st));
+  k_mpc_load<Fp><<<1, GS_TPB, 0, st>>>(pts, 3, p1);
+  LAUNCH_CHECK();
+  k_mpc_load<Fp2><<<1, GS_TPB, 0, st>>>(pts + 3 * G1A_W, 3, p2);
+  LAUNCH_CHECK();
+  if (n1) {
+    k_mpc_load<Fp><<<blocks_for(n1, GS_TPB), GS_TPB, 0, st>>>((const uint64_t*)ph->h, n1, p1_h);
+    LAUNCH_CHECK();
+  }
+
+  if (nv) {
+    GsMats mats;
+    for (int m = 0; m < 3; m++) mats.m[m] = GsMat{abc[m].offsets, abc[m].constraint, (const uint64_t*)abc[m].coeff, abc[m].nnz};
+    const uint64_t *c1 = (const uint64_t*)ph->coeffs_g1, *al1 = (const uint64_t*)ph->alpha_coeffs_g1, *be1 = (const uint64_t*)ph->beta_coeffs_g1;
+    struct { int m; const uint64_t* rows; uint64_t* sums; } g1pass[5] = {
+        {0, c1, p1_a}, {0, be1, x1}, {1, c1, p1_b}, {1, al1, x1 + G1_W * nv}, {2, c1, x1 + 2 * G1_W * nv}};
+    for (const auto& ps : g1pass) {
+      const GsMat& M = mats.m[ps.m];
+      if (M.nnz) {
+        k_mpc_qap<Fp, false, MPC_K_G1><<<blocks_for((M.nnz + MPC_CHUNK - 1) / MPC_CHUNK, GS_TPB), GS_TPB, 0, st>>>(M, nv, nc, ps.rows, ps.sums, bnd, flags);
+        LAUNCH_CHECK();
+      }
+      k_mpc_fix<Fp><<<(unsigned)nv, GS_TPB, 0, st>>>(M, nv, bnd, ps.sums);
+      LAUNCH_CHECK();
+    }
+    if (mats.m[1].nnz) {
+      k_mpc_qap<Fp2, true, MPC_K_G2><<<blocks_for((mats.m[1].nnz + MPC_CHUNK - 1) / MPC_CHUNK, GS_TPB), GS_TPB, 0, st>>>(
+          mats.m[1], nv, nc, (const uint64_t*)ph->coeffs_g2, p2_b, bnd, flags);
+      LAUNCH_CHECK();
+    }
+    k_mpc_fix<Fp2><<<(unsigned)nv, GS_TPB, 0, st>>>(mats.m[1], nv, bnd, p2_b);
+    LAUNCH_CHECK();
+    k_mpc_combine<<<blocks_for(nv, GS_TPB), GS_TPB, 0, st>>>(mats, ni, nv, x1, p1_ext, p1_a, p1_b, p2_b, wa, wb, flags);
+    LAUNCH_CHECK();
+  }
+  k_gs_scan<<<1, GS_SCAN_TPB, 0, st>>>(wa, wb, p.g.words, ni, na, pa, pb, out->lens, out->a_aux_density, out->b_input_density, out->b_aux_density);
+  LAUNCH_CHECK();
+  TRY(bls_g1_batch_normalization_dev(ctx, (bls_g1*)p1, p.g.N1, base + p.off_bn, st));
+  TRY(bls_g2_batch_normalization_dev(ctx, (bls_g2*)p2, p.g.N2, base + p.off_bn, st));
+  GsOut o{(uint64_t*)out->vk, (uint64_t*)out->ic, (uint64_t*)out->h, (uint64_t*)out->l, (uint64_t*)out->a, (uint64_t*)out->b_g1,
+          (uint64_t*)out->b_g2, out->ok};
+  k_gs_emit<<<dim3(blocks_for(p.g.N1, GS_TPB), 2), GS_TPB, 0, st>>>(p1, p2, ni, na, n1, wa, pa, wb, pb, flags, o);
+  LAUNCH_CHECK();
+  return BLS_OK;
+}
+
+static int mpc_host(bls_ctx* ctx, const bls_r1cs_matrix* abc, size_t nc, size_t ni, size_t na, const bls_groth16_phase1* ph,
+                    const bls_g1_affine* g1, const bls_g2_affine* g2, const bls_groth16_parameters_out* out) {
+  MpcPlan p;
+  if (!mpc_args_ok(ctx, abc, nc, ni, na, ph, g1, g2, out, p)) return BLS_ERR_INVALID_ARGUMENT;
+  if (!gs_matrices_ok(abc, nc, p.g.nv)) return BLS_ERR_INVALID_ARGUMENT;
+  USE_DEVICE(ctx);
+  if (!mpc_layout(ctx, abc, p)) return BLS_ERR_CUDA;
+  const size_t n = p.g.n, rows = (abc[0].nnz || abc[1].nnz || abc[2].nnz) ? n : 0, ga = sizeof(bls_g1_affine);
+  H2D(r1, rows ? ph->coeffs_g1 : nullptr, rows * ga);
+  H2D(ra, rows ? ph->alpha_coeffs_g1 : nullptr, rows * ga);
+  H2D(rb, rows ? ph->beta_coeffs_g1 : nullptr, rows * ga);
+  H2D(r2, rows ? ph->coeffs_g2 : nullptr, rows * sizeof(bls_g2_affine));
+  H2D(rh, p.g.n1 ? ph->h : nullptr, p.g.n1 * ga);
+  bls_groth16_phase1 dph = *ph;
+  dph.coeffs_g1 = (const bls_g1_affine*)r1.p;
+  dph.alpha_coeffs_g1 = (const bls_g1_affine*)ra.p;
+  dph.beta_coeffs_g1 = (const bls_g1_affine*)rb.p;
+  dph.coeffs_g2 = (const bls_g2_affine*)r2.p;
+  dph.h = (const bls_g1_affine*)rh.p;
+  return gs_host_run(ctx, abc, ni, na, p.g, p.total, out, [&](const bls_r1cs_matrix* dm, const bls_groth16_parameters_out* dp, void* scr) {
+    return mpc_dev_impl(ctx, dm, nc, ni, na, &dph, g1, g2, dp, scr, ctx->stream);
+  });
+}
+
 extern "C" {
 
 size_t bls_groth16_generate_parameters_scratch_bytes(const bls_ctx* cctx, const bls_r1cs_matrix abc[3], size_t num_constraints, size_t num_inputs,
@@ -644,6 +1010,25 @@ int bls_groth16_generate_parameters_batch(bls_ctx* ctx, const bls_r1cs_matrix ab
                                           const bls_fr* gamma, const bls_fr* delta, const bls_fr* tau, const bls_groth16_parameters_out* out) {
   const bls_fr* const sc[5] = {alpha, beta, gamma, delta, tau};
   return gs_host(ctx, abc, num_constraints, num_inputs, num_aux, g1, g2, sc, out);
+}
+
+size_t bls_groth16_mpc_new_scratch_bytes(const bls_ctx* cctx, const bls_r1cs_matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux) {
+  MpcPlan p;
+  if (!gs_shape_ok(cctx, abc, num_constraints, num_inputs, num_aux, p.g)) return 0;
+  bls_ctx* ctx = const_cast<bls_ctx*>(cctx);
+  DevGuard g;
+  if (g.enter(ctx->device) != cudaSuccess) return 0;
+  return mpc_layout(ctx, abc, p);
+}
+int bls_groth16_mpc_new_dev(bls_ctx* ctx, const bls_r1cs_matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux,
+                            const bls_groth16_phase1* phase1, const bls_g1_affine* g1, const bls_g2_affine* g2,
+                            const bls_groth16_parameters_out* out, void* scratch, void* stream) {
+  return mpc_dev_impl(ctx, abc, num_constraints, num_inputs, num_aux, phase1, g1, g2, out, scratch, stream);
+}
+int bls_groth16_mpc_new_batch(bls_ctx* ctx, const bls_r1cs_matrix abc[3], size_t num_constraints, size_t num_inputs, size_t num_aux,
+                              const bls_groth16_phase1* phase1, const bls_g1_affine* g1, const bls_g2_affine* g2,
+                              const bls_groth16_parameters_out* out) {
+  return mpc_host(ctx, abc, num_constraints, num_inputs, num_aux, phase1, g1, g2, out);
 }
 
 }  // extern "C"

@@ -275,7 +275,63 @@ class DeviceEngine:
         tensors and whose densities are numpy bool arrays, so it goes to groth16_prove unchanged.  Reading a_len and b_len to
         trim the queries synchronises the stream."""
         ni, na = int(num_inputs), int(num_aux)
-        nv = ni + na
+        mats = self._r1cs_mats(abc, ni + na)
+        host = [nat._arr(nat.np.reshape(x, (1, -1)), w, name) for x, w, name in
+                ((g1, nat.W_G1A, "g1"), (g2, nat.W_G2A, "g2"), (alpha, nat.W_FR, "alpha"), (beta, nat.W_FR, "beta"), (gamma, nat.W_FR, "gamma"),
+                 (delta, nat.W_FR, "delta"), (tau, nat.W_FR, "tau"))]
+        bufs, out = self._parameters_out(num_constraints, ni, na)
+        scr = self._buf("groth16_setup", self.ctx.groth16_generate_parameters_scratch_bytes(mats, num_constraints, ni, na))
+        self.ctx.call_dev("bls_groth16_generate_parameters_dev", mats, num_constraints, ni, na, *[nat._p(x) for x in host], ctypes.byref(out),
+                          scr.data_ptr(), self._stream())
+        return self._parameters(bufs, ni, na)
+
+    def groth16_mpc_new(self, abc, num_constraints, num_inputs, num_aux, phase1, g1, g2):
+        """phase2's MPCParameters::new on the device (bls_groth16_mpc_new_dev): abc as for groth16_generate_parameters, phase1
+        a Groth16Phase1 whose row sets are contiguous CUDA int64 tensors ((n, 13), (n, 25) for coeffs_g2, (n - 1, 13) for h)
+        and whose vk points are host rows; g1 and g2 host rows.  Returns a Groth16Parameters as groth16_generate_parameters
+        does; reading a_len and b_len synchronises the stream."""
+        ni, na = int(num_inputs), int(num_aux)
+        mats = self._r1cs_mats(abc, ni + na)
+        for name in ("coeffs_g1", "alpha_coeffs_g1", "beta_coeffs_g1", "coeffs_g2", "h"):
+            _check(getattr(phase1, name), nat.W_G2A if name == "coeffs_g2" else nat.W_G1A, name)
+        ph = nat.groth16_phase1_c(phase1, num_constraints, lambda t: t.data_ptr(), lambda t: int(t.shape[0]))
+        g1 = nat._arr(nat.np.reshape(g1, (1, -1)), nat.W_G1A, "g1")
+        g2 = nat._arr(nat.np.reshape(g2, (1, -1)), nat.W_G2A, "g2")
+        bufs, out = self._parameters_out(num_constraints, ni, na)
+        scr = self._buf("groth16_mpc", self.ctx.groth16_mpc_new_scratch_bytes(mats, num_constraints, ni, na))
+        self.ctx.call_dev("bls_groth16_mpc_new_dev", mats, num_constraints, ni, na, ctypes.byref(ph), nat._p(g1), nat._p(g2), ctypes.byref(out),
+                          scr.data_ptr(), self._stream())
+        return self._parameters(bufs, ni, na)
+
+    def groth16_mpc_contribute(self, params, delta, s, r, in_place=False):
+        """phase2's MPCParameters::contribute on the device (bls_groth16_mpc_contribute_dev): params a Groth16Parameters whose
+        vk rows and queries are CUDA int64 tensors; delta, s and r host rows as for Context.groth16_mpc_contribute.  Returns
+        (the contributed Groth16Parameters, the (89,) pubkey as a CUDA int64 tensor); in_place writes h and l over the inputs."""
+        _check(params.h, nat.W_G1A, "h"); _check(params.l, nat.W_G1A, "l")
+        host = [nat._arr(nat.np.reshape(x, (1, -1)), w, name) for x, w, name in ((delta, nat.W_FR, "delta"), (s, nat.W_G1A, "s"), (r, nat.W_G2A, "r"))]
+        vk = torch.cat([getattr(params, name).reshape(-1) for name, _, _ in nat.VK_POINT_ROWS]).contiguous()
+        h, l = (params.h, params.l) if in_place else (torch.empty_like(params.h), torch.empty_like(params.l))
+        pk = torch.zeros(nat.W_MPC_PUBKEY, dtype=torch.int64, device=self.device)
+        scr = self._buf("groth16_mpc", self.ctx.groth16_mpc_contribute_scratch_bytes(params.h.shape[0], params.l.shape[0]))
+        self.ctx.call_dev("bls_groth16_mpc_contribute_dev", *[nat._p(x) for x in host], vk.data_ptr(), params.h.data_ptr(), params.h.shape[0],
+                          params.l.data_ptr(), params.l.shape[0], h.data_ptr(), l.data_ptr(), pk.data_ptr(), scr.data_ptr(), self._stream())
+        return nat.contributed(params, vk, h, l), pk
+
+    def groth16_mpc_verify(self, before, after, pubkeys, rho_h, rho_l):
+        """phase2's MPCParameters::verify on the device (bls_groth16_mpc_verify_dev): before and after Groth16Parameters of CUDA
+        tensors, pubkeys a (k, 89) CUDA int64 tensor, rho_h and rho_l (h_len, 4) / (l_len, 4) CUDA int64 tensors.  Returns a
+        bool (reading it synchronises the stream)."""
+        row = lambda t: t.cpu().numpy().view(nat.np.uint64)
+        kb, ka = (nat.groth16_key_c(k, lambda t: t.data_ptr(), lambda t: int(t.shape[0]), row) for k in (before, after))
+        _check(pubkeys, nat.W_MPC_PUBKEY, "pubkeys"); _check(rho_h, nat.W_FR, "rho_h"); _check(rho_l, nat.W_FR, "rho_l")
+        ok = torch.zeros(1, dtype=torch.uint8, device=self.device)
+        scr = self._buf("groth16_mpc", self.ctx.groth16_mpc_verify_scratch_bytes(kb, ka, pubkeys.shape[0]))
+        self.ctx.call_dev("bls_groth16_mpc_verify_dev", ctypes.byref(kb), ctypes.byref(ka), pubkeys.data_ptr(), pubkeys.shape[0], rho_h.data_ptr(),
+                          rho_l.data_ptr(), ok.data_ptr(), scr.data_ptr(), self._stream())
+        return bool(ok.cpu()[0])
+
+    @staticmethod
+    def _r1cs_mats(abc, nv):
         if len(abc) != 3:
             raise ValueError("abc must hold the three matrices A, B and C")
         mats = (nat.R1csMatrixC * 3)()
@@ -287,19 +343,21 @@ class DeviceEngine:
                 raise ValueError("matrix %d: offsets, constraint, coeff must be contiguous CUDA tensors int64 (%d,), int32 (nnz,), int64 (nnz, 4)"
                                  % (i, nv + 1))
             mats[i] = nat.R1csMatrixC(off.data_ptr(), cons.data_ptr(), coeff.data_ptr(), cons.shape[0])
-        host = [nat._arr(nat.np.reshape(x, (1, -1)), w, name) for x, w, name in
-                ((g1, nat.W_G1A, "g1"), (g2, nat.W_G2A, "g2"), (alpha, nat.W_FR, "alpha"), (beta, nat.W_FR, "beta"), (gamma, nat.W_FR, "gamma"),
-                 (delta, nat.W_FR, "delta"), (tau, nat.W_FR, "tau"))]
-        n1 = (1 << max(int(num_constraints) - 1, 0).bit_length()) - 1
+        return mats
+
+    def _parameters_out(self, num_constraints, ni, na):
+        nv, n1 = ni + na, nat.domain_size(num_constraints) - 1
         e = lambda *shape: torch.zeros(shape, dtype=torch.int64, device=self.device)
         vk, ic, h, l, a, b_g1, b_g2 = e(nat.W_VK_POINTS), e(ni, nat.W_G1A), e(n1, nat.W_G1A), e(na, nat.W_G1A), e(nv, nat.W_G1A), e(nv, nat.W_G1A), e(nv, nat.W_G2A)
         dens = [torch.zeros((k + 31) // 32, dtype=torch.int32, device=self.device) for k in (na, ni, na)]
         lens = e(2)
         ok = torch.zeros(1, dtype=torch.uint8, device=self.device)
         out = nat.Groth16ParametersOutC(*[t.data_ptr() for t in (vk, ic, h, l, a, b_g1, b_g2, *dens, lens, ok)])
-        scr = self._buf("groth16_setup", self.ctx.groth16_generate_parameters_scratch_bytes(mats, num_constraints, ni, na))
-        self.ctx.call_dev("bls_groth16_generate_parameters_dev", mats, num_constraints, ni, na, *[nat._p(x) for x in host], ctypes.byref(out),
-                          scr.data_ptr(), self._stream())
+        return (vk, ic, h, l, a, b_g1, b_g2, dens, lens, ok), out
+
+    @staticmethod
+    def _parameters(bufs, ni, na):
+        vk, ic, h, l, a, b_g1, b_g2, dens, lens, ok = bufs
         words = [d.cpu().numpy().view(nat.np.uint32) for d in dens]
         return nat.groth16_parameters(vk, ic, h, l, a, b_g1, b_g2, words, lens.cpu().numpy(), int(ok.cpu()[0]), ni, na)
 

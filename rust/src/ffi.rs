@@ -45,11 +45,29 @@ use std::os::raw::{c_char, c_int, c_void};
     pub a_aux_density: *mut u32, pub b_input_density: *mut u32, pub b_aux_density: *mut u32,
     pub lens: *mut u64, pub ok: *mut u8,
 }
+/// powersoftau's prepare_phase2 rows for a domain of n points (include/pairing_b200_mpc.h): n rows per coefficient set, n - 1 h rows
+#[repr(C)] pub struct bls_groth16_phase1 {
+    pub alpha_g1: bls_g1_affine, pub beta_g1: bls_g1_affine, pub beta_g2: bls_g2_affine,
+    pub coeffs_g1: *const bls_g1_affine, pub alpha_coeffs_g1: *const bls_g1_affine, pub beta_coeffs_g1: *const bls_g1_affine,
+    pub coeffs_g2: *const bls_g2_affine, pub h: *const bls_g1_affine, pub n: usize,
+}
+/// phase2's PublicKey without its transcript hash, plus r = hash_to_g2(transcript)
+#[repr(C)] #[derive(Copy, Clone)] pub struct bls_groth16_mpc_pubkey {
+    pub delta_after: bls_g1_affine, pub s: bls_g1_affine, pub s_delta: bls_g1_affine, pub r: bls_g2_affine, pub r_delta: bls_g2_affine,
+}
+/// bellman's Parameters<Bls12> for bls_groth16_mpc_verify_batch: the vk by value, the queries by pointer
+#[repr(C)] pub struct bls_groth16_key {
+    pub vk: bls_groth16_vk_points,
+    pub ic: *const bls_g1_affine, pub h: *const bls_g1_affine, pub l: *const bls_g1_affine, pub a: *const bls_g1_affine,
+    pub b_g1: *const bls_g1_affine, pub b_g2: *const bls_g2_affine,
+    pub ic_len: usize, pub h_len: usize, pub l_len: usize, pub a_len: usize, pub b_len: usize,
+}
 pub enum bls_ctx {}
 /// several devices of one node behind one call (include/pairing_b200.h, "several GPUs")
 pub enum bls_mgpu {}
 
 pub const BLS_OK: c_int = 0;
+pub const BLS_ERR_INVALID_ARGUMENT: c_int = -1;
 
 extern "C" {
     pub fn bls_ctx_create(device: c_int, err: *mut c_int) -> *mut bls_ctx;
@@ -102,6 +120,16 @@ extern "C" {
                                                  num_aux: usize, g1: *const bls_g1_affine, g2: *const bls_g2_affine, alpha: *const bls_fr_repr,
                                                  beta: *const bls_fr_repr, gamma: *const bls_fr_repr, delta: *const bls_fr_repr, tau: *const bls_fr_repr,
                                                  out: *const bls_groth16_parameters_out) -> c_int;
+    pub fn bls_groth16_mpc_contribute_batch(ctx: *mut bls_ctx, delta: *const bls_fr_repr, s: *const bls_g1_affine, r: *const bls_g2_affine,
+                                            vk: *mut bls_groth16_vk_points, h: *const bls_g1_affine, h_len: usize, l: *const bls_g1_affine,
+                                            l_len: usize, h_out: *mut bls_g1_affine, l_out: *mut bls_g1_affine,
+                                            pubkey: *mut bls_groth16_mpc_pubkey) -> c_int;
+    pub fn bls_groth16_mpc_verify_batch(ctx: *mut bls_ctx, before: *const bls_groth16_key, after: *const bls_groth16_key,
+                                        pk: *const bls_groth16_mpc_pubkey, k: usize, rho_h: *const bls_fr_repr, rho_l: *const bls_fr_repr,
+                                        ok1: *mut u8) -> c_int;
+    pub fn bls_groth16_mpc_new_batch(ctx: *mut bls_ctx, abc: *const bls_r1cs_matrix, num_constraints: usize, num_inputs: usize, num_aux: usize,
+                                     phase1: *const bls_groth16_phase1, g1: *const bls_g1_affine, g2: *const bls_g2_affine,
+                                     out: *const bls_groth16_parameters_out) -> c_int;
     pub fn bls_kzg_commit_batch(ctx: *mut bls_ctx, srs: *const bls_g1_affine, srs_len: usize, p: *const bls_fr_repr, n: usize, m: usize,
                                 c: *mut bls_g1_affine) -> c_int;
     pub fn bls_kzg_open_batch(ctx: *mut bls_ctx, srs: *const bls_g1_affine, srs_len: usize, p: *const bls_fr_repr, n: usize, z: *const bls_fr_repr,

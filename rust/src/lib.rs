@@ -16,6 +16,7 @@ pub mod ffi;
 
 use self::ffi::*;
 use crate::bls12_381::{Fq12, Fr, FrRepr, G1Affine, G2Affine, G1, G2};
+use std::os::raw::c_int;
 use std::sync::Mutex;
 
 #[derive(Debug)]
@@ -365,6 +366,99 @@ impl Gpu {
     pub fn groth16_generate_parameters(&self, abc: [(&[u64], &[u32], &[Fr]); 3], num_constraints: usize, num_inputs: usize, num_aux: usize,
                                        g1: &G1Affine, g2: &G2Affine, alpha: &Fr, beta: &Fr, gamma: &Fr, delta: &Fr, tau: &Fr)
                                        -> Result<(Groth16Params, G2Affine, Vec<G1Affine>, [Vec<u32>; 3]), GpuError> {
+        let (gg1, gg2) = (marshal::g1_affine(g1), marshal::g2_affine(g2));
+        let sc: Vec<bls_fr_repr> = [alpha, beta, gamma, delta, tau].iter().map(|x| marshal::fr(x)).collect();
+        self.groth16_key(abc, num_constraints, num_inputs, num_aux, "UnconstrainedVariable: an l query point is the identity", |ctx, mats, out| unsafe {
+            bls_groth16_generate_parameters_batch(ctx, mats, num_constraints, num_inputs, num_aux, &gg1, &gg2, &sc[0], &sc[1], &sc[2], &sc[3], &sc[4], out)
+        })
+    }
+
+    /// phase2's `MPCParameters::new` (include/pairing_b200_mpc.h): the circuit's key from powersoftau's `prepare_phase2` rows
+    /// for the domain of `num_constraints` (`coeffs_g1`, `alpha_coeffs_g1`, `beta_coeffs_g1`, `coeffs_g2` of n rows, `h` of
+    /// n - 1), before any contribution: gamma_g2 = delta_g2 = g2, delta_g1 = g1.  Same matrices and result as
+    /// `groth16_generate_parameters`; `Err` on `UnconstrainedVariable` or on a transcript whose b_g1 and b_g2 disagree on the identity.
+    pub fn groth16_mpc_new(&self, abc: [(&[u64], &[u32], &[Fr]); 3], num_constraints: usize, num_inputs: usize, num_aux: usize,
+                           alpha_g1: &G1Affine, beta_g1: &G1Affine, beta_g2: &G2Affine, coeffs_g1: &[G1Affine], alpha_coeffs_g1: &[G1Affine],
+                           beta_coeffs_g1: &[G1Affine], coeffs_g2: &[G2Affine], h: &[G1Affine], g1: &G1Affine, g2: &G2Affine)
+                           -> Result<(Groth16Params, G2Affine, Vec<G1Affine>, [Vec<u32>; 3]), GpuError> {
+        let n = coeffs_g1.len();
+        if alpha_coeffs_g1.len() != n || beta_coeffs_g1.len() != n || coeffs_g2.len() != n || h.len() + 1 != n {
+            return Err(GpuError(BLS_ERR_INVALID_ARGUMENT, "groth16_mpc_new: n rows per coefficient set and n - 1 h rows".to_string()));
+        }
+        let r1 = |v: &[G1Affine]| -> Vec<bls_g1_affine> { v.iter().map(marshal::g1_affine).collect() };
+        let (c1, a1, b1, hh) = (r1(coeffs_g1), r1(alpha_coeffs_g1), r1(beta_coeffs_g1), r1(h));
+        let c2: Vec<bls_g2_affine> = coeffs_g2.iter().map(marshal::g2_affine).collect();
+        let ph = bls_groth16_phase1 {
+            alpha_g1: marshal::g1_affine(alpha_g1), beta_g1: marshal::g1_affine(beta_g1), beta_g2: marshal::g2_affine(beta_g2),
+            coeffs_g1: c1.as_ptr(), alpha_coeffs_g1: a1.as_ptr(), beta_coeffs_g1: b1.as_ptr(), coeffs_g2: c2.as_ptr(), h: hh.as_ptr(), n,
+        };
+        let (gg1, gg2) = (marshal::g1_affine(g1), marshal::g2_affine(g2));
+        self.groth16_key(abc, num_constraints, num_inputs, num_aux,
+                         "UnconstrainedVariable or an inconsistent transcript: an l query point is the identity, or b_g1 and b_g2 disagree",
+                         |ctx, mats, out| unsafe { bls_groth16_mpc_new_batch(ctx, mats, num_constraints, num_inputs, num_aux, &ph, &gg1, &gg2, out) })
+    }
+
+    /// phase2's `MPCParameters::contribute` (include/pairing_b200_mpc.h) for the caller's secret `delta`, `s` and `r =
+    /// hash_to_g2(transcript)`: `h` and `l` are multiplied by delta^-1 and `delta_g1`, `delta_g2` by delta, in place.  The
+    /// caller computes `s_delta = s * delta` first (it goes into the transcript r is derived from).  Returns phase2's public key.
+    pub fn groth16_mpc_contribute(&self, params: &mut Groth16Params, delta: &Fr, s: &G1Affine, r: &G2Affine)
+                                  -> Result<bls_groth16_mpc_pubkey, GpuError> {
+        let zero1 = bls_g1_affine { x: marshal::FQ_ZERO, y: marshal::FQ_ZERO, infinity: 1 };
+        let zero2 = bls_g2_affine { x: marshal::FQ2_ZERO, y: marshal::FQ2_ZERO, infinity: 1 };
+        let mut vk = bls_groth16_vk_points {
+            alpha_g1: marshal::g1_affine(&params.alpha_g1), beta_g1: marshal::g1_affine(&params.beta_g1), delta_g1: marshal::g1_affine(&params.delta_g1),
+            beta_g2: marshal::g2_affine(&params.beta_g2), gamma_g2: zero2, delta_g2: marshal::g2_affine(&params.delta_g2),
+        };
+        let mut h: Vec<bls_g1_affine> = params.h.iter().map(marshal::g1_affine).collect();
+        let mut l: Vec<bls_g1_affine> = params.l.iter().map(marshal::g1_affine).collect();
+        let mut pk = bls_groth16_mpc_pubkey { delta_after: zero1, s: zero1, s_delta: zero1, r: zero2, r_delta: zero2 };
+        let (dd, ss, rr) = (marshal::fr(delta), marshal::g1_affine(s), marshal::g2_affine(r));
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe {
+            bls_groth16_mpc_contribute_batch(*ctx, &dd, &ss, &rr, &mut vk, h.as_ptr(), h.len(), l.as_ptr(), l.len(), h.as_mut_ptr(), l.as_mut_ptr(), &mut pk)
+        }, *ctx)?;
+        params.h = h.iter().map(marshal::g1_affine_back).collect();
+        params.l = l.iter().map(marshal::g1_affine_back).collect();
+        params.delta_g1 = marshal::g1_affine_back(&vk.delta_g1);
+        params.delta_g2 = marshal::g2_affine_back(&vk.delta_g2);
+        Ok(pk)
+    }
+
+    /// phase2's `MPCParameters::verify`: `before` is the key of `groth16_mpc_new` and `after` the contributed key, each with
+    /// its `gamma_g2` and `ic`; `pks` the contributions' public keys in order; `rho_h`, `rho_l` the caller's randomizers of
+    /// the merged pairs (one per h and l row).  The transcript hash checks stay with the caller.
+    pub fn groth16_mpc_verify(&self, before: (&Groth16Params, &G2Affine, &[G1Affine]), after: (&Groth16Params, &G2Affine, &[G1Affine]),
+                              pks: &[bls_groth16_mpc_pubkey], rho_h: &[FrRepr], rho_l: &[FrRepr]) -> Result<bool, GpuError> {
+        let g1v = |v: &[G1Affine]| -> Vec<bls_g1_affine> { v.iter().map(marshal::g1_affine).collect() };
+        let rows = |k: &(&Groth16Params, &G2Affine, &[G1Affine])| {
+            (g1v(k.2), g1v(&k.0.h), g1v(&k.0.l), g1v(&k.0.a), g1v(&k.0.b_g1), k.0.b_g2.iter().map(marshal::g2_affine).collect::<Vec<bls_g2_affine>>())
+        };
+        let key = |k: &(&Groth16Params, &G2Affine, &[G1Affine]), r: &(Vec<bls_g1_affine>, Vec<bls_g1_affine>, Vec<bls_g1_affine>, Vec<bls_g1_affine>,
+                                                                    Vec<bls_g1_affine>, Vec<bls_g2_affine>)| bls_groth16_key {
+            vk: bls_groth16_vk_points {
+                alpha_g1: marshal::g1_affine(&k.0.alpha_g1), beta_g1: marshal::g1_affine(&k.0.beta_g1), delta_g1: marshal::g1_affine(&k.0.delta_g1),
+                beta_g2: marshal::g2_affine(&k.0.beta_g2), gamma_g2: marshal::g2_affine(k.1), delta_g2: marshal::g2_affine(&k.0.delta_g2),
+            },
+            ic: r.0.as_ptr(), h: r.1.as_ptr(), l: r.2.as_ptr(), a: r.3.as_ptr(), b_g1: r.4.as_ptr(), b_g2: r.5.as_ptr(),
+            ic_len: r.0.len(), h_len: r.1.len(), l_len: r.2.len(), a_len: r.3.len(), b_len: r.4.len(),
+        };
+        if rho_h.len() != before.0.h.len() || rho_l.len() != before.0.l.len() || before.0.b_g1.len() != before.0.b_g2.len()
+            || after.0.b_g1.len() != after.0.b_g2.len() {
+            return Err(GpuError(BLS_ERR_INVALID_ARGUMENT, "groth16_mpc_verify: one randomizer per h and l row, and b_g1 as long as b_g2".to_string()));
+        }
+        let (rb, ra) = (rows(&before), rows(&after));
+        let (kb, ka) = (key(&before, &rb), key(&after, &ra));
+        let rh: Vec<bls_fr_repr> = rho_h.iter().map(|r| bls_fr_repr { l: r.0 }).collect();
+        let rl: Vec<bls_fr_repr> = rho_l.iter().map(|r| bls_fr_repr { l: r.0 }).collect();
+        let mut ok = 0u8;
+        let ctx = self.ctx.lock().unwrap();
+        check(unsafe { bls_groth16_mpc_verify_batch(*ctx, &kb, &ka, pks.as_ptr(), pks.len(), rh.as_ptr(), rl.as_ptr(), &mut ok) }, *ctx)?;
+        Ok(ok != 0)
+    }
+
+    fn groth16_key<F>(&self, abc: [(&[u64], &[u32], &[Fr]); 3], num_constraints: usize, num_inputs: usize, num_aux: usize, not_ok: &str, call: F)
+                      -> Result<(Groth16Params, G2Affine, Vec<G1Affine>, [Vec<u32>; 3]), GpuError>
+    where F: FnOnce(*mut bls_ctx, *const bls_r1cs_matrix, *const bls_groth16_parameters_out) -> c_int {
         let nv = num_inputs + num_aux;
         let coeffs: Vec<Vec<bls_fr_repr>> = abc.iter().map(|m| m.2.iter().map(marshal::fr).collect()).collect();
         let mats: Vec<bls_r1cs_matrix> = abc.iter().zip(coeffs.iter()).map(|(m, c)| {
@@ -384,15 +478,10 @@ impl Gpu {
             a_aux_density: dens[0].as_mut_ptr(), b_input_density: dens[1].as_mut_ptr(), b_aux_density: dens[2].as_mut_ptr(),
             lens: lens.as_mut_ptr(), ok: &mut ok,
         };
-        let (gg1, gg2) = (marshal::g1_affine(g1), marshal::g2_affine(g2));
-        let sc: Vec<bls_fr_repr> = [alpha, beta, gamma, delta, tau].iter().map(|x| marshal::fr(x)).collect();
         let ctx = self.ctx.lock().unwrap();
-        check(unsafe {
-            bls_groth16_generate_parameters_batch(*ctx, mats.as_ptr(), num_constraints, num_inputs, num_aux, &gg1, &gg2, &sc[0], &sc[1], &sc[2],
-                                                  &sc[3], &sc[4], &out)
-        }, *ctx)?;
+        check(call(*ctx, mats.as_ptr(), &out as *const bls_groth16_parameters_out), *ctx)?;
         if ok == 0 {
-            return Err(GpuError(-1, "UnconstrainedVariable: an l query point is the identity".to_string()));
+            return Err(GpuError(-1, not_ok.to_string()));
         }
         let g1v = |v: &[bls_g1_affine]| -> Vec<G1Affine> { v.iter().map(marshal::g1_affine_back).collect() };
         let params = Groth16Params {
